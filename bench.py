@@ -3,6 +3,7 @@
 surrogates/sec at 1/2/4/8 B200 vs CPU").
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload wct_mc|cwt] [--impl reference]
+                    [--dump-outputs DIR]
 
 Workloads (one "step" = one pass of the hot path over one batch of synthetic input):
   wct_mc  (default, the line's `value`)  BASELINE cfg5 as stated: ONE job of 100 000 AR(1)
@@ -31,6 +32,11 @@ drives all N GPUs through the library's own worker pool (rank 0 makes the call, 
 wait on a CPU barrier), host wall clock.
 `--impl reference` times the CPU restatement of the reference's path (oracle/, NumPy float64 --
 pycwt itself is not installable offline) on all host cores instead.
+`--dump-outputs DIR` writes, after the timed steps, what the last timed step of the primary workload
+returned, as DIR/<name>.npy: wct_mc `sig95` (float64 [65]: the thresholds of the scales below
+maxscale, the ones that are defined) and `hist` (the all-reduced histogram, float64 [66, 1000]); cwt `power_sample` (float32 [64, 120, 1024]: the power planes of 64 series of
+rank 0's batch, picked by a fixed seed).  Every input is generated from a fixed seed, so two builds
+run with the same arguments can be compared output for output.
 """
 
 from __future__ import annotations
@@ -50,12 +56,23 @@ import numpy as np
 
 ROOT = Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
+sys.dont_write_bytecode = True      # the bench may run from a read-only tree: it writes nothing there
 
 DT = 1 / 12
 CWT = dict(n0=1024, dj=1 / 12, s0=2 * DT, J=119, f0=6.0, ar1=0.7)
 MC = dict(a1=0.989, a2=0.966, dj=1 / 8, s0=2 * DT, J=65, f0=6.0, seed=2024, level=0.95)
 MC_FLOP = 150e6          # SURVEY 8d: algorithmic flop per realisation (N = 4096, 66 scales, 5 N log2 N per FFT)
 FP32_PEAK_NOMINAL = 148 * 128 * 2 * 1.965e9
+DUMP_SERIES = 64         # cwt --dump-outputs: series sampled from the batch (64 x 120 x 1024 FP32 = 31 MB)
+
+
+def dump_outputs(directory, arrays):
+    """np.save each array as directory/<name>.npy."""
+    out = Path(directory)
+    out.mkdir(parents=True, exist_ok=True)
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64) and np.isfinite(a).all(), name
+        np.save(out / f"{name}.npy", a)
 
 
 def _profile_json(name):
@@ -68,7 +85,7 @@ def measured_peaks():
     if p.exists():
         d = json.loads(p.read_text())
         return float(d["hbm_gbs"]), "measured (MEASURED_PEAKS.json)"
-    return 6650.0, "fallback (B200_PROFILING.md)"
+    return 6650.0, "fallback: device copy rate of profiles/r1_hbm_write_peak.json (B200, 1000 W limit)"
 
 
 # --------------------------------------------------------------------------- clocks
@@ -253,6 +270,7 @@ def setup_gpu(args):
     if c.world != args.gpus and c.world > 1:
         args.gpus = c.world
     torch.cuda.set_device(c.local)
+    torch.manual_seed(1000 + c.rank)     # the secondaries' torch.randn inputs: the same in every run
     # Run this rank on the CPUs next to its GPU before any pinned host buffer is allocated: the
     # host-buffer (e2e) arm is a PCIe stream per rank, and first-touch places its staging memory
     # on the NUMA node the thread runs on.
@@ -369,6 +387,10 @@ def bench_mc(c, args, sampler):
     sig_host = shim.wct_sig_from_hist(total, maxscale, MC["level"], has)
     check = {"hist_sha256_16": hashlib.sha256(total.tobytes()).hexdigest()[:16], "hist_total": int(total.sum())}
     if c.rank == 0:
+        if args.dump_outputs:
+            # rows from maxscale on have no reliable samples: their threshold is NaN, as in pycwt
+            dump_outputs(args.dump_outputs, {"sig95": h_sig.numpy()[:maxscale].copy(),
+                                             "hist": total.astype(np.float64)})
         assert np.array_equal(h_sig.numpy(), sig_host, equal_nan=True), "device percentile differs from the host's"
         whole = torch.zeros_like(hist)
         if c.world > 1:
@@ -493,8 +515,9 @@ def bench_mc(c, args, sampler):
     return line
 
 
-def bench_cwt(c, args, sampler=None, steps=None, warmup=None):
-    """cfg4: fused CWT+power on the per-GPU shard (weak scaling, no collective)."""
+def bench_cwt(c, args, sampler=None, steps=None, warmup=None, dump_dir=None):
+    """cfg4: fused CWT+power on the per-GPU shard (weak scaling, no collective).  With `dump_dir`,
+    rank 0 writes a fixed sample of the last step's power planes there."""
     torch, shim = c.torch, c.shim
     from wavelet_transformer_b200 import engine
     steps = steps or args.steps
@@ -519,6 +542,9 @@ def bench_cwt(c, args, sampler=None, steps=None, warmup=None):
 
     ms, spread, launches = timed_steps(c, step, steps, warmup, sampler)
     clocks = sampler.stop() if sampler else None
+    if dump_dir and c.rank == 0:
+        rows = np.sort(np.random.default_rng(0).choice(B, size=min(B, DUMP_SERIES), replace=False))
+        dump_outputs(dump_dir, {"power_sample": power[torch.from_numpy(rows).to(c.dev)].cpu().numpy()})
     value = c.world * B * S * n0 * steps / (ms * 1e-3)
     per_launch_s = ms * 1e-3 / steps
     alg_bytes = 4.0 * B * n0 * (1 + S)          # read x once, write the power plane once
@@ -668,7 +694,7 @@ def run_gpu(args):
             line["secondary_filterbank"] = guarded("filterbank secondary", lambda: bench_filterbank(c))
             line["secondary_cwt_shapes"] = guarded("cwt shapes secondary", lambda: bench_cwt_shapes(c))
     else:
-        line = bench_cwt(c, args, sampler)
+        line = bench_cwt(c, args, sampler, dump_dir=args.dump_outputs)
         if not args.no_secondary:
             line["secondary_filterbank"] = guarded("filterbank secondary", lambda: bench_filterbank(c))
     if c.rank == 0:
@@ -702,7 +728,13 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-secondary", action="store_true")
     ap.add_argument("--no-injected", action="store_true", help="skip the host-supplied-surrogates end-to-end arm")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU path only")
     args.warmup = max(args.warmup, 0)
     if args.impl == "reference":
         return run_reference(args)

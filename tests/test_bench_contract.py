@@ -38,6 +38,14 @@ def test_reference_arm_other_ranks_exit_quietly():
     assert proc.returncode == 0 and proc.stdout.strip() == ""
 
 
+@pytest.mark.parametrize("extra,message", [(["--steps", "0"], "--steps"),
+                                           (["--impl", "reference", "--dump-outputs", "out"], "--dump-outputs")])
+def test_bad_arguments_are_refused(extra, message):
+    proc = subprocess.run([sys.executable, str(ROOT / "bench.py"), *extra], capture_output=True, text=True, timeout=120,
+                          cwd=ROOT)
+    assert proc.returncode == 2 and message in proc.stderr and proc.stdout == ""
+
+
 def test_fft_padding_rule_and_shard_ranges():
     from wavelet_transformer_b200 import _shim, engine
     assert _shim.get_fft_padding() == "pow2"
