@@ -115,6 +115,19 @@ int wtb_cwt(const void *x, int64_t batch, int n0, int nfft, double dt, double dj
  * dj sqrt(dt) / (C_delta psi_0(0)) formed by the caller.  coef: [batch, S, n0] complex. */
 int wtb_icwt(const void *coef, int64_t batch, int S, int n0, const double *scales, double factor,
              int flags, void *x_out, void *stream);
+/* Time- and scale-averaged wavelet power (Torrence & Compo 1998 eqs. 22 and 24; the pycwt sample's
+ * glbl_power and scale_avg) of a batch, without the [batch, S, n0] plane leaving the device.
+ * Transform arguments and kernel dispatch as wtb_cwt (any mother, FP32/FP64, any nfft wtb_cwt takes).
+ * global_out (may be NULL): [batch, S] real, (1/n0) sum_{t<n0} |W[b,s,t]|^2.
+ * band_out   (may be NULL): [batch, n0] real, band_factor * sum_{s=band_lo..band_hi} |W[b,s,t]|^2 / scales[s]
+ *   (band_factor = dj dt / C_delta formed by the caller, as wtb_icwt's factor; the caller may fold a variance in).
+ * Sums are accumulated in double in a fixed order; results do not depend on batch chunking or on
+ * the number of devices wherever wtb_cwt's power plane does not.
+ * WTB_EINVAL: no output requested, band_out given without 0 <= band_lo <= band_hi < S, band_factor not
+ * finite, or WTB_COI_MASK (a masked plane would make every average NaN).  batch == 0 is a no-op. */
+int wtb_cwt_averages(const void *x, int64_t batch, int n0, int nfft, double dt, double dj, double s0, int J,
+                     int mother, double param, int band_lo, int band_hi, double band_factor, int flags,
+                     void *global_out, void *band_out, void *stream);
 
 /* ---- batched pre-processing: replaces standardize_series (src/utils/wavelet_helpers.py:22-57)
  * and pycwt.ar1 (src/cwt.py:106) for batches of series ------------------------------------ */

@@ -92,6 +92,8 @@ _SIGNATURES = {
     "wtb_cwt_axes_mother": ([_i32, _f64, _f64, _f64, _i32, _i32, _f64, _pi, _pd, _pd, _pd], _i32),
     "wtb_cwt": ([_vp, _i64, _i32, _i32, _f64, _f64, _f64, _i32, _i32, _f64, _i32, _vp, _vp, _vp], _i32),
     "wtb_icwt": ([_vp, _i64, _i32, _i32, _pd, _f64, _i32, _vp, _vp], _i32),
+    "wtb_cwt_averages": ([_vp, _i64, _i32, _i32, _f64, _f64, _f64, _i32, _i32, _f64, _i32, _i32, _f64, _i32, _vp, _vp,
+                          _vp], _i32),
     "wtb_cwt_morlet": ([_vp, _i64, _i32, _i32, _f64, _f64, _f64, _i32, _f64, _i32, _vp, _vp, _vp], _i32),
     "wtb_series_prep": ([_vp, _i64, _i32, _i32, _i32, _i32, _i32, _vp, _pd, _vp], _i32),
     "wtb_ratio_planes": ([_vp, _i64, _i32, _i32, _vp, _i64, _i32, _vp, _vp, _vp], _i32),
@@ -252,6 +254,64 @@ def cwt(x, dt, dj, s0, J, mother=MORLET, param=6.0, *, nfft=None, f64=None, want
         power = power[0] if power is not None else None
         coef = coef[0] if coef is not None else None
     return power, coef
+
+
+def _averages_args(band, band_factor, want_global, S):
+    """Validates the arguments of wtb_cwt_averages before any transform runs; returns (band_lo, band_hi)."""
+    if band is None:
+        if not want_global:
+            raise ValueError("cwt_averages: no output requested (band=None and want_global=False)")
+        return 0, 0
+    if len(band) != 2 or any(isinstance(v, (bool, np.bool_)) or not isinstance(v, (int, np.integer)) for v in band):
+        raise ValueError(f"cwt_averages: band must be two scale indices (lo, hi), got {band!r}")
+    lo, hi = int(band[0]), int(band[1])
+    if not 0 <= lo <= hi < S:
+        raise ValueError(f"cwt_averages: band ({lo}, {hi}) must satisfy 0 <= lo <= hi < S = {S}")
+    if not np.isfinite(band_factor):
+        raise ValueError("cwt_averages: band_factor must be finite")
+    return lo, hi
+
+
+def cwt_averages(x, dt, dj, s0, J, mother=MORLET, param=6.0, *, band=None, band_factor=1.0, want_global=True,
+                 nfft=None, f64=None, generic_only=False):
+    """Time- and scale-averaged wavelet power of host data (wtb_cwt_averages, Torrence & Compo 1998 eqs. 22
+    and 24) without the power plane leaving the device.  x: [n0] or [batch, n0].
+    band = (lo, hi): scale indices, inclusive.  Returns (global [batch, S] or None, band [batch, n0] or None)
+    with global = mean_t |W|^2 and band = band_factor * sum_{s=lo..hi} |W_s|^2 / scales[s]; the batch axis
+    is dropped for 1-D input."""
+    f64 = _resolve_f64(f64)
+    rt = _dtype(f64)
+    x2 = np.ascontiguousarray(np.atleast_2d(np.asarray(x)), dtype=rt)
+    batch, n0 = x2.shape
+    Jr, _, _, _ = cwt_axes_mother(n0, dt, dj, s0, J, mother, param)      # host arithmetic only
+    S = Jr + 1
+    lo, hi = _averages_args(band, band_factor, want_global, S)
+    nfft = int(nfft) if nfft else default_nfft(n0)
+    flags = (F64 if f64 else 0) | (GENERIC_ONLY if generic_only else 0)
+    glob = np.empty((batch, S), dtype=rt) if want_global else None
+    bnd = np.empty((batch, n0), dtype=rt) if band is not None else None
+    _check(lib().wtb_cwt_averages(_ptr(x2), batch, n0, nfft, dt, dj, s0, int(J), int(mother), float(param), lo, hi,
+                                  float(band_factor), flags, _ptr(glob), _ptr(bnd), None), "wtb_cwt_averages")
+    if np.ndim(x) == 1:
+        glob = glob[0] if glob is not None else None
+        bnd = bnd[0] if bnd is not None else None
+    return glob, bnd
+
+
+def cwt_averages_device(x_ptr, batch, n0, dt, dj, s0, J, mother, param, global_ptr, band_ptr, *, band=None,
+                        band_factor=1.0, nfft=None, f64=False, stream=0):
+    """Device-resident wtb_cwt_averages: raw device addresses (global_ptr / band_ptr may be 0 for "not
+    wanted"), asynchronous on `stream`."""
+    if bool(band_ptr) != (band is not None):
+        raise ValueError("cwt_averages_device: band_ptr and band are given together")
+    Jr, _, _, _ = cwt_axes_mother(n0, dt, dj, s0, J, mother, param)
+    lo, hi = _averages_args(band, band_factor, bool(global_ptr), Jr + 1)
+    nfft = int(nfft) if nfft else default_nfft(n0)
+    _check(lib().wtb_cwt_averages(_ptr(int(x_ptr)), int(batch), int(n0), nfft, dt, dj, s0, int(J), int(mother),
+                                  float(param), lo, hi, float(band_factor), DEVICE_PTRS | (F64 if f64 else 0),
+                                  _ptr(int(global_ptr)) if global_ptr else None,
+                                  _ptr(int(band_ptr)) if band_ptr else None, C.c_void_p(int(stream))),
+           "wtb_cwt_averages")
 
 
 def icwt(W, scales, factor, *, f64=None):

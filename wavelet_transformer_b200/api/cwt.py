@@ -113,3 +113,54 @@ def run_cwt_batch(cwt_data_list: List[Type[DataForCWT]], normalize: bool = True,
             ratio = power[b] / (np.ones([1, len(d.t_values)]) * signif[:, None])
         out.append(ResultsFromCWT(power[b], period.copy(), ratio, coi.copy()))
     return out
+
+
+@dataclass
+class AveragesFromCWT:
+    """Time- and scale-averaged power of one series with their red-noise significance (the pycwt sample's
+    glbl_power, glbl_signif, scale_avg and scale_avg_signif; Torrence & Compo 1998 eqs. 22-28)."""
+
+    period: npt.NDArray
+    glbl_power: npt.NDArray
+    glbl_signif: npt.NDArray
+    scale_avg: npt.NDArray
+    scale_avg_signif: float
+
+
+def run_cwt_averages(cwt_data_list: List[Type[DataForCWT]], period_band=(2, 8),
+                     significance_level: float = 0.95) -> List[AveragesFromCWT]:
+    """The averages section of the pycwt sample for several equal-length series in one batched call: the
+    global wavelet spectrum (``power.mean(axis=1)``) and the scale-averaged power over the periods
+    ``lo <= period < hi`` (``dj dt / C_delta * sum |W|^2 / s``), both reduced on the device, with
+    ``significance(var, ..., sigma_test=1, dof=n0 - scales)`` and ``sigma_test=2`` over the band's scales.
+    ``var = y.var()`` and ``alpha = ar1(y)`` per series (``ar1`` raises ``Warning`` when it cannot bound the
+    estimate).  Series are transformed as given, as pycwt.cwt does; the module constants DT, DJ, S0 and J drive
+    the transform, as in ``run_cwt_batch``."""
+    if not cwt_data_list:
+        return []
+    mother = wavelet._as_mother(cwt_data_list[0].mother_wavelet)
+    ys = [np.asarray(d.y_values, dtype=float) for d in cwt_data_list]
+    if len({y.size for y in ys}) != 1:
+        raise ValueError("run_cwt_averages takes series of equal length")
+    n0 = ys[0].size
+    _, scales, freqs, _ = wavelet._resolve_s0_J(n0, DT, DJ, S0, J, mother)
+    period = 1 / freqs
+    sel = np.nonzero((period >= period_band[0]) & (period < period_band[1]))[0]
+    if sel.size == 0:
+        raise ValueError(f"no scale has a period in [{period_band[0]}, {period_band[1]})")
+    if mother.cdelta == -1:
+        raise ValueError(f"C_delta is not defined for {mother.name} with these parameters")
+    alphas = [wavelet.ar1(y)[0] for y in ys]
+    kind, param = wavelet._mother_code(mother)
+    glbl, scale_avg = _shim.cwt_averages(np.stack(ys), DT, DJ, S0, int(J), kind, param,
+                                         band=(int(sel[0]), int(sel[-1])), band_factor=DJ * DT / mother.cdelta,
+                                         f64=True)
+    out = []
+    for b, (y, alpha) in enumerate(zip(ys, alphas)):
+        var = y.var()
+        glbl_signif, _ = wavelet.significance(var, DT, scales, 1, alpha, significance_level=significance_level,
+                                              dof=n0 - scales, wavelet=mother)
+        avg_signif, _ = wavelet.significance(var, DT, scales, 2, alpha, significance_level=significance_level,
+                                             dof=[scales[sel[0]], scales[sel[-1]]], wavelet=mother)
+        out.append(AveragesFromCWT(period.copy(), glbl[b], glbl_signif, scale_avg[b], float(avg_signif)))
+    return out

@@ -124,9 +124,10 @@ __global__ void k_cwt_rows(const cplx<T> *__restrict__ xhat, int n0, FftPlan<T> 
   }
 }
 
+// also the first pass of wtb_cwt_averages (averages.cu)
 template <typename T>
-static int cwt_device(const T *d_x, int64_t batch, int n0, int N, double dt, const Axes &ax,
-                      const Mother &mo, int flags, T *d_power, cplx<T> *d_coef, cudaStream_t st) {
+int cwt_device(const T *d_x, int64_t batch, int n0, int N, double dt, const Axes &ax,
+               const Mother &mo, int flags, T *d_power, cplx<T> *d_coef, cudaStream_t st) {
   const int S = ax.J + 1;
   const double f0 = mo.kind == WTB_MORLET ? mo.param : 0.0;
   if (mo.kind == WTB_MORLET && sizeof(T) == 4 && d_coef == nullptr && d_power != nullptr &&
@@ -202,6 +203,10 @@ static int cwt_device(const T *d_x, int64_t batch, int n0, int N, double dt, con
   WTB_LAUNCH_CHECK();
   return WTB_OK;
 }
+template int cwt_device<float>(const float *, int64_t, int, int, double, const Axes &, const Mother &, int, float *,
+                               float2 *, cudaStream_t);
+template int cwt_device<double>(const double *, int64_t, int, int, double, const Axes &, const Mother &, int, double *,
+                                double2 *, cudaStream_t);
 
 static thread_local bool g_in_shard = false;   // set on a pool worker while it runs its block
 

@@ -55,6 +55,36 @@ def cwt_power_resident(x, power, dt, dj, s0, J, f0=6.0, generic_only=False):
     return power
 
 
+def cwt_averages_resident(x, global_out, band_out, dt, dj, s0, J, mother=_shim.MORLET, param=6.0, band=None,
+                          band_factor=1.0, nfft=None):
+    """Time- and scale-averaged wavelet power of a device-resident batch (wtb_cwt_averages).
+
+    x: torch CUDA float32/float64 tensor [batch, n0].  global_out: preallocated [batch, J+1] tensor of the same
+    dtype, or None; band_out: [batch, n0] or None, given together with ``band = (lo, hi)`` (scale indices,
+    inclusive).  global = mean_t |W|^2, band = band_factor * sum_{s=lo..hi} |W_s|^2 / scales[s].  Runs on the
+    device that owns x, enqueued on torch's current stream of that device; the power plane never exists
+    outside the library's scratch.  Returns (global_out, band_out)."""
+    import torch
+    outs = [t for t in (global_out, band_out) if t is not None]
+    if not (x.is_cuda and x.is_contiguous() and all(t.is_cuda and t.is_contiguous() for t in outs)):
+        raise ValueError("x and the outputs must be contiguous CUDA tensors")
+    if any(t.device != x.device for t in outs):
+        raise ValueError("x and the outputs must live on the same device")
+    if x.dtype not in (torch.float32, torch.float64) or any(t.dtype != x.dtype for t in outs):
+        raise ValueError("x and the outputs must all be float32 or all float64")
+    batch, n0 = x.shape
+    if global_out is not None and tuple(global_out.shape) != (batch, int(J) + 1):
+        raise ValueError(f"global_out must have shape {(batch, int(J) + 1)}")
+    if band_out is not None and tuple(band_out.shape) != (batch, n0):
+        raise ValueError(f"band_out must have shape {(batch, n0)}")
+    _shim.cwt_averages_device(x.data_ptr(), batch, n0, dt, dj, s0, int(J), mother, param,
+                              0 if global_out is None else global_out.data_ptr(),
+                              0 if band_out is None else band_out.data_ptr(), band=band, band_factor=band_factor,
+                              nfft=nfft, f64=x.dtype == torch.float64,
+                              stream=torch.cuda.current_stream(x.device).cuda_stream)
+    return global_out, band_out
+
+
 def cwt_batch_resident(x, dt, dj, s0, J, f0=6.0, detrend=True, remove_mean=False, standardize=True,
                        significance_level=None):
     """Device-resident batch version of the reference's CWT request (src/wavelet_plots.py:32

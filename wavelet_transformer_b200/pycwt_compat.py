@@ -213,8 +213,9 @@ def _chi2_ppf(level, dof):
 def significance(signal, dt, scales, sigma_test=0, alpha=None, significance_level=0.95, dof=-1,
                  wavelet="morlet"):
     """Red-noise significance levels (Torrence & Compo 1998 sec. 4); returns
-    ``(signif, fft_theor)``.  sigma_test 0 (no smoothing) and 1 (time average).  Any mother
-    wavelet: only flambda, dofmin and gamma enter."""
+    ``(signif, fft_theor)``.  sigma_test 0 (no smoothing), 1 (time average) and 2 (scale average over
+    ``dof = [s1, s2]``, eqs. 25-28: returns the scale-averaged ``fft_theor``).  Any mother wavelet:
+    flambda, dofmin and gamma enter, and for sigma_test 2 cdelta and deltaj0 as well."""
     wavelet = _as_mother(wavelet)
     try:
         n0 = len(signal)
@@ -236,8 +237,25 @@ def significance(signal, dt, scales, sigma_test=0, alpha=None, significance_leve
         dofv = dofmin * np.sqrt(1 + (dofv * dt / wavelet.gamma / scales) ** 2)
         dofv = np.maximum(dofv, dofmin)
         signif = fft_theor * chi2.ppf(significance_level, dofv) / dofv
+    elif sigma_test == 2:
+        from scipy.stats import chi2
+        if np.ndim(dof) != 1 or len(dof) != 2:
+            raise Exception("DOF must be set to [s1, s2], the range of scale-averages")
+        if wavelet.cdelta == -1:
+            raise ValueError(f"Cdelta and dj0 not defined for {wavelet.name} with these parameters")
+        s1, s2 = float(dof[0]), float(dof[1])
+        sel = (scales >= s1) & (scales <= s2)
+        navg = int(sel.sum())
+        if navg == 0:
+            raise ValueError(f"No valid scales between {s1} and {s2}.")
+        dj = np.log2(scales[1] / scales[0])
+        savg = 1 / np.sum(1 / scales[sel])                                         # eq. 25
+        smid = np.exp((np.log(s1) + np.log(s2)) / 2)
+        dofv = dofmin * navg * savg / smid * np.sqrt(1 + (navg * dj / wavelet.deltaj0) ** 2)   # eq. 28
+        fft_theor = savg * np.sum(fft_theor[sel] / scales[sel])                    # eq. 27
+        signif = dj * dt / (wavelet.cdelta * savg) * fft_theor * chi2.ppf(significance_level, dofv) / dofv  # eq. 26
     else:
-        raise NotImplementedError("significance: sigma_test must be 0 or 1")
+        raise NotImplementedError("significance: sigma_test must be 0, 1 or 2")
     return signif, fft_theor
 
 
