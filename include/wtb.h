@@ -92,7 +92,9 @@ int wtb_cwt_axes(int n0, double dt, double dj, double s0, int J, double f0,
 /* Batched Morlet CWT.  x: [batch, n0] real.  nfft: FFT length >= n0.  pycwt's scipy.fftpack
  * path (the reference's pip / uv install) pads to 2^ceil(log2 n0); its mkl_fft path (the conda
  * install, environment.yml:126) transforms at nfft = n0.  Powers of two run the FFT kernels
- * (fused FP32 fast paths at 512 / 1024 / 2048 / 4096); any other length runs Bluestein's chirp-z
+ * (fused FP32 fast paths at 512 / 1024 / 2048 / 4096; one CTA per transform up to 8192 in FP32,
+ * 4096 in FP64; longer powers of two return WTB_EUNSUPPORTED here and run in wtb_cwt, below); any other
+ * length runs Bluestein's chirp-z
  * transform over the next power of two >= 2 nfft - 1 in the generic kernels (nfft <= 2048 in
  * FP64, <= 4096 in FP32).  Outputs (either
  * may be NULL): power_out [batch, S, n0] real = |W|^2; coef_out [batch, S, n0]
@@ -105,7 +107,9 @@ int wtb_cwt_morlet(const void *x, int64_t batch, int n0, int nfft,
  * Paul and DOG objects next to Morlet): psi_ft is pi^-1/4 exp(-(sw-f0)^2/2) for Morlet,
  * 2^m/sqrt(m (2m-1)!) (sw)^m exp(-sw) H(sw) for Paul, -i^m/sqrt(Gamma(m+1/2)) (sw)^m exp(-(sw)^2/2)
  * for DOG; flambda = 4pi/(f0+sqrt(2+f0^2)), 4pi/(2m+1), 2pi/sqrt(m+1/2).  Morlet goes through the
- * same code as wtb_cwt_morlet (including its fused FP32 kernel). */
+ * same code as wtb_cwt_morlet (including its fused FP32 kernel).  wtb_cwt also takes the powers of two
+ * past one CTA's shared memory: nfft from 16384 in FP32, 8192 in FP64, up to 2^22 = 4194304, as
+ * four-step transforms over several CTAs; larger powers of two return WTB_EUNSUPPORTED. */
 int wtb_cwt_axes_mother(int n0, double dt, double dj, double s0, int J, int mother, double param,
                         int *J_out, double *scales, double *freqs, double *coi);
 int wtb_cwt(const void *x, int64_t batch, int n0, int nfft, double dt, double dj, double s0, int J,

@@ -331,8 +331,8 @@ def icwt(W, scales, factor, *, f64=None):
 
 def cwt_morlet(x, dt, dj, s0, J, f0=6.0, *, nfft=None, f64=None, want_power=True, want_coef=False,
                coi_mask=False, generic_only=False):
-    """Batched Morlet CWT of host data.  x: [n0] or [batch, n0].
-    Returns (power or None, coef or None) with shapes [batch, S, n0] (batch axis
+    """Batched Morlet CWT of host data (wtb_cwt_morlet: one-CTA transform lengths; `cwt` takes longer series).
+    x: [n0] or [batch, n0].  Returns (power or None, coef or None) with shapes [batch, S, n0] (batch axis
     dropped for 1-D input); dtype float32/complex64 or float64/complex128."""
     f64 = _resolve_f64(f64)
     rt = _dtype(f64)
@@ -354,11 +354,12 @@ def cwt_morlet(x, dt, dj, s0, J, f0=6.0, *, nfft=None, f64=None, want_power=True
 
 def cwt_power_device(x_ptr, batch, n0, dt, dj, s0, J, f0, power_ptr, *, nfft=None, f64=False,
                      stream=0, generic_only=False):
-    """Device-resident variant: raw device addresses, asynchronous on `stream`."""
+    """Device-resident Morlet CWT power (wtb_cwt, every transform length it takes): raw device addresses,
+    asynchronous on `stream`."""
     nfft = int(nfft) if nfft else default_nfft(n0)
     flags = DEVICE_PTRS | (F64 if f64 else 0) | (GENERIC_ONLY if generic_only else 0)
-    _check(lib().wtb_cwt_morlet(_ptr(int(x_ptr)), batch, n0, nfft, dt, dj, s0, int(J), f0, flags,
-                                _ptr(int(power_ptr)), None, C.c_void_p(int(stream))), "wtb_cwt_morlet")
+    _check(lib().wtb_cwt(_ptr(int(x_ptr)), batch, n0, nfft, dt, dj, s0, int(J), MORLET, float(f0), flags,
+                         _ptr(int(power_ptr)), None, C.c_void_p(int(stream))), "wtb_cwt")
 
 
 def series_prep(x, *, detrend=True, remove_mean=False, standardize=True, f64=None, want_y=True, want_ar1=True):

@@ -71,7 +71,7 @@ def run_cwt(cwt_data: Type[DataForCWT], normalize: bool = True, standardize: boo
         # |W|^2 straight from the fused kernel: no complex plane over PCIe, no host abs()**2, and
         # none of the side outputs of pycwt.cwt the reference discards (src/cwt.py:109)
         _, scales, freqs, coi = wavelet._resolve_s0_J(np.size(signal), DT, DJ, S0, J, mother)
-        power, _ = _shim.cwt_morlet(np.asarray(signal, dtype=float), DT, DJ, S0, int(J), mother.f0)
+        power, _ = _shim.cwt(np.asarray(signal, dtype=float), DT, DJ, S0, int(J), _shim.MORLET, mother.f0)
         power = np.asarray(power, dtype=float)
     else:
         wave, scales, freqs, coi, _, _ = wavelet.cwt(signal, DT, DJ, S0, J, mother)
@@ -101,7 +101,7 @@ def run_cwt_batch(cwt_data_list: List[Type[DataForCWT]], normalize: bool = True,
     signals = np.stack([standardize_series(y, **kwargs) if standardize else y for y in ys])
     n0 = signals.shape[1]
     _, scales, freqs, coi = wavelet._resolve_s0_J(n0, DT, DJ, S0, J, mother)
-    power, _ = _shim.cwt_morlet(signals, DT, DJ, S0, int(J), mother.f0, f64=True)
+    power, _ = _shim.cwt(signals, DT, DJ, S0, int(J), _shim.MORLET, mother.f0, f64=True)
     power = np.asarray(power, dtype=float).reshape(len(ys), scales.size, n0)
     period = 1 / freqs
     out = []

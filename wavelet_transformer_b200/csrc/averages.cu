@@ -12,13 +12,15 @@ namespace wtb {
 template <typename T>
 int cwt_device(const T *d_x, int64_t batch, int n0, int N, double dt, const Axes &ax, const Mother &mo, int flags,
                T *d_power, cplx<T> *d_coef, cudaStream_t st);
+bool cwt_long_takes(int N, size_t elem);   // cwt_long.cu
 
 constexpr int kAvgThreads = 256;
 
-// One CTA per series.  global: warp w sums rows w, w + 8, ...; each lane adds t = lane, lane + 32, ... in ascending
-// order, then a fixed xor-shuffle tree combines the lanes.  band: thread t adds rows band_lo .. band_hi in ascending
-// order.  Both read along t (coalesced) and accumulate in double; the order depends on n0 and S only, never on the
-// batch, the chunk or the device, and there are no atomics.
+// Grid (series, part).  global: warp w of part y sums rows 8 (y + Y i) + w, i = 0, 1, ...; each lane adds
+// t = lane, lane + 32, ... in ascending order, then a fixed xor-shuffle tree combines the lanes.  band: thread t
+// of part y adds rows band_lo .. band_hi in ascending order for t = 256 (y + Y i) + threadIdx.x.  Both read along
+// t (coalesced) and accumulate in double; every output is summed by one warp or one thread in an order that
+// depends on n0 and S only, never on Y, the batch, the chunk or the device, and there are no atomics.
 template <typename T>
 __global__ void __launch_bounds__(kAvgThreads)
 k_cwt_averages(const T *__restrict__ power, int S, int n0, const double *__restrict__ inv_scales, int band_lo,
@@ -27,7 +29,7 @@ k_cwt_averages(const T *__restrict__ power, int S, int n0, const double *__restr
   const T *p = power + b * (int64_t)S * n0;
   if (global) {
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    for (int s = warp; s < S; s += kAvgThreads / 32) {
+    for (int s = blockIdx.y * (kAvgThreads / 32) + warp; s < S; s += gridDim.y * (kAvgThreads / 32)) {
       const T *row = p + (int64_t)s * n0;
       double acc = 0.0;
 #pragma unroll 4
@@ -38,7 +40,7 @@ k_cwt_averages(const T *__restrict__ power, int S, int n0, const double *__restr
     }
   }
   if (band) {
-    for (int t = threadIdx.x; t < n0; t += kAvgThreads) {
+    for (int t = blockIdx.y * kAvgThreads + threadIdx.x; t < n0; t += gridDim.y * kAvgThreads) {
       double acc = 0.0;
       for (int s = band_lo; s <= band_hi; ++s) acc += (double)p[(int64_t)s * n0 + t] * inv_scales[s];
       band[b * (int64_t)n0 + t] = T(band_factor * acc);
@@ -46,12 +48,23 @@ k_cwt_averages(const T *__restrict__ power, int S, int n0, const double *__restr
   }
 }
 
+// Parts per series: one when the batch alone fills the machine (8 CTAs per SM), otherwise enough to, but no
+// more than the work has (one row group of 8 rows or one tile of 256 t per part).
+static unsigned averages_parts(int64_t nb, int S, int n0) {
+  const int64_t work = std::max<int64_t>((S + kAvgThreads / 32 - 1) / (kAvgThreads / 32), (n0 + kAvgThreads - 1) / kAvgThreads);
+  const int64_t want = (8LL * sm_count() + nb - 1) / nb;
+  return (unsigned)std::max<int64_t>(1, std::min(work, want));
+}
+
 // The chunk rule, in one place: series per chunk = the number whose power rows fit a 1 GiB budget (as cwt_entry's
 // staging), but at least 16 warps on every SM for the warp-per-series nfft-1024 kernel (148 x 16 = 2368 series on a
-// B200), rounded down to an even count so the two-series kernels pair the same neighbours in every chunk.
-static int64_t averages_chunk_rows(int64_t batch, int S, int n0, size_t elem) {
-  const int64_t fill = 16LL * sm_count();
+// B200), rounded down to an even count so the two-series kernels pair the same neighbours in every chunk.  Lengths
+// the long transforms serve (cwt_long.cu) have no such kernel and a plane of up to GBs per series: there the
+// budget alone counts, and a series whose plane exceeds it is a chunk of its own.
+static int64_t averages_chunk_rows(int64_t batch, int S, int n0, int N, size_t elem) {
   const int64_t by_bytes = (int64_t)((size_t(1) << 30) / (elem * (size_t)S * n0));
+  if (cwt_long_takes(N, elem)) return std::min(batch, std::max<int64_t>(1, by_bytes));
+  const int64_t fill = 16LL * sm_count();
   return std::min(batch, std::max(fill, by_bytes) & ~int64_t(1));
 }
 
@@ -76,7 +89,7 @@ static int averages_entry(const void *x, int64_t batch, int n0, int N, double dt
   }
   // The power chunk lives in the staging slot: cwt_device takes the arena (and its fast paths the parameter
   // buffer), and a slot that grows is moved, so a second user of either in this call would lose its data.
-  const int64_t rows = averages_chunk_rows(batch, S, n0, sizeof(T));
+  const int64_t rows = averages_chunk_rows(batch, S, n0, N, sizeof(T));
   auto al = [](size_t b) { return (b + 255) / 256 * 256; };
   const size_t b_inv = al(sizeof(double) * S), b_pow = al(sizeof(T) * (size_t)rows * S * n0);
   const size_t b_x = dev ? 0 : al(sizeof(T) * (size_t)rows * n0);
@@ -105,7 +118,7 @@ static int averages_entry(const void *x, int64_t batch, int n0, int N, double dt
       bo = band_out ? d_b : nullptr;
     }
     WTB_TRY(cwt_device<T>(xin, nb, n0, N, dt, ax, mo, flags, d_pow, nullptr, st));
-    k_cwt_averages<T><<<(unsigned)nb, kAvgThreads, 0, st>>>(d_pow, S, n0, d_inv, band_lo, band_hi, band_factor, g, bo);
+    k_cwt_averages<T><<<dim3((unsigned)nb, averages_parts(nb, S, n0)), kAvgThreads, 0, st>>>(d_pow, S, n0, d_inv, band_lo, band_hi, band_factor, g, bo);
     WTB_LAUNCH_CHECK();
     if (!dev) {
       if (global_out) WTB_TRY(copy_to_host((T *)global_out + b0 * S, d_g, sizeof(T) * nb * S, st));

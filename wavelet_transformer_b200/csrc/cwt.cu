@@ -25,6 +25,12 @@ int cwt_rows_4096_try(const float2 *d_xhat, int64_t batch, int n0, int N, double
 // implemented in wct_fast.cu: forward FFTs with the radix-16 register kernel (FP32, N = 4096); 1 = not covered
 int fwd_fft_4096_try(const float *d_y, int64_t nseries, int n0, int N, float2 *d_xhat, cudaStream_t st);
 
+// implemented in cwt_long.cu: four-step transforms for the powers of two past one CTA's shared memory
+bool cwt_long_takes(int N, size_t elem);
+template <typename T>
+int cwt_long(const T *d_x, int64_t batch, int n0, int N, double dt, const Axes &ax, const Mother &mo, int flags,
+             T *d_power, cplx<T> *d_coef, cudaStream_t st);
+
 // Forward FFT (N = 2048, FP32) for k_cwt_pair_2048: the positive half of the spectrum leaves in the layout
 // that kernel's warps load with one 16-byte access per packed pair -- per series 8 KB at the start of its
 // xhat row: float4 [parity h][m < 8][lane] = (Re X^[k0], Re X^[k1], Im X^[k0], Im X^[k1]),
@@ -80,30 +86,9 @@ __global__ void k_cwt_rows(const cplx<T> *__restrict__ xhat, int n0, FftPlan<T> 
     const T s_over_dt = T(sc / dt);
     // (s * ftfreqs[1] * N)^0.5 * pi^-0.25, times 1/N of the inverse transform
     const T norm = T(sqrt(2.0 * kPi * sc / dt) * kPiM14 / double(N));
-    if (mother == WTB_MORLET) {
-      for (int k = threadIdx.x; k < N; k += blockDim.x) {
-        const T d = morlet_daughter<T>(k, N, s_over_dt, norm, T(f0));
-        cplx<T> v = xh[k];
-        a[k] = mk<T>(v.x * d, v.y * d);
-      }
-    } else {
-      // Paul: (sw)^m exp(-sw) H(sw);  DOG: (sw)^m exp(-(sw)^2/2);  times conj(prefactor)
-      const T nrm = T(sqrt(2.0 * kPi * sc / dt) / double(N));
-      for (int k = threadIdx.x; k < N; k += blockDim.x) {
-        const int kk = (k < (N + 1) / 2) ? k : k - N;
-        const T z = s_over_dt * (T(2.0 * kPi) * T(kk) / T(N));
-        // z^m e^{-z} (Paul) and z^m e^{-z^2/2} (DOG) evaluated as one exponential: z^m alone
-        // overflows FP32 for large orders and scales while the product is tiny (inf * 0 = NaN)
-        const T az = fabs(z);
-        const T lz = T(order) * log(az);                      // -inf at z = 0: the daughter vanishes (m >= 1)
-        const T sgn = (z < T(0) && (order & 1)) ? T(-1) : T(1);
-        const T g = mother == WTB_PAUL ? (z > T(0) ? dev_exp<T>(lz - z) : T(0))
-                                       : (az > T(0) ? sgn * dev_exp<T>(lz - T(0.5) * z * z) : T(0));
-        const T dr = nrm * pre_re * g, di = nrm * pre_im * g;
-        cplx<T> v = xh[k];
-        a[k] = mk<T>(v.x * dr - v.y * di, v.x * di + v.y * dr);
-      }
-    }
+    const T nrm = T(sqrt(2.0 * kPi * sc / dt) / double(N));
+    for (int k = threadIdx.x; k < N; k += blockDim.x)
+      a[k] = daughter_mul<T>(xh[k], k, N, mother, order, s_over_dt, norm, nrm, T(f0), pre_re, pre_im);
     __syncthreads();
     cplx<T> *r = plan_fft<T, +1>(a, b, plan);
     const int64_t obase = (row * S + s) * (int64_t)n0;
@@ -135,6 +120,7 @@ int cwt_device(const T *d_x, int64_t batch, int n0, int N, double dt, const Axes
     int rc = cwt_fast_try((const float *)d_x, batch, n0, N, dt, ax, f0, flags, (float *)d_power, st);
     if (rc != 1) return rc;
   }
+  if (cwt_long_takes(N, sizeof(T))) return cwt_long<T>(d_x, batch, n0, N, dt, ax, mo, flags, d_power, d_coef, st);
   FftPlan<T> plan;
   WTB_TRY(make_plan<T>(N, &plan));
   const size_t smem = 2 * sizeof(cplx<T>) * (size_t)plan.M;
@@ -277,9 +263,15 @@ extern "C" int wtb_cwt(const void *x, int64_t batch, int n0, int nfft, double dt
   return cwt_entry<float>(x, batch, n0, nfft, dt, ax, mo, flags, power_out, coef_out, st);
 }
 
+// The Morlet entry point keeps the transform lengths it has always served: one CTA per transform (powers of two
+// up to 8192 in FP32, 4096 in FP64).  Longer series go through wtb_cwt, which takes them up to 2^22.
 extern "C" int wtb_cwt_morlet(const void *x, int64_t batch, int n0, int nfft, double dt, double dj,
                               double s0, int J, double f0, int flags, void *power_out,
                               void *coef_out, void *stream) {
+  const bool f64 = flags & WTB_F64;
+  WTB_REQUIRE(!cwt_long_takes(nfft, f64 ? sizeof(double) : sizeof(float)), WTB_EUNSUPPORTED,
+              "wtb_cwt_morlet: nfft=%d is past the one-CTA transform (a power of two up to %d for %s); wtb_cwt with "
+              "WTB_MORLET takes powers of two up to 2^22", nfft, f64 ? 4096 : 8192, f64 ? "double" : "float");
   return wtb_cwt(x, batch, n0, nfft, dt, dj, s0, J, WTB_MORLET, f0, flags, power_out, coef_out, stream);
 }
 

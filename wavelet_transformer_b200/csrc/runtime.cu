@@ -422,6 +422,7 @@ template int bluestein_tables<float>(int, int, const cplx<float> **, const cplx<
 template int bluestein_tables<double>(int, int, const cplx<double> **, const cplx<double> **);
 
 void wct_fast_release();  // wct_fast.cu: the radix-16 twiddle tables
+void cwt_long_release();  // cwt_long.cu: the inter-pass twiddle tables
 void pool_shutdown();      // multi.cu
 
 static void free_tables() {
@@ -523,6 +524,7 @@ void wtb_shutdown(void) {
   }
   free_tables();
   wct_fast_release();
+  cwt_long_release();
   cudaSetDevice(cur);
   std::lock_guard<std::mutex> lk(g_mu);
   g_default_device = -1;

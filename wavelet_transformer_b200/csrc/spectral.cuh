@@ -25,6 +25,29 @@ __device__ __forceinline__ T morlet_daughter(int k, int N, T s_over_dt, T norm, 
   return norm * dev_exp<T>(T(-0.5) * z * z);
 }
 
+// X^[k] times the conjugated daughter of one scale at bin k of an N-point grid (k_cwt_rows, and the first pass
+// of the long transforms in cwt_long.cu).  Morlet: norm = (2 pi s / dt)^0.5 pi^-1/4 / N.  Paul: (sw)^m exp(-sw)
+// H(sw); DOG: (sw)^m exp(-(sw)^2/2); both times nrm = (2 pi s / dt)^0.5 / N and conj(prefactor) = pre.
+template <typename T>
+__device__ __forceinline__ cplx<T> daughter_mul(cplx<T> v, int k, int N, int mother, int order, T s_over_dt, T norm,
+                                                T nrm, T f0, T pre_re, T pre_im) {
+  if (mother == WTB_MORLET) {
+    const T d = morlet_daughter<T>(k, N, s_over_dt, norm, f0);
+    return mk<T>(v.x * d, v.y * d);
+  }
+  const int kk = (k < (N + 1) / 2) ? k : k - N;
+  const T z = s_over_dt * (T(2.0 * kPi) * T(kk) / T(N));
+  // z^m e^{-z} (Paul) and z^m e^{-z^2/2} (DOG) evaluated as one exponential: z^m alone
+  // overflows FP32 for large orders and scales while the product is tiny (inf * 0 = NaN)
+  const T az = fabs(z);
+  const T lz = T(order) * log(az);                      // -inf at z = 0: the daughter vanishes (m >= 1)
+  const T sgn = (z < T(0) && (order & 1)) ? T(-1) : T(1);
+  const T g = mother == WTB_PAUL ? (z > T(0) ? dev_exp<T>(lz - z) : T(0))
+                                 : (az > T(0) ? sgn * dev_exp<T>(lz - T(0.5) * z * z) : T(0));
+  const T dr = nrm * pre_re * g, di = nrm * pre_im * g;
+  return mk<T>(v.x * dr - v.y * di, v.x * di + v.y * dr);
+}
+
 // Forward FFT of zero-padded real rows: xhat[row, k], k in [0, plan.n).  smem 2 * plan.M complex.
 template <typename T>
 __global__ void k_fwd_fft(const T *__restrict__ x, int n0, FftPlan<T> plan, cplx<T> *__restrict__ xhat) {
