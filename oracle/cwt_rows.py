@@ -12,8 +12,8 @@ maximum and are barely checked by it.  This module holds
 * ``resolved_rows``: the rows whose daughter band holds at least two bins below the Nyquist
   frequency and whose peak lies below it.  The other rows hold only the daughter's tail, which
   the kernels' one-sided band cut drops by design (DESIGN section 2), so they keep the plane gate;
-* a replica of the host row rules of ``cwt_fast_try`` (nfft 1024 and the two-series nfft 512),
-  ``cwt_dif_try`` (nfft 2048 / 4096) and ``fill_rows`` (``k_cwt_rows_4096`` and the coherence
+* a replica of the host row rules of ``row_params`` in ``cwt_fast.cu`` (nfft 1024 and the two-series
+  nfft 512, nfft 2048 / 4096) and ``fill_rows`` (``k_cwt_rows_4096`` and the coherence
   kernels), so that tests can prove which branches of the pruned transforms their shapes reach.
 """
 
@@ -21,7 +21,7 @@ import math
 
 import numpy as np
 
-ZCUT_F32 = float(np.float32(5.3))    # kZCut of cwt_fast.cu (a float constant, widened to double)
+ZCUT_F32 = float(np.float32(5.3))    # kZCut of cwt_paths.cuh (a float constant, widened to double)
 ZCUT_F64 = 5.3                       # fill_rows of wct_fast.cu (a double literal)
 ROW_FLOOR = 1e-5
 
@@ -74,7 +74,7 @@ def _ilog2(n):
 
 
 def fast_rows(nfft, dt, dj, s0, J, f0=6.0):
-    """(multi, L) per row as cwt_fast_try fills RowParam for k_cwt_fast_1024 (nfft 1024) and its
+    """(multi, L) per row as row_params fills RowParam for k_cwt_fast_1024 (nfft 1024) and its
     two-series HALF variant (nfft 512: 1024-point a and band edge, one bin further out)."""
     assert nfft in (512, 1024)
     half = nfft == 512
@@ -90,7 +90,7 @@ def fast_rows(nfft, dt, dj, s0, J, f0=6.0):
 
 
 def dif_rows(nfft, dt, dj, s0, J, f0=6.0):
-    """(multi, L) per row as cwt_dif_try fills RowParam for k_cwt_dif<D>, D = nfft / 1024: a warp
+    """(multi, L) per row as row_params fills RowParam for k_cwt_dif<D>, D = nfft / 1024: a warp
     transforms the bins of one residue mod D, j = k / D <= jhi.  L == 1 rows (either pass kind)
     take the two-input DFT."""
     assert nfft in (2048, 4096)

@@ -13,7 +13,7 @@ TEST INFRASTRUCTURE ONLY (see oracle/__init__.py).
   sample may sit in another bin than the reference's only if the reference puts
   it within ``delta`` of that bin edge.
 * ``direct_split``: the rule by which the FP32 nfft-4096 coherence pipeline
-  (``wct_fast.cu``, ``fill_rows`` and ``wct_fast_try``) hands its largest
+  (``wct_fast.cu``, ``fill_rows`` and ``wct_fast``) hands its largest
   scales to the direct band-limited kernel, so tests can choose and assert the
   band shapes they exercise.
 """

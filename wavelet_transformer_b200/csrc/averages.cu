@@ -5,14 +5,10 @@
 // Two passes per chunk of series: cwt_device (cwt.cu, every kernel and dispatch rule of wtb_cwt) writes the power
 // rows into device scratch, then k_cwt_averages reads them once and writes both reductions.  Only S + n0 values per
 // series leave the device.
+#include "cwt_paths.cuh"
 #include "spectral.cuh"
 
 namespace wtb {
-
-template <typename T>
-int cwt_device(const T *d_x, int64_t batch, int n0, int N, double dt, const Axes &ax, const Mother &mo, int flags,
-               T *d_power, cplx<T> *d_coef, cudaStream_t st);
-bool cwt_long_takes(int N, size_t elem);   // cwt_long.cu
 
 constexpr int kAvgThreads = 256;
 

@@ -1,69 +1,12 @@
 // Batched CWT (pycwt.cwt, src/cwt.py:110-114 of the reference), Morlet unless stated:
 //   X = fft(x, nfft);  W[s,:] = ifft(X * sqrt(2*pi*s/dt) * pi^-1/4 * exp(-(s*w-f0)^2/2));
 //   power = |W|^2, truncated to the first n0 samples.
-// Generic kernels (any pow2 nfft, float/double) live here; the FP32 fast path
-// for the headline shape is in cwt_fast.cu and is tried first.
+// Generic kernels (any pow2 nfft, float/double) live here; cwt_plan picks them or one of
+// the FP32 fast paths (cwt_fast.cu, wct_fast.cu) or the long transforms (cwt_long.cu).
+#include "cwt_paths.cuh"
 #include "spectral.cuh"
 
 namespace wtb {
-
-// implemented in cwt_fast.cu; returns 1 when the shape is not covered
-int cwt_fast_try(const float *d_x, int64_t batch, int n0, int nfft, double dt, const Axes &ax,
-                 double f0, int flags, float *d_power, cudaStream_t st);
-
-// implemented in cwt_fast.cu (two / four warps per row for nfft = 2048 / 4096, spectra in group layout); 1 = not covered
-int cwt_dif_try(const float2 *d_layout, int64_t stride, int64_t batch, int n0, int nfft, double dt, const Axes &ax,
-                double f0, int flags, float *d_power, cudaStream_t st);
-
-// implemented in cwt_fast.cu: the shape runs those kernels, which read the spectra in group layout
-bool cwt_dif_covers(int64_t batch, int n0, int nfft, int S, double f0);
-
-// implemented in wct_fast.cu (register-FFT rows for nfft = 4096); returns 1 when not covered
-int cwt_rows_4096_try(const float2 *d_xhat, int64_t batch, int n0, int N, double dt, const Axes &ax, double f0,
-                      int flags, float *d_power, float2 *d_coef, cudaStream_t st);
-
-// implemented in wct_fast.cu: forward FFTs with the radix-16 register kernel (FP32, N = 4096); 1 = not covered
-int fwd_fft_4096_try(const float *d_y, int64_t nseries, int n0, int N, float2 *d_xhat, cudaStream_t st);
-
-// implemented in cwt_long.cu: four-step transforms for the powers of two past one CTA's shared memory
-bool cwt_long_takes(int N, size_t elem);
-template <typename T>
-int cwt_long(const T *d_x, int64_t batch, int n0, int N, double dt, const Axes &ax, const Mother &mo, int flags,
-             T *d_power, cplx<T> *d_coef, cudaStream_t st);
-
-// Forward FFT (N = 2048, FP32) for k_cwt_pair_2048: the positive half of the spectrum leaves in the layout
-// that kernel's warps load with one 16-byte access per packed pair -- per series 8 KB at the start of its
-// xhat row: float4 [parity h][m < 8][lane] = (Re X^[k0], Re X^[k1], Im X^[k0], Im X^[k1]),
-// k0 = 2 (lane + 64 m) + h, k1 = k0 + 64.
-__global__ void k_fwd_fft_pair2048(const float *__restrict__ x, int n0, FftPlan<float> plan, float2 *__restrict__ xhat) {
-  extern __shared__ __align__(16) unsigned char smem_raw[];
-  float2 *a = reinterpret_cast<float2 *>(smem_raw);
-  float2 *b = a + plan.M;
-  const int N = plan.n;
-  const int64_t row = blockIdx.x;
-  const float *xr = x + row * n0;
-  for (int t = threadIdx.x; t < N; t += blockDim.x) a[t] = make_float2(t < n0 ? xr[t] : 0.0f, 0.0f);
-  __syncthreads();
-  const float2 *r = plan_fft<float, -1>(a, b, plan);
-  float4 *o = reinterpret_cast<float4 *>(xhat + row * N);
-  for (int i = threadIdx.x; i < 2 * 8 * 32; i += blockDim.x) {
-    const int lane = i & 31, m = (i >> 5) & 7, h = i >> 8;
-    const float2 v0 = r[2 * (lane + 64 * m) + h], v1 = r[2 * (lane + 64 * m) + h + 64];
-    o[i] = make_float4(v0.x, v1.x, v0.y, v1.y);
-  }
-}
-
-// The same layout for N = 4096 (four warps per row: k0 = 4 (lane + 64 m) + r, k1 = k0 + 128, r < 4; 16 KB), built from
-// the natural-order spectrum of the radix-16 forward kernel into the unused negative-frequency half of the row.
-__global__ void k_dif_layout4096(float2 *__restrict__ xhat) {
-  const float2 *r = xhat + (int64_t)blockIdx.x * 4096;
-  float4 *o = reinterpret_cast<float4 *>(xhat + (int64_t)blockIdx.x * 4096 + 2048);
-  for (int i = threadIdx.x; i < 4 * 8 * 32; i += blockDim.x) {
-    const int lane = i & 31, m = (i >> 5) & 7, h = i >> 8;
-    const float2 v0 = r[4 * (lane + 64 * m) + h], v1 = r[4 * (lane + 64 * m) + h + 128];
-    o[i] = make_float4(v0.x, v1.x, v0.y, v1.y);
-  }
-}
 
 // One CTA = one (series, chunk of scales).  smem: 2 * N complex.
 template <typename T>
@@ -109,18 +52,59 @@ __global__ void k_cwt_rows(const cplx<T> *__restrict__ xhat, int n0, FftPlan<T> 
   }
 }
 
+// smallest batch a fast kernel takes: WTB_CWT_MIN_BATCH overrides the default (the tests set 1); read on every call
+static int64_t min_fast_batch(int64_t dflt) {
+  const char *e = std::getenv("WTB_CWT_MIN_BATCH");
+  return e ? std::atoll(e) : dflt;
+}
+
+CwtPlan cwt_plan(int64_t batch, int n0, int N, int S, double f0, int mother, size_t elem, int flags, bool power,
+                 bool coef) {
+  const bool fast = elem == sizeof(float) && mother == WTB_MORLET && !(flags & WTB_GENERIC_ONLY);
+  const bool power_only = power && !coef;
+  // With the rows of a series split over warps, k_cwt_fast_1024 is ahead of the generic kernel at every batch size
+  // for nfft = 1024 (0.017 ms for one series against 0.018); two series per warp (nfft = 512) pays off from about
+  // 20 series (0.021 ms flat against 0.017 + 0.4 us per series).
+  if (fast && power_only && (N == 1024 || N == 512) && f0 >= kZCut && S <= kMaxRows &&
+      batch >= min_fast_batch(N == 512 ? 20 : 1))
+    return {Fwd::kInKernel, N == 512 ? Rows::kFast512Pairs : Rows::kFast1024};
+  if (cwt_long_takes(N, elem)) return {Fwd::kInKernel, Rows::kLong};
+  if (!fast) return {Fwd::kGeneric, Rows::kGeneric};
+  // k_cwt_dif stores the first half of a row unconditionally (n0 > nfft / 2).  The rows of a series are split over
+  // CTAs when the batch is small, but this path also pays for the separate forward-FFT launch: 0.040 ms for 12
+  // series of 1346 samples against 0.021 ms + 1.7 us per series for the generic kernel (nfft = 2048 starts at 12
+  // series).  nfft = 4096: the register rows of wct_fast.cu (one CTA per two series and scale: finer work items)
+  // are faster or equal up to a few series per SM -- 0.037 / 0.064 / 0.110 / 0.185 / 0.286 ms for 12 / 64 / 148 /
+  // 300 / 500 series against 0.061 / 0.075 / 0.107 / 0.194 / 0.281 ms for k_cwt_dif<4>; 1000 series: 0.532 against
+  // 0.505 ms, 4000: 2.04 against 1.87.
+  if (power_only && (N == 2048 || N == 4096) && f0 >= kZCut && S <= kMaxRowsF && n0 > N / 2 &&
+      batch >= min_fast_batch(N == 2048 ? kMinBatchF : 4 * (int64_t)sm_count()))
+    return N == 2048 ? CwtPlan{Fwd::kPair2048, Rows::kDif2048} : CwtPlan{Fwd::kRadix16Layout4096, Rows::kDif4096};
+  if (N == 4096) {
+    if (f0 >= kMinF0 && S <= kMaxRowsC) return {Fwd::kRadix16_4096, Rows::kRows4096};
+    // no fast row kernel takes this f0 or this many scales, but k_cwt_rows reads the radix-16 kernel's spectra
+    return {Fwd::kRadix16_4096, Rows::kGeneric};
+  }
+  return {Fwd::kGeneric, Rows::kGeneric};
+}
+
 // also the first pass of wtb_cwt_averages (averages.cu)
 template <typename T>
 int cwt_device(const T *d_x, int64_t batch, int n0, int N, double dt, const Axes &ax,
                const Mother &mo, int flags, T *d_power, cplx<T> *d_coef, cudaStream_t st) {
   const int S = ax.J + 1;
   const double f0 = mo.kind == WTB_MORLET ? mo.param : 0.0;
-  if (mo.kind == WTB_MORLET && sizeof(T) == 4 && d_coef == nullptr && d_power != nullptr &&
-      !(flags & WTB_GENERIC_ONLY)) {
-    int rc = cwt_fast_try((const float *)d_x, batch, n0, N, dt, ax, f0, flags, (float *)d_power, st);
-    if (rc != 1) return rc;
+  const CwtPlan pl = cwt_plan(batch, n0, N, S, f0, mo.kind, sizeof(T), flags, d_power != nullptr, d_coef != nullptr);
+  switch (pl.rows) {
+    case Rows::kFast1024:
+    case Rows::kFast512Pairs:
+      return cwt_fast_1024(pl, (const float *)d_x, batch, n0, dt, ax, f0, flags, (float *)d_power, st);
+    case Rows::kLong:
+      return cwt_long<T>(d_x, batch, n0, N, dt, ax, mo, flags, d_power, d_coef, st);
+    default:
+      break;
   }
-  if (cwt_long_takes(N, sizeof(T))) return cwt_long<T>(d_x, batch, n0, N, dt, ax, mo, flags, d_power, d_coef, st);
+  // the other row kernels read the forward spectra from the arena
   FftPlan<T> plan;
   WTB_TRY(make_plan<T>(N, &plan));
   const size_t smem = 2 * sizeof(cplx<T>) * (size_t)plan.M;
@@ -137,42 +121,16 @@ int cwt_device(const T *d_x, int64_t batch, int n0, int N, double dt, const Axes
   const int threads = plan.M >= 1024 ? 256 : (plan.M >= 256 ? 128 : 64);
   WTB_CUDA(cudaFuncSetAttribute(k_fwd_fft<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   WTB_CUDA(cudaFuncSetAttribute(k_cwt_rows<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  int fwd_rc = 1;
-  if constexpr (sizeof(T) == 4) {
-    if (mo.kind == WTB_MORLET && !(flags & WTB_GENERIC_ONLY))
-      fwd_rc = fwd_fft_4096_try((const float *)d_x, batch, n0, N, (float2 *)d_xhat, st);
-    if (fwd_rc < 0) return fwd_rc;
-  }
-  bool dif = false;            // the two / four-warps-per-row kernels take this shape (spectra in group layout)
-  if constexpr (sizeof(T) == 4) {
-    dif = mo.kind == WTB_MORLET && !(flags & WTB_GENERIC_ONLY) && d_power && !d_coef && cwt_dif_covers(batch, n0, N, S, f0);
-    if (dif && N == 2048) {
-      WTB_CUDA(cudaFuncSetAttribute(k_fwd_fft_pair2048, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      k_fwd_fft_pair2048<<<(unsigned)batch, threads, smem, st>>>((const float *)d_x, n0, plan, (float2 *)d_xhat);
-      WTB_LAUNCH_CHECK();
-      fwd_rc = 0;
-    }
-  }
-  if (fwd_rc == 1) {
+  if (pl.rows == Rows::kDif2048 || pl.rows == Rows::kDif4096)   // with its own forward transforms (group layout)
+    return cwt_dif(pl, (const float *)d_x, (float2 *)d_xhat, batch, n0, dt, ax, f0, flags, (float *)d_power, st);
+  if (pl.fwd == Fwd::kRadix16_4096) {
+    WTB_TRY(fwd_fft_4096((const float *)d_x, batch, n0, (float2 *)d_xhat, st));
+  } else {
     k_fwd_fft<T><<<(unsigned)batch, threads, smem, st>>>(d_x, n0, plan, d_xhat);
     WTB_LAUNCH_CHECK();
   }
-  if constexpr (sizeof(T) == 4) {
-    if (dif) {
-      if (N == 4096) {
-        k_dif_layout4096<<<(unsigned)batch, 256, 0, st>>>((float2 *)d_xhat);
-        WTB_LAUNCH_CHECK();
-      }
-      const int rc = cwt_dif_try((const float2 *)d_xhat + (N == 4096 ? 2048 : 0), N, batch, n0, N, dt, ax, f0, flags,
-                                 (float *)d_power, st);
-      if (rc != 1) return rc;
-    }
-    if (mo.kind == WTB_MORLET && !(flags & WTB_GENERIC_ONLY)) {
-      const int rc = cwt_rows_4096_try((const float2 *)d_xhat, batch, n0, N, dt, ax, f0, flags, (float *)d_power,
-                                       (float2 *)d_coef, st);
-      if (rc != 1) return rc;
-    }
-  }
+  if (pl.rows == Rows::kRows4096)
+    return cwt_rows_4096((const float2 *)d_xhat, batch, n0, dt, ax, f0, flags, (float *)d_power, (float2 *)d_coef, st);
   // enough CTAs to fill the machine for small batches, few forward-FFT re-reads for large ones
   int chunk = S;
   const int64_t want = 4LL * sm_count();

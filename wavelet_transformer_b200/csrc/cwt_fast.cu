@@ -19,11 +19,10 @@
 // the daughter peak, far inside the FP32 tolerance): negative frequencies, and
 // bins above k_hi(s) = (f0 + 5.3) N dt / (2 pi s).  Rows with k_hi < 32 need no
 // step A and no transpose; rows with fewer non-zero inputs skip butterfly stages.
-#include <type_traits>
-
-#include "common.cuh"
+#include "cwt_paths.cuh"
 #include "fft32_gen.cuh"
 #include "filterbank_common.cuh"
+#include "spectral.cuh"
 
 namespace wtb {
 
@@ -36,13 +35,8 @@ using fft32::fma2;
 using fft32::mul2;
 
 constexpr int kN = 1024;
-constexpr int kWarpsDefault = 16;     // warps per CTA, one CTA per SM (WTB_CWT_WARPS overrides: 12, 14, 15)
+constexpr int kWarps = 16;            // warps per CTA, one CTA per SM
 constexpr int kTrStride = 34;         // floats per row of the transpose buffer (even, == 2 mod 32)
-constexpr float kZCut = 5.3f;         // daughter dropped where |s*w - f0| > kZCut  (exp(-14) ~ 8e-7)
-// pycwt's Morlet has no Heaviside step: at negative frequencies the daughter is exp(-(f0 + |s*w|)^2 / 2)
-// of its peak.  The one-sided transforms here drop that tail, which is below the same 8e-7 only
-// for f0 >= kZCut (f0 = 6, the reference's only value: 1.5e-8); smaller f0 take the generic kernel.
-constexpr int kMaxRows = 256;         // scale rows staged in shared memory
 
 struct RowParam {
   float a;         // (s/dt) * 2*pi/N : s*w_k = a*k
@@ -60,7 +54,7 @@ struct WarpSmem {
   float yi[32];
 };
 
-template <int kWarps> struct CtaSmem {
+struct CtaSmem {
   // exp(+2*pi*i*a*b/1024) tables, float4 = (re_0, re_1, im_0, im_1) for a packed pair
   float4 tw_a[16][32];              // pair (t2, t2+16) x k1=lane   : step A output twiddle
   float4 tw_b[16][32];              // pair (2m, 2m+1)  x t2=lane   : single-pass input twiddle
@@ -99,13 +93,13 @@ __device__ __forceinline__ constexpr int below_pow2(int m) {
 // src/utils/wavelet_helpers.py:60-78, pycwt's `outsidecoi`): row s keeps samples coi[s].x ..
 // coi[s].y and writes NaN elsewhere -- the interval is evaluated on the host in double exactly as
 // the generic kernel evaluates `period > coi(t)`, so the mask is bit-equal and costs no traffic.
-template <int kWarps, bool HALF, bool COI>
+template <bool HALF, bool COI>
 __global__ void __launch_bounds__(kWarps * 32, 1)
 k_cwt_fast_1024(const float *__restrict__ x, int64_t batch, int n0, int S,
                 const RowParam *__restrict__ rows, const ushort2 *__restrict__ coi, float f0,
                 float *__restrict__ power, int split) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
-  CtaSmem<kWarps> &sm = *reinterpret_cast<CtaSmem<kWarps> *>(smem_raw);
+  CtaSmem &sm = *reinterpret_cast<CtaSmem *>(smem_raw);
   const int lane = threadIdx.x & 31;
   const int warp = threadIdx.x >> 5;
   for (int i = threadIdx.x; i < 16 * 32; i += blockDim.x) {
@@ -366,8 +360,6 @@ k_cwt_fast_1024(const float *__restrict__ x, int64_t batch, int n0, int S,
 // 2u + q, `k_cwt_fast_fold`: stride-2 or staged stores, X^ re-read through L1; 4.0e11 coeff/s at 1346
 // samples, 5.6e11 at 2048 -- DESIGN.md section 4 keeps its measurements); this kernel is faster at every batch
 // size (4.6e11 / 6.9e11, 0.040 ms against 0.055 ms for 12 series) and replaced it.
-constexpr int kMaxRowsF = 128;
-constexpr int kMinBatchF = 12;
 // nfft = 4096 (series of 2049..4096 samples) is the same kernel with D = 4 warps per row: warp r owns the bins
 // k = 4 j + r of the one-sided spectrum (k < 2048, again 512 per warp), and
 //   x[u + 1024 q] = sum_r i^(q r) w4096^(r u) G_r[u],   q = 0..3,
@@ -721,6 +713,39 @@ k_cwt_dif(const float2 *__restrict__ xhat, int64_t xhat_stride, int64_t batch, i
 
 }  // namespace
 
+// Forward FFT (N = 2048) for k_cwt_dif<2>: the positive half of the spectrum leaves in the group layout
+// (CtaSmemP::xh) -- per series 8 KB at the start of its xhat row: float4 [parity h][m < 8][lane] =
+// (Re X^[k0], Re X^[k1], Im X^[k0], Im X^[k1]), k0 = 2 (lane + 64 m) + h, k1 = k0 + 64.
+__global__ void k_fwd_fft_pair2048(const float *__restrict__ x, int n0, FftPlan<float> plan, float2 *__restrict__ xhat) {
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  float2 *a = reinterpret_cast<float2 *>(smem_raw);
+  float2 *b = a + plan.M;
+  const int N = plan.n;
+  const int64_t row = blockIdx.x;
+  const float *xr = x + row * n0;
+  for (int t = threadIdx.x; t < N; t += blockDim.x) a[t] = make_float2(t < n0 ? xr[t] : 0.0f, 0.0f);
+  __syncthreads();
+  const float2 *r = plan_fft<float, -1>(a, b, plan);
+  float4 *o = reinterpret_cast<float4 *>(xhat + row * N);
+  for (int i = threadIdx.x; i < 2 * 8 * 32; i += blockDim.x) {
+    const int lane = i & 31, m = (i >> 5) & 7, h = i >> 8;
+    const float2 v0 = r[2 * (lane + 64 * m) + h], v1 = r[2 * (lane + 64 * m) + h + 64];
+    o[i] = make_float4(v0.x, v1.x, v0.y, v1.y);
+  }
+}
+
+// The same layout for N = 4096 (four warps per row: k0 = 4 (lane + 64 m) + r, k1 = k0 + 128, r < 4; 16 KB), built from
+// the natural-order spectrum of the radix-16 forward kernel into the unused negative-frequency half of the row.
+__global__ void k_dif_layout4096(float2 *__restrict__ xhat) {
+  const float2 *r = xhat + (int64_t)blockIdx.x * 4096;
+  float4 *o = reinterpret_cast<float4 *>(xhat + (int64_t)blockIdx.x * 4096 + 2048);
+  for (int i = threadIdx.x; i < 4 * 8 * 32; i += blockDim.x) {
+    const int lane = i & 31, m = (i >> 5) & 7, h = i >> 8;
+    const float2 v0 = r[4 * (lane + 64 * m) + h], v1 = r[4 * (lane + 64 * m) + h + 128];
+    o[i] = make_float4(v0.x, v1.x, v0.y, v1.y);
+  }
+}
+
 // Per-row sample interval inside the cone of influence, evaluated in double with the expression
 // the generic kernel (cwt.cu) and pycwt use -- period(s) > coi(t) is masked -- so that the fused
 // mask is bit-equal.  Rows with no valid sample get the empty interval [1, 0].
@@ -754,48 +779,38 @@ void coi_row_ranges(int n0, double dt, const Axes &ax, double f0, std::vector<us
   }
 }
 
-// smallest batch the warp-per-series kernels take (WTB_CWT_MIN_BATCH overrides; tests set 1)
-static int64_t min_fast_batch(int64_t dflt) {
-  const char *e = std::getenv("WTB_CWT_MIN_BATCH");
-  return e ? std::atoll(e) : dflt;
-}
-
-int cwt_fast_try(const float *d_x, int64_t batch, int n0, int nfft, double dt, const Axes &ax, double f0,
-                 int flags, float *d_power, cudaStream_t st) {
-  const int S = ax.J + 1;
-  // nfft = 512 runs two series per warp on the interleaved 1024-point spectrum (HALF): in that
-  // domain a series' bin kk sits at k = 2 kk + parity, so a, lognorm and the band edge are those
-  // of a 1024-point transform with the edge one bin further out
-  const bool half = nfft == kN / 2;
-  if ((nfft != kN && !half) || f0 < kZCut || S > kMaxRows) return 1;
-  const bool coi = flags & WTB_COI_MASK;
-  // With the rows of a series split over warps (below) this kernel is ahead of the generic one at
-  // every batch size for nfft = 1024 (0.017 ms for one series against 0.018); two series per warp
-  // (nfft = 512) pays off from about 20 series (0.021 ms flat against 0.017 + 0.4 us per series).
-  if (batch < min_fast_batch(half ? 20 : 1)) return 1;
-  // fewer series than warps on the machine: split each series' rows over up to 16 warps
-  const int64_t series_items = half ? (batch + 1) / 2 : batch;
-  const int64_t machine_warps = (int64_t)sm_count() * kWarpsDefault;
-  const int split = (int)std::max<int64_t>(1, std::min<int64_t>(std::min<int64_t>(16, S), machine_warps / series_items));
-  std::vector<RowParam> rows(S);
-  for (int s = 0; s < S; ++s) {
-    const double a = ax.scales[s] / dt * 2.0 * kPi / kN;
-    int khi = (int)std::floor((f0 + kZCut) / a) + (half ? 1 : 0);
-    if (khi > kN / 2 - 1) khi = kN / 2 - 1;
-    if (khi < 1) khi = 1;
+// RowParam of every scale row for an n-point transform whose one-sided spectrum a group of D warps splits by residue
+// mod D (k_cwt_fast_1024: n = 1024, D = 1; k_cwt_dif<D>: n = 1024 D).  `extra` moves the band edge one bin further
+// out: for nfft = 512 two series share the interleaved 1024-point spectrum, where a series' bin kk sits at
+// k = 2 kk + parity, so a, lognorm and the band edge are those of a 1024-point transform with the edge one bin on.
+static std::vector<RowParam> row_params(int n, int D, int extra, double dt, const Axes &ax, double f0) {
+  std::vector<RowParam> rows(ax.J + 1);
+  for (size_t s = 0; s < rows.size(); ++s) {
+    const double a = ax.scales[s] / dt * 2.0 * kPi / n;
+    int khi = (int)std::floor((f0 + kZCut) / a) + extra;
+    khi = std::max(1, std::min(khi, n / 2 - 1));
     RowParam &r = rows[s];
     r.a = (float)a;
-    r.lognorm = (float)std::log2(std::sqrt(2.0 * kPi * ax.scales[s] / dt) * 0.75112554446494248286 / kN);
-    if (khi >= 32) {
-      r.multi = 1;
-      r.L = ilog2(khi / 32 + 1);       // K2 = 2^L >= ceil((khi+1)/32), at most 16 (one-sided)
-      if (r.L > 4) r.L = 4;
-      if (r.L < 1) r.L = 1;
-    } else {
-      r.multi = 0;
-      r.L = ilog2(khi + 1);            // K1 = 2^L >= khi+1, at least 2
-    }
+    r.lognorm = (float)std::log2(std::sqrt(2.0 * kPi * ax.scales[s] / dt) * 0.75112554446494248286 / n);
+    // a warp transforms the bins of one residue mod D, j = k / D <= jhi < 512: K2 = 2^L >= ceil((jhi+1)/32), at most
+    // 16 (one-sided), for a two-pass row; K1 = 2^L >= jhi+1, at least 2, for a single-pass one
+    const int jhi = khi / D;
+    r.multi = jhi >= 32;
+    r.L = r.multi ? std::max(1, std::min(4, ilog2(jhi / 32 + 1))) : std::max(1, ilog2(jhi + 1));
   }
+  return rows;
+}
+
+int cwt_fast_1024(const CwtPlan &pl, const float *d_x, int64_t batch, int n0, double dt, const Axes &ax, double f0,
+                  int flags, float *d_power, cudaStream_t st) {
+  const int S = ax.J + 1;
+  const bool half = pl.rows == Rows::kFast512Pairs;   // two series per warp (HALF)
+  const bool coi = flags & WTB_COI_MASK;
+  // fewer series than warps on the machine: split each series' rows over up to 16 warps
+  const int64_t items = half ? (batch + 1) / 2 : batch;
+  const int64_t machine_warps = (int64_t)sm_count() * kWarps;
+  const int split = (int)std::max<int64_t>(1, std::min<int64_t>(std::min<int64_t>(16, S), machine_warps / items));
+  const std::vector<RowParam> rows = row_params(kN, 1, half ? 1 : 0, dt, ax, f0);
   void *scratch = nullptr;
   WTB_TRY(arena_reserve(sizeof(RowParam) * S + sizeof(ushort2) * S, &scratch));
   RowParam *d_rows = (RowParam *)scratch;
@@ -808,70 +823,38 @@ int cwt_fast_try(const float *d_x, int64_t batch, int n0, int nfft, double dt, c
     d_coi = (ushort2 *)(d_rows + S);
     WTB_CUDA(cudaMemcpyAsync(d_coi, rng.data(), sizeof(ushort2) * S, cudaMemcpyHostToDevice, st));
   }
-  int warps = kWarpsDefault;
-  if (const char *e = std::getenv("WTB_CWT_WARPS")) warps = std::atoi(e);
-  auto launch_k = [&](auto kern, int W, int64_t items) -> int {
-    const size_t smem = sizeof(CtaSmem<kWarpsDefault>) - sizeof(WarpSmem) * (kWarpsDefault - W);
-    WTB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  auto launch = [&](auto kern) -> int {
+    WTB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(CtaSmem)));
     const int grid = (int)std::min<int64_t>(items * split, (int64_t)sm_count());
-    kern<<<grid, W * 32, smem, st>>>(d_x, batch, n0, S, d_rows, d_coi, (float)f0, d_power, split);
+    kern<<<grid, kWarps * 32, sizeof(CtaSmem), st>>>(d_x, batch, n0, S, d_rows, d_coi, (float)f0, d_power, split);
     WTB_LAUNCH_CHECK();
     return WTB_OK;
   };
-  auto launch = [&](auto tag) -> int {
-    constexpr int W = decltype(tag)::value;
-    static_assert(sizeof(CtaSmem<W>) == sizeof(CtaSmem<kWarpsDefault>) - sizeof(WarpSmem) * (kWarpsDefault - W), "layout");
-    return launch_k(k_cwt_fast_1024<W, false, false>, W, batch);
-  };
-  if (half) {
-    if (coi) return launch_k(k_cwt_fast_1024<kWarpsDefault, true, true>, kWarpsDefault, series_items);
-    return launch_k(k_cwt_fast_1024<kWarpsDefault, true, false>, kWarpsDefault, series_items);
-  }
-  if (coi) return launch_k(k_cwt_fast_1024<kWarpsDefault, false, true>, kWarpsDefault, batch);
-  switch (warps) {
-    case 12: return launch(std::integral_constant<int, 12>{});
-    case 14: return launch(std::integral_constant<int, 14>{});
-    case 15: return launch(std::integral_constant<int, 15>{});
-    default: return launch(std::integral_constant<int, 16>{});
-  }
+  if (half) return coi ? launch(k_cwt_fast_1024<true, true>) : launch(k_cwt_fast_1024<true, false>);
+  return coi ? launch(k_cwt_fast_1024<false, true>) : launch(k_cwt_fast_1024<false, false>);
 }
 
-
-// true: cwt_dif_try runs this shape and wants the forward spectra in its group layout (CtaSmemP::xh; written by
-// k_fwd_fft_pair2048 / k_dif_layout4096 in cwt.cu).  The kernels store the first half of a row unconditionally
-// (n0 > nfft / 2).  The rows of a series are split over CTAs when the batch is small, but this path also pays for
-// the separate forward-FFT launch: 0.040 ms for 12 series of 1346 samples against 0.021 ms + 1.7 us per series
-// for the generic kernel (nfft = 2048 starts at 12 series).
-bool cwt_dif_covers(int64_t batch, int n0, int nfft, int S, double f0) {
-  // nfft = 4096: the register rows of wct_fast.cu (one CTA per two series and scale: finer work items) are faster or
-  // equal up to a few series per SM -- 0.037 / 0.064 / 0.110 / 0.185 / 0.286 ms for 12 / 64 / 148 / 300 / 500 series
-  // against 0.061 / 0.075 / 0.107 / 0.194 / 0.281 ms here; 1000 series: 0.532 against 0.505 ms, 4000: 2.04 against 1.87
-  const int64_t min_batch = min_fast_batch(nfft == 2 * kN ? kMinBatchF : 4 * (int64_t)sm_count());
-  return (nfft == 2 * kN || nfft == 4 * kN) && f0 >= kZCut && S <= kMaxRowsF && batch >= min_batch && n0 > nfft / 2;
-}
-
-// FP32 CWT + power rows for nfft = 2048 / 4096 from forward spectra in group layout (`d_layout`: per series
-// `stride` float2 apart, 8 KB / 16 KB each; cwt.cu tries this after its forward-FFT kernel).  Returns 1 when the
-// shape is not covered.
-int cwt_dif_try(const float2 *d_layout, int64_t stride, int64_t batch, int n0, int nfft, double dt, const Axes &ax,
-                double f0, int flags, float *d_power, cudaStream_t st) {
+int cwt_dif(const CwtPlan &pl, const float *d_x, float2 *d_xhat, int64_t batch, int n0, double dt, const Axes &ax,
+            double f0, int flags, float *d_power, cudaStream_t st) {
   const int S = ax.J + 1;
-  if (!cwt_dif_covers(batch, n0, nfft, S, f0)) return 1;
+  const int nfft = pl.rows == Rows::kDif2048 ? 2 * kN : 4 * kN;
   const int D = nfft / kN;
-  const bool coi = flags & WTB_COI_MASK;
-  std::vector<RowParam> rows(S);
-  for (int s = 0; s < S; ++s) {
-    const double a = ax.scales[s] / dt * 2.0 * kPi / nfft;
-    int khi = (int)std::floor((f0 + kZCut) / a);
-    khi = std::max(1, std::min(khi, nfft / 2 - 1));
-    RowParam &r = rows[s];
-    r.a = (float)a;
-    r.lognorm = (float)std::log2(std::sqrt(2.0 * kPi * ax.scales[s] / dt) * 0.75112554446494248286 / nfft);
-    // a warp transforms the bins of one residue mod D, j = k / D <= jhi < 512
-    const int jhi = khi / D;
-    r.multi = jhi >= 32;
-    r.L = r.multi ? std::max(1, std::min(4, ilog2(jhi / 32 + 1))) : std::max(1, ilog2(jhi + 1));
+  const float2 *d_layout = d_xhat;
+  if (pl.fwd == Fwd::kPair2048) {
+    FftPlan<float> plan;
+    WTB_TRY(make_plan<float>(nfft, &plan));
+    const size_t smem = 2 * sizeof(float2) * (size_t)plan.M;
+    WTB_CUDA(cudaFuncSetAttribute(k_fwd_fft_pair2048, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    k_fwd_fft_pair2048<<<(unsigned)batch, 256, smem, st>>>(d_x, n0, plan, d_xhat);
+    WTB_LAUNCH_CHECK();
+  } else {
+    WTB_TRY(fwd_fft_4096(d_x, batch, n0, d_xhat, st));
+    k_dif_layout4096<<<(unsigned)batch, 256, 0, st>>>(d_xhat);
+    WTB_LAUNCH_CHECK();
+    d_layout = d_xhat + 2048;
   }
+  const bool coi = flags & WTB_COI_MASK;
+  const std::vector<RowParam> rows = row_params(nfft, D, 0, dt, ax, f0);
   // the caller's arena holds xhat: row parameters go to the per-thread parameter buffer
   void *prm = nullptr;
   WTB_TRY(params_reserve((sizeof(RowParam) + sizeof(ushort2)) * kMaxRowsF, &prm));
@@ -902,7 +885,7 @@ int cwt_dif_try(const float2 *d_layout, int64_t stride, int64_t batch, int n0, i
   WTB_REQUIRE(batch * split < (1LL << 31), WTB_EUNSUPPORTED, "batch too large for one launch");
   auto run = [&](auto kern, size_t smem) -> int {
     WTB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    kern<<<grid, kDifWarps * 32, smem, st>>>(d_layout, stride, batch, n0, S, d_rows, d_coi, (float)f0, d_power, split);
+    kern<<<grid, kDifWarps * 32, smem, st>>>(d_layout, nfft, batch, n0, S, d_rows, d_coi, (float)f0, d_power, split);
     WTB_LAUNCH_CHECK();
     return WTB_OK;
   };

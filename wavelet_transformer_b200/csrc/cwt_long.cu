@@ -17,6 +17,7 @@
 // k_cwt_rows' arithmetic) and power / coefficients for t < n0 (pass 2).  Rows run in waves whose
 // intermediate Y fits half the B200's 126 MB L2 (long_wave_rows); a row's arithmetic does not depend on
 // its wave, so results do not depend on the batch, the host chunk or the pool.
+#include "cwt_paths.cuh"
 #include "spectral.cuh"
 
 namespace wtb {

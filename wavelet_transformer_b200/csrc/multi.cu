@@ -16,12 +16,11 @@
 #include <memory>
 #include <thread>
 
-#include "common.cuh"
+#include "cwt_paths.cuh"
 
 namespace wtb {
 
 extern thread_local int tl_worker_device;   // runtime.cu: CallScope picks this device on pool threads
-void mc_row_has_points(int nsurr, double dt, const Axes &ax, double f0, std::vector<uint8_t> *any);  // wct.cu
 
 namespace {
 

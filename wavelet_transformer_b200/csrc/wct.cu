@@ -12,22 +12,12 @@
 //
 // The Gaussian filter is real and even, so filtering the packed field P gives
 // smooth(|W1|^2) in its real part and smooth(|W2|^2) in its imaginary part.
+#include "cwt_paths.cuh"
 #include "spectral.cuh"
-#include "wct_common.cuh"
 
 #include <type_traits>
 
 namespace wtb {
-
-// wct_fast.cu: FP32 nfft=4096 register-FFT pipeline (spectra kernel + coherence kernel);
-// returns 1 when the shape is not covered.  d_spec: [pairs, S, 4096] float4 scratch.
-int wct_fast_try(const float2 *d_xhat, int64_t pairs, int n0, int N, double dt, const Axes &ax, double f0,
-                 void *d_rows_scratch, size_t rows_scratch_bytes, float4 *d_spec, const ScaleWin &win,
-                 float *d_wct, float *d_phase, float2 *d_w12, unsigned long long *d_hist,
-                 const int *d_tlo, const int *d_thi, int maxscale, cudaStream_t st);
-
-// wct_fast.cu: forward FFTs with the radix-16 register kernel (FP32, N = 4096); 1 = not covered
-int fwd_fft_4096_try(const float *d_y, int64_t nseries, int n0, int N, float2 *d_xhat, cudaStream_t st);
 
 template <typename T> struct vec4_of;
 template <> struct vec4_of<float> { using type = float4; };
@@ -110,9 +100,6 @@ __global__ void k_wct_rows(const cplx<T> *__restrict__ xhat, int n0, FftPlan<T> 
   }
 }
 
-// set per call from WTB_GENERIC_ONLY (testing the generic kernels at the fast path's shapes)
-static thread_local bool g_force_generic = false;
-
 // One thread = one (pair, t) column; walks the scales.  MODE 0: write WCT plane;
 // MODE 1: add to the per-scale histogram for t inside [tlo[s], thi[s]] and s < maxscale.
 template <typename T, int MODE>
@@ -164,10 +151,11 @@ static int make_win(double dj, ScaleWin *win) {
   return WTB_OK;
 }
 
-// Shared device pipeline.  d_y: [pairs, 2, n0] (series interleaved per pair).
+// Shared device pipeline.  d_y: [pairs, 2, n0] (series interleaved per pair).  generic: the generic kernels at
+// every shape (WTB_GENERIC_ONLY).
 template <typename T>
 static int wct_device(const T *d_y, int64_t pairs, int n0, int N, double dt, double dj,
-                      const Axes &ax, double f0, T *d_wct, T *d_phase, cplx<T> *d_w12,
+                      const Axes &ax, double f0, bool generic, T *d_wct, T *d_phase, cplx<T> *d_w12,
                       unsigned long long *d_hist, const int *h_tlo, const int *h_thi, int maxscale,
                       cudaStream_t st) {
   const int S = ax.J + 1;
@@ -182,13 +170,17 @@ static int wct_device(const T *d_y, int64_t pairs, int n0, int N, double dt, dou
               sizeof(T) == 4 ? "float" : "double");
   ScaleWin win;
   WTB_TRY(make_win(dj, &win));
+  // FP32, nfft = 4096: the radix-16 forward kernel, and the register-FFT pipeline of wct_fast.cu where its one-sided
+  // daughters hold (f0 >= kMinF0), its shared-memory rows and its boxcar ring fit
+  const bool fast_fwd = std::is_same<T, float>::value && !generic && N == 4096;
+  const bool fast = fast_fwd && f0 >= kMinF0 && S <= kMaxRowsC && win.K <= 32;
   auto al = [](size_t b) { return (b + 255) / 256 * 256; };
   const size_t b_sc = al(sizeof(double) * S);
   const size_t b_rng = al(sizeof(int) * S);
   const size_t b_xh = al(sizeof(cplx<T>) * (size_t)pairs * 2 * N);
   const size_t b_ts = smooth ? al(sizeof(vec4<T>) * (size_t)pairs * S * N) : 0;  // N >= n0: also fits the fast path's spectra
   void *scratch = nullptr;
-  const size_t b_rows = al(32 * (size_t)S);
+  const size_t b_rows = al(32 * (size_t)S);   // the fast path's row parameters (WRow)
   WTB_TRY(arena_reserve(b_sc + 2 * b_rng + b_rows + b_xh + b_ts, &scratch));
   char *p = (char *)scratch;
   void *d_rows_scratch = p; p += b_rows;
@@ -207,37 +199,27 @@ static int wct_device(const T *d_y, int64_t pairs, int n0, int N, double dt, dou
   WTB_CUDA(cudaFuncSetAttribute(k_wct_rows<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_rows));
   WTB_REQUIRE(pairs * S < (1LL << 31) && pairs * 2 < (1LL << 31), WTB_EUNSUPPORTED, "batch too large");
   WTB_TRACE_POINT(st, "wct: scratch + small copies");
-  int fwd_rc = 1;
-  if constexpr (std::is_same<T, float>::value) {
-    if (!g_force_generic) fwd_rc = fwd_fft_4096_try((const float *)d_y, pairs * 2, n0, N, (float2 *)d_xhat, st);
-    if (fwd_rc < 0) return fwd_rc;
-  }
-  if (fwd_rc == 1) {
+  if (fast_fwd) {
+    WTB_TRY(fwd_fft_4096((const float *)d_y, pairs * 2, n0, (float2 *)d_xhat, st));
+  } else {
     k_fwd_fft<T><<<(unsigned)(pairs * 2), threads, smem_fwd, st>>>(d_y, n0, plan, d_xhat);
     WTB_LAUNCH_CHECK();
   }
   WTB_TRACE_POINT(st, "wct: forward transforms");
-  int fast_rc = 1;
-  if constexpr (std::is_same<T, float>::value) {
-    if (!g_force_generic)
-      fast_rc = wct_fast_try((const float2 *)d_xhat, pairs, n0, N, dt, ax, f0, d_rows_scratch, b_rows,
-                             (float4 *)d_tsm, win, (float *)d_wct, (float *)d_phase, (float2 *)d_w12, d_hist,
-                             d_tlo, d_thi, maxscale, st);
-    if (fast_rc < 0) return fast_rc;
-  }
-  if (fast_rc == 1) {
-    k_wct_rows<T><<<(unsigned)(pairs * S), threads, smem_rows, st>>>(
-        d_xhat, n0, plan, S, d_scales, dt, f0, d_tsm, d_phase, d_w12, smooth ? 1 : 0);
+  if (fast)
+    return wct_fast((const float2 *)d_xhat, pairs, n0, dt, ax, f0, d_rows_scratch, (float4 *)d_tsm, win,
+                    (float *)d_wct, (float *)d_phase, (float2 *)d_w12, d_hist, d_tlo, d_thi, maxscale, st);
+  k_wct_rows<T><<<(unsigned)(pairs * S), threads, smem_rows, st>>>(
+      d_xhat, n0, plan, S, d_scales, dt, f0, d_tsm, d_phase, d_w12, smooth ? 1 : 0);
+  WTB_LAUNCH_CHECK();
+  if (smooth) {
+    const int64_t cols = pairs * n0;
+    const unsigned blocks = (unsigned)((cols + 255) / 256);
+    if (d_hist)
+      k_wct_scale<T, 1><<<blocks, 256, 0, st>>>(d_tsm, pairs, n0, S, win, nullptr, d_hist, d_tlo, d_thi, maxscale);
+    else
+      k_wct_scale<T, 0><<<blocks, 256, 0, st>>>(d_tsm, pairs, n0, S, win, d_wct, nullptr, nullptr, nullptr, 0);
     WTB_LAUNCH_CHECK();
-    if (smooth) {
-      const int64_t cols = pairs * n0;
-      const unsigned blocks = (unsigned)((cols + 255) / 256);
-      if (d_hist)
-        k_wct_scale<T, 1><<<blocks, 256, 0, st>>>(d_tsm, pairs, n0, S, win, nullptr, d_hist, d_tlo, d_thi, maxscale);
-      else
-        k_wct_scale<T, 0><<<blocks, 256, 0, st>>>(d_tsm, pairs, n0, S, win, d_wct, nullptr, nullptr, nullptr, 0);
-      WTB_LAUNCH_CHECK();
-    }
   }
   return WTB_OK;
 }
@@ -259,7 +241,6 @@ static int xwt_wct_entry(const void *y1, const void *y2, int64_t batch, int n0, 
   if (!(flags & WTB_DEVICE_PTRS) && pool_size() > 1 && batch >= 2 * pool_size() && !g_in_shard) {
     return run_sharded_fn(batch, 2, st, [&](int, int64_t first, int64_t count, cudaStream_t s) {
       g_in_shard = true;
-      g_force_generic = flags & WTB_GENERIC_ONLY;
       const int rc = xwt_wct_entry<T>((const T *)y1 + first * n0, (const T *)y2 + first * n0, count, n0, N, dt, dj, ax,
                                       f0, flags, wct_out ? (T *)wct_out + first * plane : nullptr,
                                       phase_out ? (T *)phase_out + first * plane : nullptr,
@@ -296,8 +277,8 @@ static int xwt_wct_entry(const void *y1, const void *y2, int64_t batch, int n0, 
     T *o_wct = dev && wct_out ? (T *)wct_out + b0 * plane : d_wct;
     T *o_phase = dev && phase_out ? (T *)phase_out + b0 * plane : d_phase;
     cplx<T> *o_w12 = dev && w12_out ? (cplx<T> *)w12_out + b0 * plane : d_w12;
-    WTB_TRY(wct_device<T>(d_y, nb, n0, N, dt, dj, ax, f0, o_wct, o_phase, o_w12, nullptr, nullptr,
-                          nullptr, 0, st));
+    WTB_TRY(wct_device<T>(d_y, nb, n0, N, dt, dj, ax, f0, flags & WTB_GENERIC_ONLY, o_wct, o_phase, o_w12, nullptr,
+                          nullptr, nullptr, 0, st));
     if (!dev) {
       if (wct_out)
         WTB_TRY(copy_to_host((T *)wct_out + b0 * plane, d_wct, sizeof(T) * nb * plane, st));
@@ -349,7 +330,6 @@ static void coi_ranges(int nsurr, double dt, const Axes &ax, double f0, std::vec
   }
 }
 
-// rows with at least one sample inside the reliable region (multi.cu's percentile step)
 void mc_row_has_points(int nsurr, double dt, const Axes &ax, double f0, std::vector<uint8_t> *any) {
   std::vector<int> tlo, thi;
   coi_ranges(nsurr, dt, ax, f0, &tlo, &thi, any);
@@ -484,8 +464,8 @@ static int mc_hist_entry(double a1, double a2, double dt, double dj, const Axes 
       WTB_TRY(rednoise_device<T>(a1, a2, nsurr, mc_first + m0, nb, seed, flags & WTB_NOISE_WHITE, d_ybuf[0], st));
     }
     WTB_TRACE_POINT(st, "mc: surrogates");
-    WTB_TRY(wct_device<T>(src, nb, nsurr, N, dt, dj, ax, f0, nullptr, nullptr, nullptr, hist_dev,
-                          tlo.data(), thi.data(), maxscale, st));
+    WTB_TRY(wct_device<T>(src, nb, nsurr, N, dt, dj, ax, f0, flags & WTB_GENERIC_ONLY, nullptr, nullptr, nullptr,
+                          hist_dev, tlo.data(), thi.data(), maxscale, st));
     if (pipelined) WTB_CUDA(cudaEventRecord(ev[2 + buf], st));
     // chunks reuse the arena without a host sync: every kernel and copy is ordered on `st`
     WTB_TRACE_POINT(st, "mc: pipeline (fft, A, C, B)");
@@ -519,7 +499,6 @@ extern "C" int wtb_xwt_wct(const void *y1, const void *y2, int64_t batch, int n0
   WTB_TRY(resolve_axes(n0, dt, dj, s0, J, f0, &ax));
   if (batch == 0) return WTB_OK;
   cudaStream_t st = (cudaStream_t)stream;
-  g_force_generic = flags & WTB_GENERIC_ONLY;
   if (flags & WTB_F64)
     return xwt_wct_entry<double>(y1, y2, batch, n0, nfft, dt, dj, ax, f0, flags, wct_out, phase_out, w12_out, st);
   return xwt_wct_entry<float>(y1, y2, batch, n0, nfft, dt, dj, ax, f0, flags, wct_out, phase_out, w12_out, st);
@@ -538,7 +517,6 @@ extern "C" int wtb_wct_mc_hist(double a1, double a2, double dt, double dj, doubl
   WTB_TRY(resolve_axes(nsurr, dt, dj, s0, J, f0, &ax));
   if (mc_count == 0) return WTB_OK;
   cudaStream_t st = (cudaStream_t)stream;
-  g_force_generic = flags & WTB_GENERIC_ONLY;
   if (flags & WTB_F64)
     return mc_hist_entry<double>(a1, a2, dt, dj, ax, f0, nsurr, maxscale, mc_first, mc_count, seed,
                                  surrogates, flags, hist, st);

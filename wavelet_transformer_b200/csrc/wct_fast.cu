@@ -22,12 +22,10 @@
 // The boxcar is a linear combination of rows, so it commutes with the inverse transform;
 // applying it to the filtered spectra removes the time-domain plane round trip and the
 // separate scale-smoothing pass of the generic path.
-#include "wct_common.cuh"
+#include "cwt_paths.cuh"
 #include "fft16_gen.cuh"
 
 namespace wtb {
-
-void coi_row_ranges(int n0, double dt, const Axes &ax, double f0, std::vector<ushort2> *out);   // cwt_fast.cu
 
 namespace {
 
@@ -36,9 +34,6 @@ using fft16::br4;
 constexpr int kN = 4096;
 constexpr int kThreads = 256;
 constexpr int kBuf = kN + kN / 16;     // padded: index i lives at pad(i) = i + (i >> 4)
-constexpr int kMaxRowsC = 512;         // scale rows the boxcar kernel stages in shared memory
-constexpr double kMinF0 = 5.3;         // one-sided daughters: the dropped negative-frequency tail is
-                                       // exp(-f0^2/2) of the peak (8e-7 at 5.3, 1.5e-8 at the reference's f0 = 6)
 
 struct WRow {
   float a;        // (s/dt) * 2*pi/N : s*w_k = a*k
@@ -50,6 +45,7 @@ struct WRow {
   float kc2;      // squared bin index beyond which the Gaussian filter is < 1e-7
   int kc;         // floor(sqrt(kc2))
 };
+static_assert(sizeof(WRow) == 32, "wct_device reserves 32 bytes of row parameters per scale");
 
 struct CohWin {
   int K, up;
@@ -703,10 +699,7 @@ static void fill_rows(const Axes &ax, double dt, double f0, std::vector<WRow> *r
   }
 }
 
-// Forward FFTs of [nseries, n0] real rows into xhat [nseries, 4096] with the radix-16 register
-// kernel (FP32, N = 4096 only).  Returns 1 when the shape is not covered.
-int fwd_fft_4096_try(const float *d_y, int64_t nseries, int n0, int N, float2 *d_xhat, cudaStream_t st) {
-  if (N != kN || n0 > kN || nseries < 1) return 1;
+int fwd_fft_4096(const float *d_y, int64_t nseries, int n0, float2 *d_xhat, cudaStream_t st) {
   const float2 *tw2 = nullptr, *tw3 = nullptr;
   WTB_TRY(ensure_tables(&tw2, &tw3));
   const size_t smem = 2 * sizeof(float2) * kBuf + sizeof(float2) * 256;
@@ -718,12 +711,9 @@ int fwd_fft_4096_try(const float *d_y, int64_t nseries, int n0, int N, float2 *d
   return WTB_OK;
 }
 
-// FP32 CWT rows for nfft = 4096 from forward spectra xhat [batch, 4096] (cwt.cu tries this
-// before its generic row kernel).  Returns 1 when the shape is not covered.
-int cwt_rows_4096_try(const float2 *d_xhat, int64_t batch, int n0, int N, double dt, const Axes &ax, double f0,
-                      int flags, float *d_power, float2 *d_coef, cudaStream_t st) {
+int cwt_rows_4096(const float2 *d_xhat, int64_t batch, int n0, double dt, const Axes &ax, double f0, int flags,
+                  float *d_power, float2 *d_coef, cudaStream_t st) {
   const int S = ax.J + 1;
-  if (N != kN || f0 < kMinF0 || S > kMaxRowsC) return 1;
   std::vector<WRow> rows;
   fill_rows(ax, dt, f0, &rows);
   const float2 *tw2 = nullptr, *tw3 = nullptr;
@@ -750,14 +740,10 @@ int cwt_rows_4096_try(const float2 *d_xhat, int64_t batch, int n0, int N, double
   return WTB_OK;
 }
 
-// d_rows_scratch: device scratch for S WRow entries (caller's arena); d_spec: scratch of
-// pairs*S*4096 float4-equivalents.  Returns 1 when the shape is not covered.
-int wct_fast_try(const float2 *d_xhat, int64_t pairs, int n0, int N, double dt, const Axes &ax, double f0,
-                 void *d_rows_scratch, size_t rows_scratch_bytes, float4 *d_spec, const ScaleWin &win,
-                 float *d_wct, float *d_phase, float2 *d_w12, unsigned long long *d_hist,
-                 const int *d_tlo, const int *d_thi, int maxscale, cudaStream_t st) {
+int wct_fast(const float2 *d_xhat, int64_t pairs, int n0, double dt, const Axes &ax, double f0, void *d_rows_scratch,
+             float4 *d_spec, const ScaleWin &win, float *d_wct, float *d_phase, float2 *d_w12,
+             unsigned long long *d_hist, const int *d_tlo, const int *d_thi, int maxscale, cudaStream_t st) {
   const int S = ax.J + 1;
-  if (N != kN || f0 < kMinF0 || sizeof(WRow) * S > rows_scratch_bytes || win.K > 32 || S > kMaxRowsC) return 1;
   const bool smooth = d_wct || d_hist;
   std::vector<WRow> rows;
   fill_rows(ax, dt, f0, &rows);
