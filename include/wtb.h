@@ -160,7 +160,10 @@ int wtb_phase_arrows(const void *phase, int64_t count, int flags, void *u_out, v
  * (src/wct.py:106, src/xwt.py:122) minus the host-side normalisation ------- */
 /* y1, y2: [batch, n0] real (already normalised by the caller).  Outputs (any
  * may be NULL): wct_out [batch,S,n0] real = |S12|^2/(S1*S2); phase_out
- * [batch,S,n0] real = angle(W1*conj(W2)); w12_out [batch,S,n0] complex. */
+ * [batch,S,n0] real = angle(W1*conj(W2)); w12_out [batch,S,n0] complex.
+ * nfft: one CTA per transform up to 8192 in FP32 / 4096 in FP64 (any length up to 4096 / 2048 with
+ * WTB_FFT_NO_PAD-style unpadded nfft); longer powers of two, up to 2^22 = 4194304, take four-step
+ * transforms over several CTAs (same arithmetic per row); larger nfft returns WTB_EUNSUPPORTED. */
 int wtb_xwt_wct(const void *y1, const void *y2, int64_t batch, int n0, int nfft,
                 double dt, double dj, double s0, int J, double f0, int flags,
                 void *wct_out, void *phase_out, void *w12_out, void *stream);
@@ -176,7 +179,9 @@ int wtb_wct_mc_geometry(double dt, double dj, double s0, int J, double f0,
  * keyed by the global index, so any partition over GPUs sums to the same
  * histogram).  surrogates: NULL -> AR(1) (or white) noise generated on device
  * from `seed`; else [mc_count, 2, nsurr] real ready-made series (host-injected
- * parity mode).  hist: [S, WTB_NBINS] uint64, ADDED to (caller zeroes). */
+ * parity mode).  hist: [S, WTB_NBINS] uint64, ADDED to (caller zeroes).  The surrogates are padded to
+ * the next power of two up to 2^22 (nsurr past 8192 in FP32 / 4096 in FP64 takes the four-step rows of
+ * wtb_xwt_wct); with WTB_FFT_NO_PAD the one-CTA limits of wtb_xwt_wct apply. */
 int wtb_wct_mc_hist(double a1, double a2, double dt, double dj, double s0, int J,
                     double f0, int64_t mc_first, int64_t mc_count, uint64_t seed,
                     const void *surrogates, int flags, uint64_t *hist, void *stream);
@@ -197,7 +202,7 @@ int wtb_wct_sig_from_hist_device(const uint64_t *hist, int S, int maxscale, doub
  * memory over NVLink, and the percentile step gives sig95 [J+1].  surrogates: NULL (device Philox
  * AR(1) noise keyed by the global realisation index: the result does not depend on the number of
  * GPUs) or a HOST array [mc_count, 2, nsurr].  hist_out (may be NULL): [J+1, WTB_NBINS] summed
- * histogram.  Host buffers only. */
+ * histogram.  Host buffers only.  Surrogate lengths as wtb_wct_mc_hist (padded: up to 2^22). */
 int wtb_wct_significance(double a1, double a2, double dt, double dj, double s0, int J, double f0,
                          double level, int64_t mc_count, uint64_t seed, const void *surrogates,
                          int flags, double *sig95, uint64_t *hist_out);

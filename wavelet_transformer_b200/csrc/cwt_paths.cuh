@@ -58,11 +58,23 @@ int wct_fast(const float2 *d_xhat, int64_t pairs, int n0, double dt, const Axes 
              float4 *d_spec, const ScaleWin &win, float *d_wct, float *d_phase, float2 *d_w12,
              unsigned long long *d_hist, const int *d_tlo, const int *d_thi, int maxscale, cudaStream_t st);
 
-// cwt_long.cu: four-step transforms for the powers of two past one CTA's shared memory
+// cwt_long.cu: four-step transforms for the powers of two past one CTA's shared memory (long_fft.cuh)
 bool cwt_long_takes(int N, size_t elem);
+template <typename T> struct LongPlan;
+template <typename T> int long_plan(int N, cudaStream_t st, LongPlan<T> *p);
 template <typename T>
 int cwt_long(const T *d_x, int64_t batch, int n0, int N, double dt, const Axes &ax, const Mother &mo, int flags,
              T *d_power, cplx<T> *d_coef, cudaStream_t st);
+
+// wct_long.cu: the smoothed spectra tsm [pairs, S, n0] (when smooth), W12 and its phase of the interleaved
+// series d_y [pairs, 2, n0] at a length cwt_long_takes; scales, COI ranges (when h_tlo) and tsm live in its scratch.
+template <typename T> struct WctLongOut {
+  vec4<T> *tsm;
+  int *tlo, *thi;
+};
+template <typename T>
+int wct_long(const T *d_y, int64_t pairs, int n0, int N, double dt, const Axes &ax, double f0, bool smooth,
+             T *d_phase, cplx<T> *d_w12, const int *h_tlo, const int *h_thi, WctLongOut<T> *out, cudaStream_t st);
 
 // wct.cu: rows with at least one sample inside the reliable region (multi.cu's percentile step)
 void mc_row_has_points(int nsurr, double dt, const Axes &ax, double f0, std::vector<uint8_t> *any);

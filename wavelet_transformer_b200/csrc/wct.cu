@@ -19,11 +19,6 @@
 
 namespace wtb {
 
-template <typename T> struct vec4_of;
-template <> struct vec4_of<float> { using type = float4; };
-template <> struct vec4_of<double> { using type = double4; };
-template <typename T> using vec4 = typename vec4_of<T>::type;
-
 // One CTA = one (pair, scale).  smem: 3 * N complex (U, V, tmp).
 // xhat: [pairs, 2, N].  tsm: [pairs, S, n0] vec4.  phase/w12 optional [pairs,S,n0].
 template <typename T>
@@ -151,6 +146,21 @@ static int make_win(double dj, ScaleWin *win) {
   return WTB_OK;
 }
 
+// Scale boxcar and coherence of tsm [pairs, S, n0]: the plane, or the histogram when d_hist.
+template <typename T>
+static int wct_scale_pass(const vec4<T> *d_tsm, int64_t pairs, int n0, int S, const ScaleWin &win, T *d_wct,
+                          unsigned long long *d_hist, const int *d_tlo, const int *d_thi, int maxscale,
+                          cudaStream_t st) {
+  const int64_t cols = pairs * n0;
+  const unsigned blocks = (unsigned)((cols + 255) / 256);
+  if (d_hist)
+    k_wct_scale<T, 1><<<blocks, 256, 0, st>>>(d_tsm, pairs, n0, S, win, nullptr, d_hist, d_tlo, d_thi, maxscale);
+  else
+    k_wct_scale<T, 0><<<blocks, 256, 0, st>>>(d_tsm, pairs, n0, S, win, d_wct, nullptr, nullptr, nullptr, 0);
+  WTB_LAUNCH_CHECK();
+  return WTB_OK;
+}
+
 // Shared device pipeline.  d_y: [pairs, 2, n0] (series interleaved per pair).  generic: the generic kernels at
 // every shape (WTB_GENERIC_ONLY).
 template <typename T>
@@ -160,6 +170,18 @@ static int wct_device(const T *d_y, int64_t pairs, int n0, int N, double dt, dou
                       cudaStream_t st) {
   const int S = ax.J + 1;
   const bool smooth = d_wct || d_hist;
+  if (cwt_long_takes(N, sizeof(T))) {
+    // powers of two past one CTA's shared memory, up to 2^22: the four-step rows of wct_long.cu, then the same
+    // scale boxcar and coherence kernels (WTB_GENERIC_ONLY has no other kernels for these lengths)
+    ScaleWin win;
+    WTB_TRY(make_win(dj, &win));
+    WTB_REQUIRE(pairs * S < (1LL << 31) && pairs * 2 < (1LL << 31), WTB_EUNSUPPORTED, "batch too large");
+    WctLongOut<T> o;
+    WTB_TRY(wct_long<T>(d_y, pairs, n0, N, dt, ax, f0, smooth, d_phase, d_w12, d_hist ? h_tlo : nullptr,
+                        d_hist ? h_thi : nullptr, &o, st));
+    if (smooth) WTB_TRY(wct_scale_pass<T>(o.tsm, pairs, n0, S, win, d_wct, d_hist, o.tlo, o.thi, maxscale, st));
+    return WTB_OK;
+  }
   FftPlan<T> plan;
   WTB_TRY(make_plan<T>(N, &plan));
   const size_t smem_fwd = 2 * sizeof(cplx<T>) * (size_t)plan.M;
@@ -212,15 +234,7 @@ static int wct_device(const T *d_y, int64_t pairs, int n0, int N, double dt, dou
   k_wct_rows<T><<<(unsigned)(pairs * S), threads, smem_rows, st>>>(
       d_xhat, n0, plan, S, d_scales, dt, f0, d_tsm, d_phase, d_w12, smooth ? 1 : 0);
   WTB_LAUNCH_CHECK();
-  if (smooth) {
-    const int64_t cols = pairs * n0;
-    const unsigned blocks = (unsigned)((cols + 255) / 256);
-    if (d_hist)
-      k_wct_scale<T, 1><<<blocks, 256, 0, st>>>(d_tsm, pairs, n0, S, win, nullptr, d_hist, d_tlo, d_thi, maxscale);
-    else
-      k_wct_scale<T, 0><<<blocks, 256, 0, st>>>(d_tsm, pairs, n0, S, win, d_wct, nullptr, nullptr, nullptr, 0);
-    WTB_LAUNCH_CHECK();
-  }
+  if (smooth) WTB_TRY(wct_scale_pass<T>(d_tsm, pairs, n0, S, win, d_wct, d_hist, d_tlo, d_thi, maxscale, st));
   return WTB_OK;
 }
 

@@ -5,6 +5,11 @@
 
 namespace wtb {
 
+template <typename T> struct vec4_of;
+template <> struct vec4_of<float> { using type = float4; };
+template <> struct vec4_of<double> { using type = double4; };
+template <typename T> using vec4 = typename vec4_of<T>::type;
+
 constexpr int kMaxWin = 64;
 // Scale-axis boxcar of Morlet.smooth: out[i] = sum_k w[k] * T[i + up - k], rows outside
 // [0, S) count as zero and the window is not renormalised (scipy convolve2d 'same').
