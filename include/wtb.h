@@ -212,7 +212,15 @@ int wtb_rednoise(double a1, double a2, int nsurr, int64_t first, int64_t count,
                  uint64_t seed, int flags, void *out, void *stream);
 
 /* ---- MODWT: replaces src/modwt.py:126 modwt, :147 imodwt, :163 modwtmra --- */
-/* g = dec_lo, h = dec_hi (pywt.Wavelet taps, length L, NOT yet divided by
+/* Every filterbank entry point below (wtb_modwt .. wtb_waverec) takes any n.
+ * One CTA holds a series in shared memory while its buffers fit 227 KB: up to
+ * n = 14484 in FP64 / 29004 in FP32 for wtb_modwt, 9656 / 19336 for wtb_imodwt,
+ * 14524 / 29052 for wtb_modwtmra, wtb_modwtmra_taps and wtb_wavedec, about
+ * 14520 / 29050 output samples for wtb_waverec.  Longer series run level by
+ * level, one launch per level, with their intermediates in device scratch (the
+ * long path, which WTB_GENERIC_ONLY does not change).  The choice is made from
+ * the shape.
+ * g = dec_lo, h = dec_hi (pywt.Wavelet taps, length L, NOT yet divided by
  * sqrt 2).  x: [batch, n]; w: [batch, J+1, n] rows w_1..w_J, v_J. */
 int wtb_modwt(const void *x, int64_t batch, int n, const double *g, const double *h,
               int L, int J, int flags, void *w_out, void *stream);
@@ -226,7 +234,10 @@ int wtb_modwtmra(const void *w, int64_t batch, int n, const double *filt, int J,
  * each row runs the synthesis cascade G_1'..G_{j-1}' H_j' w_j, which equals the
  * correlation with the periodised equivalent filter.  Shapes the cascade
  * kernel does not cover (L not in {2,4,6,8}, dilated filter longer than n)
- * are served by building those filters on the host and correlating. */
+ * are served by building those filters on the host and correlating, up to
+ * the one-CTA length; longer rows run the cascade one level per launch for
+ * every row at once, without building the filters.  wtb_modwtmra past that
+ * length correlates over each row's non-zero taps only. */
 int wtb_modwtmra_taps(const void *w, int64_t batch, int n, const double *g,
                       const double *h, int L, int J, int flags, void *out,
                       void *stream);

@@ -4,7 +4,9 @@
 // One CTA owns one series.  The row is staged into shared memory with a 1-D TMA
 // bulk copy (cp.async.bulk + mbarrier) when it is 16-byte aligned, all pyramid
 // levels run out of shared memory, and only coefficients leave the SM.  These
-// paths are HBM-bound: bytes in = N, bytes out = (J+1) N per series.
+// paths are HBM-bound: bytes in = N, bytes out = (J+1) N per series.  A shape whose generic kernel would need more
+// than kSmemLimit of shared memory, its static tables included, runs level by level instead (filterbank_long.cu);
+// each *_impl decides that from the shape before any launch.
 #include "filterbank_common.cuh"
 
 namespace wtb {
@@ -239,6 +241,9 @@ static int modwt_impl(const void *x, int64_t batch, int n, const Taps &taps, int
                       cudaStream_t st) {
   const size_t smem = sizeof(T) * 2 * (size_t)((n + 3) & ~3);
   auto kern = taps.L == 8 ? k_modwt<T, 8> : taps.L == 4 ? k_modwt<T, 4> : taps.L == 2 ? k_modwt<T, 2> : k_modwt<T, 0>;
+  bool fits;
+  WTB_TRY(fits_one_cta(kern, smem, &fits));
+  if (!fits) return modwt_long<T>(x, batch, n, taps, J, flags, out, st);
   const bool fast = !(flags & WTB_GENERIC_ONLY) && fast_taps_ok(taps.L);
   if (!fast) WTB_TRY(set_smem(kern, smem));
   return run_batched(x, out, batch, sizeof(T) * n, sizeof(T) * (size_t)(J + 1) * n, flags, st,
@@ -259,6 +264,9 @@ static int imodwt_impl(const void *w, int64_t batch, int n, const Taps &taps, in
                        cudaStream_t st) {
   const size_t smem = sizeof(T) * 3 * (size_t)((n + 3) & ~3);
   auto kern = taps.L == 8 ? k_imodwt<T, 8> : taps.L == 4 ? k_imodwt<T, 4> : taps.L == 2 ? k_imodwt<T, 2> : k_imodwt<T, 0>;
+  bool fits;
+  WTB_TRY(fits_one_cta(kern, smem, &fits));
+  if (!fits) return imodwt_long<T>(w, batch, n, taps, J, flags, out, st);
   const bool fast = !(flags & WTB_GENERIC_ONLY) && fast_taps_ok(taps.L);
   if (!fast) WTB_TRY(set_smem(kern, smem));
   return run_batched(w, out, batch, sizeof(T) * (size_t)(J + 1) * n, sizeof(T) * n, flags, st,
@@ -278,6 +286,9 @@ template <typename T>
 static int mra_impl(const void *w, int64_t batch, int n, const double *filt, int J, int flags, void *out,
                     cudaStream_t st) {
   const size_t smem = sizeof(T) * 2 * (size_t)((n + 3) & ~3);
+  bool fits;
+  WTB_TRY(fits_one_cta(k_modwtmra<T>, smem, &fits));
+  if (!fits) return mra_filt_long<T>(w, batch, n, filt, J, flags, out, st);
   WTB_TRY(set_smem(k_modwtmra<T>, smem));
   // effective filter length per level (trailing zeros of the periodised filter are skipped)
   std::vector<int> flen(J + 1);
@@ -338,6 +349,12 @@ template <typename T>
 static int mra_taps_impl(const void *w, int64_t batch, int n, const Taps &taps, const double *g, const double *h,
                          int J, int flags, void *out, cudaStream_t st) {
   const size_t row = sizeof(T) * (size_t)(J + 1) * n;
+  // neither the cascade kernel nor mra_impl's one CTA holds the row: the cascade level by level, without the
+  // equivalent filters
+  bool fits;
+  WTB_TRY(fits_one_cta(k_modwtmra<T>, sizeof(T) * 2 * (size_t)((n + 3) & ~3), &fits));
+  if (!fits && !(!(flags & WTB_GENERIC_ONLY) && mra_fast_covers(n, taps.L, J, sizeof(T))))
+    return mra_taps_long<T>(w, batch, n, taps, J, flags, out, st);
   bool covered = !(flags & WTB_GENERIC_ONLY) && fast_taps_ok(taps.L);
   if (covered) {
     int rc = run_batched(w, out, batch, row, row, flags, st, [&](const void *di, void *dout, int64_t nb) -> int {
@@ -377,6 +394,9 @@ static int wavedec_impl(const void *x, int64_t batch, int n, const Taps &taps, i
   WTB_TRY(make_plan(n, taps.L, level, nullptr, &plan));
   plan.buf = (n + 3) & ~3;
   const size_t smem = sizeof(T) * 2 * (size_t)plan.buf;
+  bool fits;
+  WTB_TRY(fits_one_cta(k_wavedec<T>, smem, &fits));
+  if (!fits) return wavedec_long<T>(x, batch, plan, taps, flags, coeffs, st);
   const bool fast = !(flags & WTB_GENERIC_ONLY) && fast_taps_ok(taps.L);
   if (!fast) WTB_TRY(set_smem(k_wavedec<T>, smem));
   return run_batched(x, coeffs, batch, sizeof(T) * n, sizeof(T) * (size_t)plan.total, flags, st,
@@ -403,6 +423,9 @@ static int waverec_impl(const void *coeffs, int64_t batch, const int *lens, int 
   for (int i = 0; i <= level; ++i) longest = std::max(longest, plan.len[i]);
   plan.buf = (longest + taps.L + 3) & ~3;
   const size_t smem = sizeof(T) * 2 * (size_t)plan.buf;
+  bool fits;
+  WTB_TRY(fits_one_cta(k_waverec<T>, smem, &fits));
+  if (!fits) return waverec_long<T>(coeffs, batch, plan, taps, flags, x, st);
   const bool fast = !(flags & WTB_GENERIC_ONLY) && fast_taps_ok(taps.L);
   if (!fast) WTB_TRY(set_smem(k_waverec<T>, smem));
   return run_batched(coeffs, x, batch, sizeof(T) * (size_t)plan.total, sizeof(T) * (size_t)nout, flags, st,

@@ -143,6 +143,15 @@ template <typename K> static int set_smem(K kernel, size_t bytes) {
   return WTB_OK;
 }
 
+// Whether `kernel` runs with `dyn` bytes of dynamic shared memory: its static shared memory (tap tables, barrier)
+// counts against the same 227 KB.  A shape whose generic kernel does not fit runs the long path (filterbank_long.cu).
+template <typename K> static int fits_one_cta(K kernel, size_t dyn, bool *fits) {
+  cudaFuncAttributes a;
+  WTB_CUDA(cudaFuncGetAttributes(&a, kernel));
+  *fits = dyn + a.sharedSizeBytes <= kSmemLimit;
+  return WTB_OK;
+}
+
 // ---- register-blocked kernels (filterbank_fast.cu); each returns WTB_OK after launching or
 // WTB_EUNSUPPORTED (without setting an error) when the shape is not covered, in which case
 // the caller falls back to the generic kernels of filterbank.cu ---------------------------
@@ -158,6 +167,27 @@ int wavedec_fast(const void *x, int64_t batch, const LevelPlan &plan, const Taps
                  cudaStream_t st);
 template <typename T>
 int waverec_fast(const void *coeffs, int64_t batch, const LevelPlan &plan, const Taps &taps, void *x,
+                 cudaStream_t st);
+// whether mra_fast serves this shape (any batch the one-CTA kernels are asked for), decided without a launch
+bool mra_fast_covers(int n, int L, int J, size_t elem);
+
+// ---- long series (filterbank_long.cu): one launch per level per wave of series, for the shapes whose generic
+// kernel above needs more than kSmemLimit of shared memory.  Each runs the whole call, host chunks included ----
+template <typename T>
+int modwt_long(const void *x, int64_t batch, int n, const Taps &taps, int J, int flags, void *out, cudaStream_t st);
+template <typename T>
+int imodwt_long(const void *w, int64_t batch, int n, const Taps &taps, int J, int flags, void *out, cudaStream_t st);
+template <typename T>
+int mra_taps_long(const void *w, int64_t batch, int n, const Taps &taps, int J, int flags, void *out,
+                  cudaStream_t st);
+template <typename T>
+int mra_filt_long(const void *w, int64_t batch, int n, const double *filt, int J, int flags, void *out,
+                  cudaStream_t st);
+template <typename T>
+int wavedec_long(const void *x, int64_t batch, const LevelPlan &plan, const Taps &taps, int flags, void *coeffs,
+                 cudaStream_t st);
+template <typename T>
+int waverec_long(const void *coeffs, int64_t batch, const LevelPlan &plan, const Taps &taps, int flags, void *x,
                  cudaStream_t st);
 
 }  // namespace wtb

@@ -636,12 +636,27 @@ int imodwt_fast(const void *w, int64_t batch, int n, const Taps &taps, int J, vo
   return WTB_OK;
 }
 
+// shared memory of k_mra_blk<T, L, R> (elem = sizeof(T)) for this shape; 0 when its chains do not cover it
+static size_t mra_blk_smem(int n, int L, int J, int R, size_t elem) {
+  if (!chain_threads(n, L, J, R)) return 0;
+  return elem * (size_t)((n + (R + L - 2) * (1 << (J - 1)) + 4 + 3) & ~3);
+}
+
+// mra_fast's choice below, without a launch (its batch * (J + 1) < 2^31 test cannot fail at a length that the
+// generic kernel's shared memory refuses)
+bool mra_fast_covers(int n, int L, int J, size_t elem) {
+  auto fits = [&](int R) {
+    const size_t smem = mra_blk_smem(n, L, J, R, elem);
+    return smem && smem <= kSmemLimit;
+  };
+  return fast_taps_ok(L) && ((n >= kLongRow && fits(kRA)) || fits(kRM));
+}
+
 template <typename T, int R>
 static int mra_fast_r(const void *w, int64_t batch, int n, const Taps &taps, int J, void *out, cudaStream_t st) {
   const int threads = chain_threads(n, taps.L, J, R);
-  if (!threads) return WTB_EUNSUPPORTED;
-  const size_t smem = sizeof(T) * (size_t)((n + (R + taps.L - 2) * (1 << (J - 1)) + 4 + 3) & ~3);
-  if (smem > kSmemLimit) return WTB_EUNSUPPORTED;
+  const size_t smem = mra_blk_smem(n, taps.L, J, R, sizeof(T));
+  if (!smem || smem > kSmemLimit) return WTB_EUNSUPPORTED;
   WTB_TAPS_SWITCH(taps.L, {
     WTB_TRY(set_smem(k_mra_blk<T, LT, R>, smem));
     k_mra_blk<T, LT, R><<<(unsigned)(batch * (J + 1)), threads, smem, st>>>((const T *)w, n, J,
