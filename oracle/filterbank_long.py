@@ -12,8 +12,8 @@ definitions at short lengths, and tests/test_oracle_filterbank_long.py holds the
   sum_j j L gathers per sample.
 * ``modwt`` / ``imodwt`` are modwt_oracle's, which already gather one tap at a time.
 
-The replica mirrors filterbank.cu / filterbank_long.cu: ``route`` says whether a call takes the long path,
-``launches`` how many kernels it runs there.
+The replica mirrors filterbank.cu's ``fb_plan`` and filterbank_long.cu: ``route`` says whether a call takes the long
+path, ``launches`` how many kernels it runs there.
 """
 
 from __future__ import annotations
@@ -131,7 +131,8 @@ def _chain_threads(n, L, J, R):
 
 
 def mra_fast_covers(n, L, J, f64):
-    """filterbank_fast.cu mra_fast_covers: the MRA cascade kernel k_mra_blk serves the shape."""
+    """filterbank_fast.cu blk_shape(FbOp::kMraTaps, ...).threads != 0: the MRA cascade kernel k_mra_blk serves the
+    shape."""
     def fits(R):
         return _chain_threads(n, L, J, R) and _elem(f64) * _ceil4(n + (R + L - 2) * (1 << (J - 1)) + 4) <= SMEM_LIMIT
     return L in (2, 4, 6, 8) and ((n >= 2048 and fits(17)) or fits(9))
@@ -155,7 +156,7 @@ def waverec_len(lens, L):
 
 
 # Static shared memory of the generic one-CTA kernels (ptxas: tap tables and mbarrier, padded to 16 B), FP32 / FP64.
-# It counts against the 227 KB with the dynamic buffers: fits_one_cta in filterbank_common.cuh.
+# It counts against the 227 KB with the dynamic buffers: fits_one_cta, called by fb_plan in filterbank.cu.
 STATIC_SMEM = {"modwt": (400, 656), "imodwt": (400, 656), "modwtmra": (16, 16), "modwtmra_taps": (16, 16),
                "wavedec": (16, 16), "waverec": (0, 0)}
 

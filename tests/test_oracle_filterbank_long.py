@@ -55,7 +55,7 @@ def test_first_long_lengths(key):
 
 
 def test_mra_cascade_kernel_never_reaches_the_long_lengths():
-    """mra_fast declines every length past the generic kernel's limit, so the long MRA starts where that limit is."""
+    """blk_shape covers no MRA length past the generic kernel's limit, so the long MRA starts where that limit is."""
     for f64 in (False, True):
         for L in (2, 4, 6, 8):
             for J in range(1, 11):

@@ -236,24 +236,48 @@ static int make_taps(const double *lo, const double *hi, int L, double scale, Ta
 
 static int threads_for(int n) { return n >= 2048 ? 512 : (n >= 512 ? 256 : 128); }
 
+enum class FbPath { kBlocked, kGeneric, kLong };
+struct FbPlan { FbPath path; BlkShape cta; };  // cta: the launch of the chosen one-CTA kernel
+
+// The kernels for a call of `op` on series of n samples (DWT: of *dwt, whose buf it sets), from the shape alone:
+// kBlocked (filterbank_fast.cu) where blk_shape covers the shape, unless WTB_GENERIC_ONLY; else kGeneric, the
+// one-CTA kernel `generic` (for the MRA from taps: k_modwtmra with the host-built equivalent filters), if it fits
+// kSmemLimit with its static shared memory; else kLong (filterbank_long.cu).  The blocked kernels are asked only
+// where `generic` fits, except for the MRA from taps, whose cascade kernel keeps every shape it covers.
+template <typename T, typename K>
+static int fb_plan(FbOp op, K generic, int n, int L, int J, LevelPlan *dwt, int flags, FbPlan *p) {
+  int buf = (n + 3) & ~3;  // generic kernels: two ping-pong buffers, three for the inverse MODWT
+  if (op == FbOp::kWaverec) {
+    int longest = n;
+    for (int i = 0; i <= dwt->level; ++i) longest = std::max(longest, dwt->len[i]);
+    buf = (longest + L + 3) & ~3;
+  }
+  const size_t smem = sizeof(T) * (op == FbOp::kImodwt ? 3 : 2) * (size_t)buf;
+  bool fits;
+  WTB_TRY(fits_one_cta(generic, smem, &fits));
+  const bool ask = !(flags & WTB_GENERIC_ONLY) && (fits || op == FbOp::kMraTaps);
+  const BlkShape blk = ask ? blk_shape(op, n, L, J, dwt, sizeof(T)) : BlkShape{};
+  *p = {FbPath::kGeneric, {threads_for(n), smem, 0, buf}};
+  if (blk.threads)
+    *p = {FbPath::kBlocked, blk};
+  else if (!fits)
+    p->path = FbPath::kLong;
+  if (dwt) dwt->buf = p->cta.buf;
+  return WTB_OK;
+}
+
 template <typename T>
 static int modwt_impl(const void *x, int64_t batch, int n, const Taps &taps, int J, int flags, void *out,
                       cudaStream_t st) {
-  const size_t smem = sizeof(T) * 2 * (size_t)((n + 3) & ~3);
   auto kern = taps.L == 8 ? k_modwt<T, 8> : taps.L == 4 ? k_modwt<T, 4> : taps.L == 2 ? k_modwt<T, 2> : k_modwt<T, 0>;
-  bool fits;
-  WTB_TRY(fits_one_cta(kern, smem, &fits));
-  if (!fits) return modwt_long<T>(x, batch, n, taps, J, flags, out, st);
-  const bool fast = !(flags & WTB_GENERIC_ONLY) && fast_taps_ok(taps.L);
-  if (!fast) WTB_TRY(set_smem(kern, smem));
+  FbPlan p;
+  WTB_TRY(fb_plan<T>(FbOp::kModwt, kern, n, taps.L, J, nullptr, flags, &p));
+  if (p.path == FbPath::kLong) return modwt_long<T>(x, batch, n, taps, J, flags, out, st);
+  if (p.path == FbPath::kGeneric) WTB_TRY(set_smem(kern, p.cta.smem));
   return run_batched(x, out, batch, sizeof(T) * n, sizeof(T) * (size_t)(J + 1) * n, flags, st,
                      [&](const void *di, void *dout, int64_t nb) -> int {
-                       if (fast) {
-                         const int rc = modwt_fast<T>(di, nb, n, taps, J, dout, st);
-                         if (rc != WTB_EUNSUPPORTED) return rc;
-                         WTB_TRY(set_smem(kern, smem));
-                       }
-                       kern<<<(unsigned)nb, threads_for(n), smem, st>>>((const T *)di, n, J, taps, (T *)dout);
+                       if (p.path == FbPath::kBlocked) return modwt_fast<T>(p.cta, di, nb, n, taps, J, dout, st);
+                       kern<<<(unsigned)nb, p.cta.threads, p.cta.smem, st>>>((const T *)di, n, J, taps, (T *)dout);
                        WTB_LAUNCH_CHECK();
                        return WTB_OK;
                      });
@@ -262,34 +286,25 @@ static int modwt_impl(const void *x, int64_t batch, int n, const Taps &taps, int
 template <typename T>
 static int imodwt_impl(const void *w, int64_t batch, int n, const Taps &taps, int J, int flags, void *out,
                        cudaStream_t st) {
-  const size_t smem = sizeof(T) * 3 * (size_t)((n + 3) & ~3);
   auto kern = taps.L == 8 ? k_imodwt<T, 8> : taps.L == 4 ? k_imodwt<T, 4> : taps.L == 2 ? k_imodwt<T, 2> : k_imodwt<T, 0>;
-  bool fits;
-  WTB_TRY(fits_one_cta(kern, smem, &fits));
-  if (!fits) return imodwt_long<T>(w, batch, n, taps, J, flags, out, st);
-  const bool fast = !(flags & WTB_GENERIC_ONLY) && fast_taps_ok(taps.L);
-  if (!fast) WTB_TRY(set_smem(kern, smem));
+  FbPlan p;
+  WTB_TRY(fb_plan<T>(FbOp::kImodwt, kern, n, taps.L, J, nullptr, flags, &p));
+  if (p.path == FbPath::kLong) return imodwt_long<T>(w, batch, n, taps, J, flags, out, st);
+  if (p.path == FbPath::kGeneric) WTB_TRY(set_smem(kern, p.cta.smem));
   return run_batched(w, out, batch, sizeof(T) * (size_t)(J + 1) * n, sizeof(T) * n, flags, st,
                      [&](const void *di, void *dout, int64_t nb) -> int {
-                       if (fast) {
-                         const int rc = imodwt_fast<T>(di, nb, n, taps, J, dout, st);
-                         if (rc != WTB_EUNSUPPORTED) return rc;
-                         WTB_TRY(set_smem(kern, smem));
-                       }
-                       kern<<<(unsigned)nb, threads_for(n), smem, st>>>((const T *)di, n, J, taps, (T *)dout);
+                       if (p.path == FbPath::kBlocked) return imodwt_fast<T>(p.cta, di, nb, n, taps, J, dout, st);
+                       kern<<<(unsigned)nb, p.cta.threads, p.cta.smem, st>>>((const T *)di, n, J, taps, (T *)dout);
                        WTB_LAUNCH_CHECK();
                        return WTB_OK;
                      });
 }
 
+// k_modwtmra over the batch with the periodised filters filt [J+1, n] (host), on a kGeneric plan
 template <typename T>
-static int mra_impl(const void *w, int64_t batch, int n, const double *filt, int J, int flags, void *out,
-                    cudaStream_t st) {
-  const size_t smem = sizeof(T) * 2 * (size_t)((n + 3) & ~3);
-  bool fits;
-  WTB_TRY(fits_one_cta(k_modwtmra<T>, smem, &fits));
-  if (!fits) return mra_filt_long<T>(w, batch, n, filt, J, flags, out, st);
-  WTB_TRY(set_smem(k_modwtmra<T>, smem));
+static int mra_generic(const FbPlan &p, const void *w, int64_t batch, int n, const double *filt, int J, int flags,
+                       void *out, cudaStream_t st) {
+  WTB_TRY(set_smem(k_modwtmra<T>, p.cta.smem));
   // effective filter length per level (trailing zeros of the periodised filter are skipped)
   std::vector<int> flen(J + 1);
   for (int j = 0; j <= J; ++j) {
@@ -308,10 +323,19 @@ static int mra_impl(const void *w, int64_t batch, int n, const double *filt, int
   const size_t row = sizeof(T) * (size_t)(J + 1) * n;
   return run_batched(w, out, batch, row, row, flags, st, [&](const void *di, void *dout, int64_t nb) -> int {
     WTB_REQUIRE(nb * (J + 1) < (1LL << 31), WTB_EUNSUPPORTED, "batch too large");
-    k_modwtmra<T><<<(unsigned)(nb * (J + 1)), threads_for(n), smem, st>>>((const T *)di, n, J, d_filt, d_flen, (T *)dout);
+    k_modwtmra<T><<<(unsigned)(nb * (J + 1)), p.cta.threads, p.cta.smem, st>>>((const T *)di, n, J, d_filt, d_flen, (T *)dout);
     WTB_LAUNCH_CHECK();
     return WTB_OK;
   });
+}
+
+template <typename T>
+static int mra_impl(const void *w, int64_t batch, int n, const double *filt, int J, int flags, void *out,
+                    cudaStream_t st) {
+  FbPlan p;
+  WTB_TRY(fb_plan<T>(FbOp::kMra, k_modwtmra<T>, n, 0, J, nullptr, flags, &p));
+  if (p.path == FbPath::kLong) return mra_filt_long<T>(w, batch, n, filt, J, flags, out, st);
+  return mra_generic<T>(p, w, batch, n, filt, J, flags, out, st);
 }
 
 // Periodised equivalent filters [h_1 .. h_J, g_J] of the reference's modwtmra
@@ -348,24 +372,19 @@ static void equivalent_filters(const double *g, const double *h, int L, int J, i
 template <typename T>
 static int mra_taps_impl(const void *w, int64_t batch, int n, const Taps &taps, const double *g, const double *h,
                          int J, int flags, void *out, cudaStream_t st) {
-  const size_t row = sizeof(T) * (size_t)(J + 1) * n;
-  // neither the cascade kernel nor mra_impl's one CTA holds the row: the cascade level by level, without the
-  // equivalent filters
-  bool fits;
-  WTB_TRY(fits_one_cta(k_modwtmra<T>, sizeof(T) * 2 * (size_t)((n + 3) & ~3), &fits));
-  if (!fits && !(!(flags & WTB_GENERIC_ONLY) && mra_fast_covers(n, taps.L, J, sizeof(T))))
-    return mra_taps_long<T>(w, batch, n, taps, J, flags, out, st);
-  bool covered = !(flags & WTB_GENERIC_ONLY) && fast_taps_ok(taps.L);
-  if (covered) {
-    int rc = run_batched(w, out, batch, row, row, flags, st, [&](const void *di, void *dout, int64_t nb) -> int {
-      return mra_fast<T>(di, nb, n, taps, J, dout, st);
-    });
-    if (rc != WTB_EUNSUPPORTED) return rc;
+  FbPlan p;
+  WTB_TRY(fb_plan<T>(FbOp::kMraTaps, k_modwtmra<T>, n, taps.L, J, nullptr, flags, &p));
+  if (p.path == FbPath::kLong) return mra_taps_long<T>(w, batch, n, taps, J, flags, out, st);
+  if (p.path == FbPath::kGeneric) {  // shape outside the cascade kernel: correlate with the periodised filters
+    std::vector<double> filt;
+    equivalent_filters(g, h, taps.L, J, n, &filt);
+    return mra_generic<T>(p, w, batch, n, filt.data(), J, flags, out, st);
   }
-  // shape outside the cascade kernel: correlate with the host-built periodised filters
-  std::vector<double> filt;
-  equivalent_filters(g, h, taps.L, J, n, &filt);
-  return mra_impl<T>(w, batch, n, filt.data(), J, flags, out, st);
+  const size_t row = sizeof(T) * (size_t)(J + 1) * n;
+  return run_batched(w, out, batch, row, row, flags, st, [&](const void *di, void *dout, int64_t nb) -> int {
+    WTB_REQUIRE(nb * (J + 1) < (1LL << 31), WTB_EUNSUPPORTED, "batch too large");
+    return mra_fast<T>(p.cta, di, nb, n, taps, J, dout, st);
+  });
 }
 
 static int make_plan(int n, int L, int level, const int *lens_in, LevelPlan *p) {
@@ -392,21 +411,14 @@ static int wavedec_impl(const void *x, int64_t batch, int n, const Taps &taps, i
                         void *coeffs, cudaStream_t st) {
   LevelPlan plan;
   WTB_TRY(make_plan(n, taps.L, level, nullptr, &plan));
-  plan.buf = (n + 3) & ~3;
-  const size_t smem = sizeof(T) * 2 * (size_t)plan.buf;
-  bool fits;
-  WTB_TRY(fits_one_cta(k_wavedec<T>, smem, &fits));
-  if (!fits) return wavedec_long<T>(x, batch, plan, taps, flags, coeffs, st);
-  const bool fast = !(flags & WTB_GENERIC_ONLY) && fast_taps_ok(taps.L);
-  if (!fast) WTB_TRY(set_smem(k_wavedec<T>, smem));
+  FbPlan p;
+  WTB_TRY(fb_plan<T>(FbOp::kWavedec, k_wavedec<T>, n, taps.L, level, &plan, flags, &p));
+  if (p.path == FbPath::kLong) return wavedec_long<T>(x, batch, plan, taps, flags, coeffs, st);
+  if (p.path == FbPath::kGeneric) WTB_TRY(set_smem(k_wavedec<T>, p.cta.smem));
   return run_batched(x, coeffs, batch, sizeof(T) * n, sizeof(T) * (size_t)plan.total, flags, st,
                      [&](const void *di, void *dout, int64_t nb) -> int {
-                       if (fast) {
-                         const int rc = wavedec_fast<T>(di, nb, plan, taps, dout, st);
-                         if (rc != WTB_EUNSUPPORTED) return rc;
-                         WTB_TRY(set_smem(k_wavedec<T>, smem));
-                       }
-                       k_wavedec<T><<<(unsigned)nb, threads_for(n), smem, st>>>((const T *)di, plan, taps, (T *)dout);
+                       if (p.path == FbPath::kBlocked) return wavedec_fast<T>(p.cta, di, nb, plan, taps, dout, st);
+                       k_wavedec<T><<<(unsigned)nb, p.cta.threads, p.cta.smem, st>>>((const T *)di, plan, taps, (T *)dout);
                        WTB_LAUNCH_CHECK();
                        return WTB_OK;
                      });
@@ -419,23 +431,14 @@ static int waverec_impl(const void *coeffs, int64_t batch, const int *lens, int 
   if (nout < 0) return nout;
   LevelPlan plan;
   WTB_TRY(make_plan(nout, taps.L, level, lens, &plan));
-  int longest = nout;
-  for (int i = 0; i <= level; ++i) longest = std::max(longest, plan.len[i]);
-  plan.buf = (longest + taps.L + 3) & ~3;
-  const size_t smem = sizeof(T) * 2 * (size_t)plan.buf;
-  bool fits;
-  WTB_TRY(fits_one_cta(k_waverec<T>, smem, &fits));
-  if (!fits) return waverec_long<T>(coeffs, batch, plan, taps, flags, x, st);
-  const bool fast = !(flags & WTB_GENERIC_ONLY) && fast_taps_ok(taps.L);
-  if (!fast) WTB_TRY(set_smem(k_waverec<T>, smem));
+  FbPlan p;
+  WTB_TRY(fb_plan<T>(FbOp::kWaverec, k_waverec<T>, nout, taps.L, level, &plan, flags, &p));
+  if (p.path == FbPath::kLong) return waverec_long<T>(coeffs, batch, plan, taps, flags, x, st);
+  if (p.path == FbPath::kGeneric) WTB_TRY(set_smem(k_waverec<T>, p.cta.smem));
   return run_batched(coeffs, x, batch, sizeof(T) * (size_t)plan.total, sizeof(T) * (size_t)nout, flags, st,
                      [&](const void *di, void *dout, int64_t nb) -> int {
-                       if (fast) {
-                         const int rc = waverec_fast<T>(di, nb, plan, taps, dout, st);
-                         if (rc != WTB_EUNSUPPORTED) return rc;
-                         WTB_TRY(set_smem(k_waverec<T>, smem));
-                       }
-                       k_waverec<T><<<(unsigned)nb, threads_for(nout), smem, st>>>((const T *)di, plan, taps, (T *)dout);
+                       if (p.path == FbPath::kBlocked) return waverec_fast<T>(p.cta, di, nb, plan, taps, dout, st);
+                       k_waverec<T><<<(unsigned)nb, p.cta.threads, p.cta.smem, st>>>((const T *)di, plan, taps, (T *)dout);
                        WTB_LAUNCH_CHECK();
                        return WTB_OK;
                      });

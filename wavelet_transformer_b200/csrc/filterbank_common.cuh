@@ -152,24 +152,26 @@ template <typename K> static int fits_one_cta(K kernel, size_t dyn, bool *fits) 
   return WTB_OK;
 }
 
-// ---- register-blocked kernels (filterbank_fast.cu); each returns WTB_OK after launching or
-// WTB_EUNSUPPORTED (without setting an error) when the shape is not covered, in which case
-// the caller falls back to the generic kernels of filterbank.cu ---------------------------
-inline bool fast_taps_ok(int L) { return L == 2 || L == 4 || L == 6 || L == 8; }
-template <typename T>
-int modwt_fast(const void *x, int64_t batch, int n, const Taps &taps, int J, void *out, cudaStream_t st);
-template <typename T>
-int imodwt_fast(const void *w, int64_t batch, int n, const Taps &taps, int J, void *out, cudaStream_t st);
-template <typename T>
-int mra_fast(const void *w, int64_t batch, int n, const Taps &taps, int J, void *out, cudaStream_t st);
-template <typename T>
-int wavedec_fast(const void *x, int64_t batch, const LevelPlan &plan, const Taps &taps, void *coeffs,
-                 cudaStream_t st);
-template <typename T>
-int waverec_fast(const void *coeffs, int64_t batch, const LevelPlan &plan, const Taps &taps, void *x,
-                 cudaStream_t st);
-// whether mra_fast serves this shape (any batch the one-CTA kernels are asked for), decided without a launch
-bool mra_fast_covers(int n, int L, int J, size_t elem);
+// wtb_modwt, wtb_imodwt, wtb_modwtmra, wtb_modwtmra_taps, wtb_wavedec, wtb_waverec
+enum class FbOp { kModwt, kImodwt, kMra, kMraTaps, kWavedec, kWaverec };
+// One-CTA launch of a shape: CTA size (0: not covered), dynamic shared memory, k_mra_blk's chain length R and the
+// DWT's LevelPlan::buf
+struct BlkShape { int threads; size_t smem; int R, buf; };
+
+// ---- register-blocked kernels (filterbank_fast.cu).  blk_shape: whether they cover a shape and how they launch
+// for it, from host arithmetic alone (`dwt`: the DWT ops' level plan, read instead of n and J; nullptr for the
+// others).  The launchers take its result and launch ----------------------------------------------------------------
+BlkShape blk_shape(FbOp op, int n, int L, int J, const LevelPlan *dwt, size_t elem);
+template <typename T> int modwt_fast(const BlkShape &s, const void *x, int64_t batch, int n, const Taps &taps, int J,
+                                     void *out, cudaStream_t st);
+template <typename T> int imodwt_fast(const BlkShape &s, const void *w, int64_t batch, int n, const Taps &taps, int J,
+                                      void *out, cudaStream_t st);
+template <typename T> int mra_fast(const BlkShape &s, const void *w, int64_t batch, int n, const Taps &taps, int J,
+                                   void *out, cudaStream_t st);
+template <typename T> int wavedec_fast(const BlkShape &s, const void *x, int64_t batch, const LevelPlan &plan,
+                                       const Taps &taps, void *coeffs, cudaStream_t st);
+template <typename T> int waverec_fast(const BlkShape &s, const void *coeffs, int64_t batch, const LevelPlan &plan,
+                                       const Taps &taps, void *x, cudaStream_t st);
 
 // ---- long series (filterbank_long.cu): one launch per level per wave of series, for the shapes whose generic
 // kernel above needs more than kSmemLimit of shared memory.  Each runs the whole call, host chunks included ----

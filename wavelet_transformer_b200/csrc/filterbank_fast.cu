@@ -588,7 +588,7 @@ static int round_threads(int64_t items) {
     case 4: { constexpr int LT = 4; __VA_ARGS__; } break;   \
     case 6: { constexpr int LT = 6; __VA_ARGS__; } break;   \
     case 8: { constexpr int LT = 8; __VA_ARGS__; } break;   \
-    default: return WTB_EUNSUPPORTED;                       \
+    default: return WTB_EUNSUPPORTED; /* unreachable: blk_shape covers these L only */ \
   }
 
 // CTA size for the a-trous kernels: one chain per thread at every level.  0 = not coverable:
@@ -604,131 +604,124 @@ static int chain_threads(int n, int L, int J, int R = kRM) {
   return most <= kChainThreads ? round_threads(most) : 0;
 }
 
-template <typename T>
-int modwt_fast(const void *x, int64_t batch, int n, const Taps &taps, int J, void *out, cudaStream_t st) {
-  if (!fast_taps_ok(taps.L)) return WTB_EUNSUPPORTED;
-  const int threads = chain_threads(n, taps.L, J);
-  if (!threads) return WTB_EUNSUPPORTED;
-  const size_t v_len = (size_t)halo_of(taps.L, J - 1) + (size_t)((n + (kRM - 1) * (1 << (J - 1)) + 4 + 3) & ~3);
-  const size_t smem = sizeof(T) * (v_len + (size_t)((n + 4 + 3) & ~3));
-  if (smem > kSmemLimit) return WTB_EUNSUPPORTED;
-  WTB_TAPS_SWITCH(taps.L, {
-    WTB_TRY(set_smem(k_modwt_blk<T, LT>, smem));
-    k_modwt_blk<T, LT><<<(unsigned)batch, threads, smem, st>>>((const T *)x, n, J, narrow_taps<T, LT>(taps), (T *)out);
-  });
-  WTB_LAUNCH_CHECK();
-  return WTB_OK;
-}
-
-template <typename T>
-int imodwt_fast(const void *w, int64_t batch, int n, const Taps &taps, int J, void *out, cudaStream_t st) {
-  if (!fast_taps_ok(taps.L)) return WTB_EUNSUPPORTED;
-  const int threads = chain_threads(n, taps.L, J);
-  if (!threads) return WTB_EUNSUPPORTED;
-  const size_t np = (size_t)((n + (kRM + taps.L - 2) * (1 << (J - 1)) + 4 + 3) & ~3);
-  const size_t smem = sizeof(T) * 3 * np;
-  if (smem > kSmemLimit) return WTB_EUNSUPPORTED;
-  WTB_TAPS_SWITCH(taps.L, {
-    WTB_TRY(set_smem(k_imodwt_blk<T, LT>, smem));
-    k_imodwt_blk<T, LT><<<(unsigned)batch, threads, smem, st>>>((const T *)w, n, J, narrow_taps<T, LT>(taps), (T *)out);
-  });
-  WTB_LAUNCH_CHECK();
-  return WTB_OK;
-}
-
-// shared memory of k_mra_blk<T, L, R> (elem = sizeof(T)) for this shape; 0 when its chains do not cover it
-static size_t mra_blk_smem(int n, int L, int J, int R, size_t elem) {
-  if (!chain_threads(n, L, J, R)) return 0;
-  return elem * (size_t)((n + (R + L - 2) * (1 << (J - 1)) + 4 + 3) & ~3);
-}
-
-// mra_fast's choice below, without a launch (its batch * (J + 1) < 2^31 test cannot fail at a length that the
-// generic kernel's shared memory refuses)
-bool mra_fast_covers(int n, int L, int J, size_t elem) {
-  auto fits = [&](int R) {
-    const size_t smem = mra_blk_smem(n, L, J, R, elem);
-    return smem && smem <= kSmemLimit;
+BlkShape blk_shape(FbOp op, int n, int L, int J, const LevelPlan *dwt, size_t elem) {
+  if (L != 2 && L != 4 && L != 6 && L != 8) return {};
+  BlkShape s{};
+  auto mra = [&](int R) {  // k_mra_blk<T, L, R>
+    BlkShape m{chain_threads(n, L, J, R), 0, R, 0};
+    if (m.threads) m.smem = elem * (size_t)((n + (R + L - 2) * (1 << (J - 1)) + 4 + 3) & ~3);
+    return m.threads && m.smem <= kSmemLimit ? m : BlkShape{};
   };
-  return fast_taps_ok(L) && ((n >= kLongRow && fits(kRA)) || fits(kRM));
+  switch (op) {
+    case FbOp::kModwt:
+      s.threads = chain_threads(n, L, J);
+      if (!s.threads) return {};
+      s.smem = elem * ((size_t)halo_of(L, J - 1) + (size_t)((n + (kRM - 1) * (1 << (J - 1)) + 4 + 3) & ~3) +
+                       (size_t)((n + 4 + 3) & ~3));
+      break;
+    case FbOp::kImodwt:
+      s.threads = chain_threads(n, L, J);
+      if (!s.threads) return {};
+      s.smem = elem * 3 * (size_t)((n + (kRM + L - 2) * (1 << (J - 1)) + 4 + 3) & ~3);
+      break;
+    case FbOp::kMraTaps: {
+      // chains of kRA on long rows, unless the longer chains' halo no longer fits
+      const BlkShape r = n >= kLongRow ? mra(kRA) : BlkShape{};
+      return r.threads ? r : mra(kRM);
+    }
+    case FbOp::kWavedec: {
+      // every level's input must hold one whole mirror image of the filter overhang
+      int cur = dwt->n;
+      for (int lev = 1; lev <= dwt->level; ++lev) {
+        if (cur < L - 1) return {};
+        cur = dwt->len[dwt->level - lev + 1];
+      }
+      const int64_t items = ((dwt->n + L - 1) / 2 + kRD - 1) / kRD;
+      if (items > 1024) return {};
+      s.buf = (kHalo + dwt->n + L + 2 * kRD + 4 + 3) & ~3;  // halo | shift | signal | mirror + discarded tail
+      s.smem = elem * ((size_t)s.buf + (size_t)((dwt->total + 4 + 3) & ~3));
+      s.threads = round_threads(items);
+      break;
+    }
+    case FbOp::kWaverec: {
+      int longest = dwt->n;
+      for (int i = 0; i <= dwt->level; ++i) {
+        longest = std::max(longest, dwt->len[i]);
+        if (i > 0 && dwt->len[i] < L / 2) return {};  // no full output pair
+      }
+      s.buf = (longest + L + 4 + 3) & ~3;
+      s.smem = elem * (2 * (size_t)s.buf + (size_t)((dwt->total + 4 + 3) & ~3));
+      s.threads = round_threads((dwt->n / 2 + kRD - 1) / kRD);
+      break;
+    }
+    case FbOp::kMra:  // explicit filters: no blocked kernel
+      return {};
+  }
+  return s.smem <= kSmemLimit ? s : BlkShape{};
 }
 
-template <typename T, int R>
-static int mra_fast_r(const void *w, int64_t batch, int n, const Taps &taps, int J, void *out, cudaStream_t st) {
-  const int threads = chain_threads(n, taps.L, J, R);
-  const size_t smem = mra_blk_smem(n, taps.L, J, R, sizeof(T));
-  if (!smem || smem > kSmemLimit) return WTB_EUNSUPPORTED;
+template <typename T>
+int modwt_fast(const BlkShape &s, const void *x, int64_t batch, int n, const Taps &taps, int J, void *out,
+               cudaStream_t st) {
   WTB_TAPS_SWITCH(taps.L, {
-    WTB_TRY(set_smem(k_mra_blk<T, LT, R>, smem));
-    k_mra_blk<T, LT, R><<<(unsigned)(batch * (J + 1)), threads, smem, st>>>((const T *)w, n, J,
-                                                                           narrow_taps<T, LT>(taps), (T *)out);
+    WTB_TRY(set_smem(k_modwt_blk<T, LT>, s.smem));
+    k_modwt_blk<T, LT><<<(unsigned)batch, s.threads, s.smem, st>>>((const T *)x, n, J, narrow_taps<T, LT>(taps), (T *)out);
   });
   WTB_LAUNCH_CHECK();
   return WTB_OK;
 }
 
 template <typename T>
-int mra_fast(const void *w, int64_t batch, int n, const Taps &taps, int J, void *out, cudaStream_t st) {
-  if (!fast_taps_ok(taps.L) || batch * (J + 1) >= (1LL << 31)) return WTB_EUNSUPPORTED;
-  if (n >= kLongRow) {
-    const int rc = mra_fast_r<T, kRA>(w, batch, n, taps, J, out, st);
-    if (rc != WTB_EUNSUPPORTED) return rc;   // e.g. the longer chains' halo no longer fits
-  }
-  return mra_fast_r<T, kRM>(w, batch, n, taps, J, out, st);
-}
-
-template <typename T>
-int wavedec_fast(const void *x, int64_t batch, const LevelPlan &plan_in, const Taps &taps, void *coeffs,
-                 cudaStream_t st) {
-  if (!fast_taps_ok(taps.L)) return WTB_EUNSUPPORTED;
-  LevelPlan plan = plan_in;
-  // every level's input must hold one whole mirror image of the filter overhang
-  int cur = plan.n;
-  for (int lev = 1; lev <= plan.level; ++lev) {
-    if (cur < taps.L - 1) return WTB_EUNSUPPORTED;
-    cur = plan.len[plan.level - lev + 1];
-  }
-  const int64_t items = ((plan.n + taps.L - 1) / 2 + kRD - 1) / kRD;
-  if (items > 1024) return WTB_EUNSUPPORTED;
-  plan.buf = (kHalo + plan.n + taps.L + 2 * kRD + 4 + 3) & ~3;  // halo | shift | signal | mirror + discarded tail
-  const size_t smem = sizeof(T) * ((size_t)plan.buf + (size_t)((plan.total + 4 + 3) & ~3));
-  if (smem > kSmemLimit) return WTB_EUNSUPPORTED;
-  const int threads = round_threads(items);
+int imodwt_fast(const BlkShape &s, const void *w, int64_t batch, int n, const Taps &taps, int J, void *out,
+                cudaStream_t st) {
   WTB_TAPS_SWITCH(taps.L, {
-    WTB_TRY(set_smem(k_wavedec_blk<T, LT>, smem));
-    k_wavedec_blk<T, LT><<<(unsigned)batch, threads, smem, st>>>((const T *)x, plan, narrow_taps<T, LT>(taps), (T *)coeffs);
+    WTB_TRY(set_smem(k_imodwt_blk<T, LT>, s.smem));
+    k_imodwt_blk<T, LT><<<(unsigned)batch, s.threads, s.smem, st>>>((const T *)w, n, J, narrow_taps<T, LT>(taps), (T *)out);
   });
   WTB_LAUNCH_CHECK();
   return WTB_OK;
 }
 
 template <typename T>
-int waverec_fast(const void *coeffs, int64_t batch, const LevelPlan &plan_in, const Taps &taps, void *x,
-                 cudaStream_t st) {
-  if (!fast_taps_ok(taps.L)) return WTB_EUNSUPPORTED;
-  LevelPlan plan = plan_in;
-  int longest = plan.n;
-  for (int i = 0; i <= plan.level; ++i) {
-    longest = std::max(longest, plan.len[i]);
-    if (i > 0 && plan.len[i] < taps.L / 2) return WTB_EUNSUPPORTED;  // no full output pair
-  }
-  plan.buf = (longest + taps.L + 4 + 3) & ~3;
-  const size_t smem = sizeof(T) * (2 * (size_t)plan.buf + (size_t)((plan.total + 4 + 3) & ~3));
-  if (smem > kSmemLimit) return WTB_EUNSUPPORTED;
-  const int threads = round_threads((plan.n / 2 + kRD - 1) / kRD);
+int mra_fast(const BlkShape &s, const void *w, int64_t batch, int n, const Taps &taps, int J, void *out,
+             cudaStream_t st) {
   WTB_TAPS_SWITCH(taps.L, {
-    WTB_TRY(set_smem(k_waverec_blk<T, LT>, smem));
-    k_waverec_blk<T, LT><<<(unsigned)batch, threads, smem, st>>>((const T *)coeffs, plan, narrow_taps<T, LT>(taps), (T *)x);
+    auto kern = s.R == kRA ? k_mra_blk<T, LT, kRA> : k_mra_blk<T, LT, kRM>;
+    WTB_TRY(set_smem(kern, s.smem));
+    kern<<<(unsigned)(batch * (J + 1)), s.threads, s.smem, st>>>((const T *)w, n, J, narrow_taps<T, LT>(taps), (T *)out);
   });
   WTB_LAUNCH_CHECK();
   return WTB_OK;
 }
 
-#define WTB_INSTANTIATE(T)                                                                               \
-  template int modwt_fast<T>(const void *, int64_t, int, const Taps &, int, void *, cudaStream_t);       \
-  template int imodwt_fast<T>(const void *, int64_t, int, const Taps &, int, void *, cudaStream_t);      \
-  template int mra_fast<T>(const void *, int64_t, int, const Taps &, int, void *, cudaStream_t);         \
-  template int wavedec_fast<T>(const void *, int64_t, const LevelPlan &, const Taps &, void *, cudaStream_t); \
-  template int waverec_fast<T>(const void *, int64_t, const LevelPlan &, const Taps &, void *, cudaStream_t);
+template <typename T>
+int wavedec_fast(const BlkShape &s, const void *x, int64_t batch, const LevelPlan &plan, const Taps &taps,
+                 void *coeffs, cudaStream_t st) {
+  WTB_TAPS_SWITCH(taps.L, {
+    WTB_TRY(set_smem(k_wavedec_blk<T, LT>, s.smem));
+    k_wavedec_blk<T, LT><<<(unsigned)batch, s.threads, s.smem, st>>>((const T *)x, plan, narrow_taps<T, LT>(taps), (T *)coeffs);
+  });
+  WTB_LAUNCH_CHECK();
+  return WTB_OK;
+}
+
+template <typename T>
+int waverec_fast(const BlkShape &s, const void *coeffs, int64_t batch, const LevelPlan &plan, const Taps &taps,
+                 void *x, cudaStream_t st) {
+  WTB_TAPS_SWITCH(taps.L, {
+    WTB_TRY(set_smem(k_waverec_blk<T, LT>, s.smem));
+    k_waverec_blk<T, LT><<<(unsigned)batch, s.threads, s.smem, st>>>((const T *)coeffs, plan, narrow_taps<T, LT>(taps), (T *)x);
+  });
+  WTB_LAUNCH_CHECK();
+  return WTB_OK;
+}
+
+#define WTB_INSTANTIATE(T)                                                                                          \
+  template int modwt_fast<T>(const BlkShape &, const void *, int64_t, int, const Taps &, int, void *, cudaStream_t);   \
+  template int imodwt_fast<T>(const BlkShape &, const void *, int64_t, int, const Taps &, int, void *, cudaStream_t);  \
+  template int mra_fast<T>(const BlkShape &, const void *, int64_t, int, const Taps &, int, void *, cudaStream_t);     \
+  template int wavedec_fast<T>(const BlkShape &, const void *, int64_t, const LevelPlan &, const Taps &, void *, cudaStream_t); \
+  template int waverec_fast<T>(const BlkShape &, const void *, int64_t, const LevelPlan &, const Taps &, void *, cudaStream_t);
 WTB_INSTANTIATE(float)
 WTB_INSTANTIATE(double)
 
