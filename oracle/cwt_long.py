@@ -19,7 +19,9 @@ AVG_BUDGET = 1 << 30
 
 def cwt_rows(signal, dt, dj, s0, J, wavelet, rows, nfft=None):
     """W[rows, :n0] (complex128) of ``po.cwt(signal, dt, dj, s0, J, wavelet)``; nfft defaults to pycwt's
-    padding to the next power of two."""
+    padding to the next power of two.  The normalisation (s |ftfreqs[1]| N)^0.5 is pycwt's at every N > 2; at
+    N = 2 ftfreqs[1] is the Nyquist frequency, negative in numpy's layout, and pycwt's own value is NaN: there the
+    rows follow the kernels' normalisation (2 pi s / dt)^0.5 of every other length, not pycwt."""
     x = np.asarray(signal, dtype=float)
     n0 = x.size
     sj, _, _ = po.cwt_axes(n0, dt, dj, s0, J, wavelet)
@@ -28,7 +30,7 @@ def cwt_rows(signal, dt, dj, s0, J, wavelet, rows, nfft=None):
     ftfreqs = 2 * np.pi * np.fft.fftfreq(N, dt)
     out = np.empty((len(rows), n0), dtype=np.complex128)
     for i, s in enumerate(rows):
-        psi_bar = (sj[s] * ftfreqs[1] * N) ** 0.5 * np.conjugate(wavelet.psi_ft(sj[s] * ftfreqs))
+        psi_bar = (sj[s] * abs(ftfreqs[1]) * N) ** 0.5 * np.conjugate(wavelet.psi_ft(sj[s] * ftfreqs))
         out[i] = np.fft.ifft(xf * psi_bar)[:n0]
     return out
 

@@ -25,6 +25,21 @@ def test_rows_match_the_whole_plane(n0, mother):
     assert np.abs(gotn - Wn[rows]).max() <= 1e-13 * np.abs(Wn).max()
 
 
+@pytest.mark.parametrize("mother", list(MOTHERS))
+def test_two_point_transform(mother):
+    """N = 2: the rows are the two-point DFT written out, with the daughter at 0 and at the Nyquist frequency
+    -pi / dt (numpy's layout) and the normalisation (2 pi s / dt)^0.5 of every other length."""
+    x = np.array([0.7, -1.9])
+    wl = MOTHERS[mother]
+    sj, _, _ = po.cwt_axes(2, 1.0, 1 / 4, -1, 3, wl)
+    got = cl.cwt_rows(x, 1.0, 1 / 4, -1, 3, wl, range(4), nfft=2)
+    X = np.array([x[0] + x[1], x[0] - x[1]])
+    for s in range(4):
+        d = (2 * np.pi * sj[s]) ** 0.5 * np.conjugate(wl.psi_ft(sj[s] * np.array([0.0, -np.pi])))
+        want = 0.5 * np.array([X[0] * d[0] + X[1] * d[1], X[0] * d[0] - X[1] * d[1]])
+        assert np.all(np.isfinite(got[s])) and np.abs(got[s] - want).max() <= 1e-14 * max(np.abs(want).max(), 1e-300)
+
+
 def test_dispatch_boundaries():
     assert cl.route(8192, f64=False) == "generic" and cl.route(16384, f64=False) == "long"
     assert cl.route(4096, f64=True) == "generic" and cl.route(8192, f64=True) == "long"

@@ -257,7 +257,10 @@ static int icwt_impl(const void *coef, int64_t batch, int S, int n0, const doubl
   double *d_scales = (double *)scratch;
   WTB_CUDA(cudaMemcpyAsync(d_scales, scales, sizeof(double) * S, cudaMemcpyHostToDevice, st));
   const size_t in_row = sizeof(cplx<T>) * (size_t)S * n0, out_row = sizeof(T) * (size_t)n0;
-  const int64_t rows = dev ? batch : std::max<int64_t>(1, std::min<int64_t>(batch, (int64_t)((size_t(1) << 30) / in_row)));
+  // series per launch: they run on grid.y (at most 65535); host buffers also stage at most 1 GiB of coefficients
+  const int64_t max_launch = 65535;
+  const int64_t rows = std::min<int64_t>(
+      max_launch, dev ? batch : std::max<int64_t>(1, std::min<int64_t>(batch, (int64_t)((size_t(1) << 30) / in_row))));
   const cplx<T> *d_in = (const cplx<T> *)coef;
   T *d_out = (T *)out;
   if (!dev) {
@@ -268,9 +271,11 @@ static int icwt_impl(const void *coef, int64_t batch, int S, int n0, const doubl
   }
   for (int64_t b0 = 0; b0 < batch; b0 += rows) {
     const int64_t nb = std::min(rows, batch - b0);
-    WTB_REQUIRE(nb < 65536, WTB_EUNSUPPORTED, "wtb_icwt: at most 65535 series per launch");
     if (!dev) WTB_CUDA(cudaMemcpyAsync((void *)d_in, (const char *)coef + b0 * in_row, in_row * nb, cudaMemcpyHostToDevice, st));
-    k_icwt<T><<<dim3((n0 + 255) / 256, (unsigned)nb), 256, 0, st>>>(d_in, S, n0, d_scales, factor, d_out);
+    // device buffers: each launch reads and writes its own block of series in place
+    const cplx<T> *src = dev ? (const cplx<T> *)((const char *)coef + b0 * in_row) : d_in;
+    T *dst = dev ? (T *)((char *)out + b0 * out_row) : d_out;
+    k_icwt<T><<<dim3((n0 + 255) / 256, (unsigned)nb), 256, 0, st>>>(src, S, n0, d_scales, factor, dst);
     WTB_LAUNCH_CHECK();
     if (!dev) {
       WTB_TRY(copy_to_host((char *)out + b0 * out_row, d_out, out_row * nb, st));
