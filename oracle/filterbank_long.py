@@ -219,7 +219,7 @@ def wave_rows(per_series_bytes, rows):
 
 
 def launches(entry, n, f64, batch, L=8, J=1, level=1, device_ptrs=False):
-    """Kernel launches of one long-path call: per host chunk of run_batched (1 GiB of input and output rows,
+    """Kernel launches of one long-path call: per host chunk of stage_rows (1 GiB of input and output rows,
     the whole batch with device pointers), waves of wave_rows series, each with its launches per wave."""
     E = _elem(f64)
     in_row, out_row, inter, per_wave = _rows(entry, n, L, J, level)

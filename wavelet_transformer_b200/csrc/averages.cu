@@ -64,65 +64,35 @@ static int64_t averages_chunk_rows(int64_t batch, int S, int n0, int N, size_t e
   return std::min(batch, std::max(fill, by_bytes) & ~int64_t(1));
 }
 
-static thread_local bool g_in_shard = false;   // set on a pool worker while it runs its block
-
 template <typename T>
 static int averages_entry(const void *x, int64_t batch, int n0, int N, double dt, const Axes &ax, const Mother &mo,
                           int band_lo, int band_hi, double band_factor, int flags, void *global_out, void *band_out,
                           cudaStream_t st) {
   const int S = ax.J + 1;
-  const bool dev = flags & WTB_DEVICE_PTRS;
-  // host buffers, several GPUs (wtb_init_multi): contiguous blocks of series, one per device, as cwt_entry
-  if (!dev && pool_size() > 1 && batch >= 2 * pool_size() && !g_in_shard) {
-    return run_sharded_fn(batch, 2, st, [&](int, int64_t first, int64_t count, cudaStream_t s) {
-      g_in_shard = true;
-      const int rc = averages_entry<T>((const T *)x + first * n0, count, n0, N, dt, ax, mo, band_lo, band_hi,
-                                       band_factor, flags, global_out ? (T *)global_out + first * S : nullptr,
-                                       band_out ? (T *)band_out + first * n0 : nullptr, s);
-      g_in_shard = false;
-      return rc;
-    });
-  }
-  // The power chunk lives in the staging slot: cwt_device takes the arena (and its fast paths the parameter
-  // buffer), and a slot that grows is moved, so a second user of either in this call would lose its data.
-  const int64_t rows = averages_chunk_rows(batch, S, n0, N, sizeof(T));
-  auto al = [](size_t b) { return (b + 255) / 256 * 256; };
-  const size_t b_inv = al(sizeof(double) * S), b_pow = al(sizeof(T) * (size_t)rows * S * n0);
-  const size_t b_x = dev ? 0 : al(sizeof(T) * (size_t)rows * n0);
-  const size_t b_g = dev || !global_out ? 0 : al(sizeof(T) * (size_t)rows * S);
-  const size_t b_b = dev || !band_out ? 0 : al(sizeof(T) * (size_t)rows * n0);
-  void *stage = nullptr;
-  WTB_TRY(staging_reserve(b_inv + b_pow + b_x + b_g + b_b, &stage));
-  double *d_inv = (double *)stage;
-  T *d_pow = (T *)((char *)d_inv + b_inv);
-  T *d_x = (T *)((char *)d_pow + b_pow);
-  T *d_g = (T *)((char *)d_x + b_x);
-  T *d_b = (T *)((char *)d_g + b_g);
+  const InRows xs{x, sizeof(T) * n0};
+  const OutRows gl{global_out, sizeof(T) * S}, bd{band_out, sizeof(T) * n0};
   std::vector<double> inv(S);
   for (int s = 0; s < S; ++s) inv[s] = 1.0 / ax.scales[s];
-  // inv.data() is pageable: the copy is staged before the call returns
-  WTB_CUDA(cudaMemcpyAsync(d_inv, inv.data(), sizeof(double) * S, cudaMemcpyHostToDevice, st));
-  for (int64_t b0 = 0; b0 < batch; b0 += rows) {
-    const int64_t nb = std::min(rows, batch - b0);
-    const T *xin = (const T *)x + b0 * n0;
-    T *g = global_out ? (T *)global_out + b0 * S : nullptr;
-    T *bo = band_out ? (T *)band_out + b0 * n0 : nullptr;
-    if (!dev) {
-      WTB_CUDA(cudaMemcpyAsync(d_x, xin, sizeof(T) * nb * n0, cudaMemcpyHostToDevice, st));
-      xin = d_x;
-      g = global_out ? d_g : nullptr;
-      bo = band_out ? d_b : nullptr;
-    }
-    WTB_TRY(cwt_device<T>(xin, nb, n0, N, dt, ax, mo, flags, d_pow, nullptr, st));
-    k_cwt_averages<T><<<dim3((unsigned)nb, averages_parts(nb, S, n0)), kAvgThreads, 0, st>>>(d_pow, S, n0, d_inv, band_lo, band_hi, band_factor, g, bo);
-    WTB_LAUNCH_CHECK();
-    if (!dev) {
-      if (global_out) WTB_TRY(copy_to_host((T *)global_out + b0 * S, d_g, sizeof(T) * nb * S, st));
-      if (band_out) WTB_TRY(copy_to_host((T *)band_out + b0 * n0, d_b, sizeof(T) * nb * n0, st));
-      WTB_CUDA(cudaStreamSynchronize(st));
-    }
-  }
-  return WTB_OK;
+  return shard_host_rows(batch, flags, st, [&](int64_t first, int64_t count, cudaStream_t s) {
+    // 1/s_j and the power chunk live in the staging slot, next to the host-path I/O: cwt_device takes the arena
+    // (and its fast paths the parameter buffer)
+    const int64_t rows = averages_chunk_rows(count, S, n0, N, sizeof(T));
+    const size_t b_inv = align256(sizeof(double) * S);
+    return stage_rows(count, rows, flags, s, {xs.at(first)}, {gl.at(first), bd.at(first)},
+                      b_inv + sizeof(T) * (size_t)rows * S * n0,
+                      [&](const void *const *in, void *const *out, void *extra, int64_t b0, int64_t nb) {
+                        double *d_inv = (double *)extra;
+                        T *d_pow = (T *)((char *)extra + b_inv);
+                        // inv.data() is pageable: the copy is staged before it returns
+                        if (b0 == 0)
+                          WTB_CUDA(cudaMemcpyAsync(d_inv, inv.data(), sizeof(double) * S, cudaMemcpyHostToDevice, s));
+                        WTB_TRY(cwt_device<T>((const T *)in[0], nb, n0, N, dt, ax, mo, flags, d_pow, nullptr, s));
+                        k_cwt_averages<T><<<dim3((unsigned)nb, averages_parts(nb, S, n0)), kAvgThreads, 0, s>>>(
+                            d_pow, S, n0, d_inv, band_lo, band_hi, band_factor, (T *)out[0], (T *)out[1]);
+                        WTB_LAUNCH_CHECK();
+                        return WTB_OK;
+                      });
+  });
 }
 
 }  // namespace wtb

@@ -4,10 +4,12 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <algorithm>
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <initializer_list>
 #include <map>
 #include <mutex>
 #include <string>
@@ -171,6 +173,82 @@ template <typename F> int run_sharded_fn(int64_t total, int64_t min_total, cudaS
                      (void *)&f);
 }
 const char *last_error();     // this thread's message (workers hand theirs to the caller)
+
+// ---- batches of rows: the split over the pool and the host staging of every batched entry point -------------------
+inline size_t align256(size_t bytes) { return (bytes + 255) / 256 * 256; }
+
+// Host-buffer batches with a pool of two or more devices (wtb_init_multi) and at least two rows per device:
+// call(first, count, stream) once per device for a contiguous block of rows, on that device's worker thread.
+// Otherwise call(0, batch, stream) once.  The caller offsets its pointers by `first`; the worker runs `call` itself
+// and never comes back here, so a block is never split again.
+template <typename F> int shard_host_rows(int64_t batch, int flags, cudaStream_t st, F &&call) {
+  if ((flags & WTB_DEVICE_PTRS) || pool_size() < 2 || batch < 2 * pool_size()) return call(int64_t(0), batch, st);
+  return run_sharded_fn(batch, 2, st, [&](int, int64_t first, int64_t count, cudaStream_t s) {
+    return call(first, count, s);
+  });
+}
+
+// Rows per host chunk: as many as keep `row_bytes` each within 1 GiB of staging, at least one, at most the batch;
+// with device pointers the whole batch
+inline int64_t host_rows(int64_t batch, size_t row_bytes, int flags) {
+  if (flags & WTB_DEVICE_PTRS) return batch;
+  return std::max<int64_t>(1, std::min<int64_t>(batch, (int64_t)((size_t(1) << 30) / row_bytes)));
+}
+
+// One buffer of the caller's batch: rows of row_bytes bytes each.  ptr is null for an output not asked for.
+template <typename P> struct RowBuf {
+  P *ptr;
+  size_t row_bytes;
+  RowBuf at(int64_t row) const { return {ptr ? (P *)((const char *)ptr + row * row_bytes) : nullptr, row_bytes}; }
+};
+using InRows = RowBuf<const void>;
+using OutRows = RowBuf<void>;
+
+// Runs launch(in, out, extra, b0, nb) over [0, batch) in chunks of `rows` (the caller's chunk rule).  in[i] / out[i]
+// are the device rows b0 .. b0 + nb of ins[i] / outs[i], null where the caller's pointer is; extra is extra_bytes of
+// staging scratch (null when 0).
+//   Host buffers: the inputs go up with cudaMemcpyAsync before the launch, the outputs come back through copy_to_host,
+//   then the stream is synchronised, chunk by chunk.
+//   WTB_DEVICE_PTRS: the caller's pointers, offset by b0; nothing is copied or synchronised.
+// The staging slot is reserved once for the whole call (every non-null port at `rows` rows and extra_bytes, each
+// region 256-byte aligned): a second reservation that grew the slot would move it under the first one's data, so
+// nothing inside `launch` may take staging.
+template <typename F>
+int stage_rows(int64_t batch, int64_t rows, int flags, cudaStream_t st, std::initializer_list<InRows> ins,
+               std::initializer_list<OutRows> outs, size_t extra_bytes, F &&launch) {
+  const bool dev = flags & WTB_DEVICE_PTRS;
+  const size_t n_in = ins.size(), n_out = outs.size();
+  const InRows *in = ins.begin();
+  const OutRows *out = outs.begin();
+  size_t bytes = align256(extra_bytes);
+  for (size_t i = 0; i < n_in && !dev; ++i) bytes += in[i].ptr ? align256(in[i].row_bytes * rows) : 0;
+  for (size_t i = 0; i < n_out && !dev; ++i) bytes += out[i].ptr ? align256(out[i].row_bytes * rows) : 0;
+  char *stage = nullptr;
+  if (bytes) WTB_TRY(staging_reserve(bytes, (void **)&stage));
+  void *extra = extra_bytes ? stage : nullptr;
+  std::vector<const void *> d_in(n_in, nullptr);
+  std::vector<void *> d_out(n_out, nullptr);
+  char *p = stage + align256(extra_bytes);
+  for (size_t i = 0; i < n_in && !dev; ++i)
+    if (in[i].ptr) { d_in[i] = p; p += align256(in[i].row_bytes * rows); }
+  for (size_t i = 0; i < n_out && !dev; ++i)
+    if (out[i].ptr) { d_out[i] = p; p += align256(out[i].row_bytes * rows); }
+  for (int64_t b0 = 0; b0 < batch; b0 += rows) {
+    const int64_t nb = std::min(rows, batch - b0);
+    for (size_t i = 0; i < n_in; ++i) {
+      if (dev) d_in[i] = in[i].at(b0).ptr;
+      else if (in[i].ptr)
+        WTB_CUDA(cudaMemcpyAsync((void *)d_in[i], in[i].at(b0).ptr, in[i].row_bytes * nb, cudaMemcpyHostToDevice, st));
+    }
+    for (size_t i = 0; i < n_out && dev; ++i) d_out[i] = out[i].at(b0).ptr;
+    WTB_TRY(launch(d_in.data(), d_out.data(), extra, b0, nb));
+    if (dev) continue;   // every chunk is ordered on st
+    for (size_t i = 0; i < n_out; ++i)
+      if (out[i].ptr) WTB_TRY(copy_to_host(out[i].at(b0).ptr, d_out[i], out[i].row_bytes * nb, st));
+    WTB_CUDA(cudaStreamSynchronize(st));
+  }
+  return WTB_OK;
+}
 
 inline int ilog2(int n) { int l = 0; while ((1 << l) < n) ++l; return l; }
 inline bool is_pow2(int n) { return n > 0 && (n & (n - 1)) == 0; }

@@ -113,7 +113,7 @@ int cwt_device(const T *d_x, int64_t batch, int n0, int N, double dt, const Axes
               "length up to %d for %s", N, smem, sizeof(T) == 4 ? 8192 : 4096, sizeof(T) == 4 ? 4096 : 2048,
               sizeof(T) == 4 ? "float" : "double");
   void *scratch = nullptr;
-  const size_t sc_bytes = ((sizeof(double) * S + 255) / 256) * 256;
+  const size_t sc_bytes = align256(sizeof(double) * S);
   WTB_TRY(arena_reserve(sc_bytes + sizeof(cplx<T>) * (size_t)batch * N, &scratch));
   double *d_scales = (double *)scratch;
   cplx<T> *d_xhat = (cplx<T> *)((char *)scratch + sc_bytes);
@@ -152,50 +152,21 @@ template int cwt_device<float>(const float *, int64_t, int, int, double, const A
 template int cwt_device<double>(const double *, int64_t, int, int, double, const Axes &, const Mother &, int, double *,
                                 double2 *, cudaStream_t);
 
-static thread_local bool g_in_shard = false;   // set on a pool worker while it runs its block
-
 template <typename T>
 static int cwt_entry(const void *x, int64_t batch, int n0, int N, double dt, const Axes &ax,
-                     const Mother &f0, int flags, void *power_out, void *coef_out, cudaStream_t st) {
-  const int S = ax.J + 1;
-  if (flags & WTB_DEVICE_PTRS)
-    return cwt_device<T>((const T *)x, batch, n0, N, dt, ax, f0, flags, (T *)power_out,
-                         (cplx<T> *)coef_out, st);
-  // host buffers, several GPUs (wtb_init_multi): contiguous blocks of series, one per device
-  if (pool_size() > 1 && batch >= 2 * pool_size() && !g_in_shard) {
-    return run_sharded_fn(batch, 2, st, [&](int, int64_t first, int64_t count, cudaStream_t s) {
-      g_in_shard = true;
-      const int rc = cwt_entry<T>((const T *)x + first * n0, count, n0, N, dt, ax, f0, flags,
-                                  power_out ? (T *)power_out + first * S * n0 : nullptr,
-                                  coef_out ? (cplx<T> *)coef_out + first * S * n0 : nullptr, s);
-      g_in_shard = false;
-      return rc;
-    });
-  }
-  // host buffers: stream the batch through a bounded staging arena
-  const size_t per_row = sizeof(T) * ((size_t)n0 + (power_out ? (size_t)S * n0 : 0) +
-                                      (coef_out ? 2 * (size_t)S * n0 : 0));
-  const size_t budget = size_t(1) << 30;
-  int64_t rows = std::max<int64_t>(1, std::min<int64_t>(batch, (int64_t)(budget / per_row)));
-  void *stage = nullptr;
-  WTB_TRY(staging_reserve(per_row * rows + 1024, &stage));
-  T *d_x = (T *)stage;
-  size_t off = (sizeof(T) * (size_t)rows * n0 + 255) / 256 * 256;
-  T *d_power = nullptr;
-  cplx<T> *d_coef = nullptr;
-  if (power_out) { d_power = (T *)((char *)stage + off); off += (sizeof(T) * (size_t)rows * S * n0 + 255) / 256 * 256; }
-  if (coef_out) d_coef = (cplx<T> *)((char *)stage + off);
-  for (int64_t b0 = 0; b0 < batch; b0 += rows) {
-    const int64_t nb = std::min(rows, batch - b0);
-    WTB_CUDA(cudaMemcpyAsync(d_x, (const T *)x + b0 * n0, sizeof(T) * nb * n0, cudaMemcpyHostToDevice, st));
-    WTB_TRY(cwt_device<T>(d_x, nb, n0, N, dt, ax, f0, flags, d_power, d_coef, st));
-    if (power_out)
-      WTB_TRY(copy_to_host((T *)power_out + b0 * S * n0, d_power, sizeof(T) * nb * S * n0, st));
-    if (coef_out)
-      WTB_TRY(copy_to_host((cplx<T> *)coef_out + b0 * S * n0, d_coef, sizeof(cplx<T>) * nb * S * n0, st));
-    WTB_CUDA(cudaStreamSynchronize(st));
-  }
-  return WTB_OK;
+                     const Mother &mo, int flags, void *power_out, void *coef_out, cudaStream_t st) {
+  const size_t plane = (size_t)(ax.J + 1) * n0;
+  const InRows xs{x, sizeof(T) * n0};
+  const OutRows pw{power_out, sizeof(T) * plane}, cf{coef_out, sizeof(cplx<T>) * plane};
+  // host buffers: chunks of at most 1 GiB of staged input and output rows
+  const size_t per_row = xs.row_bytes + (power_out ? pw.row_bytes : 0) + (coef_out ? cf.row_bytes : 0);
+  return shard_host_rows(batch, flags, st, [&](int64_t first, int64_t count, cudaStream_t s) {
+    return stage_rows(count, host_rows(count, per_row, flags), flags, s, {xs.at(first)}, {pw.at(first), cf.at(first)},
+                      0, [&](const void *const *in, void *const *out, void *, int64_t, int64_t nb) {
+                        return cwt_device<T>((const T *)in[0], nb, n0, N, dt, ax, mo, flags, (T *)out[0],
+                                             (cplx<T> *)out[1], s);
+                      });
+  });
 }
 
 }  // namespace wtb
@@ -250,39 +221,20 @@ __global__ void k_icwt(const cplx<T> *__restrict__ coef, int S, int n0, const do
 template <typename T>
 static int icwt_impl(const void *coef, int64_t batch, int S, int n0, const double *scales, double factor, int flags,
                      void *out, cudaStream_t st) {
-  const bool dev = flags & WTB_DEVICE_PTRS;
-  auto al = [](size_t b) { return (b + 255) / 256 * 256; };
   void *scratch = nullptr;
-  WTB_TRY(arena_reserve(al(sizeof(double) * S), &scratch));
+  WTB_TRY(arena_reserve(align256(sizeof(double) * S), &scratch));
   double *d_scales = (double *)scratch;
   WTB_CUDA(cudaMemcpyAsync(d_scales, scales, sizeof(double) * S, cudaMemcpyHostToDevice, st));
-  const size_t in_row = sizeof(cplx<T>) * (size_t)S * n0, out_row = sizeof(T) * (size_t)n0;
+  const size_t in_row = sizeof(cplx<T>) * (size_t)S * n0;
   // series per launch: they run on grid.y (at most 65535); host buffers also stage at most 1 GiB of coefficients
-  const int64_t max_launch = 65535;
-  const int64_t rows = std::min<int64_t>(
-      max_launch, dev ? batch : std::max<int64_t>(1, std::min<int64_t>(batch, (int64_t)((size_t(1) << 30) / in_row))));
-  const cplx<T> *d_in = (const cplx<T> *)coef;
-  T *d_out = (T *)out;
-  if (!dev) {
-    void *stage = nullptr;
-    WTB_TRY(staging_reserve(al(in_row * rows) + al(out_row * rows), &stage));
-    d_in = (const cplx<T> *)stage;
-    d_out = (T *)((char *)stage + al(in_row * rows));
-  }
-  for (int64_t b0 = 0; b0 < batch; b0 += rows) {
-    const int64_t nb = std::min(rows, batch - b0);
-    if (!dev) WTB_CUDA(cudaMemcpyAsync((void *)d_in, (const char *)coef + b0 * in_row, in_row * nb, cudaMemcpyHostToDevice, st));
-    // device buffers: each launch reads and writes its own block of series in place
-    const cplx<T> *src = dev ? (const cplx<T> *)((const char *)coef + b0 * in_row) : d_in;
-    T *dst = dev ? (T *)((char *)out + b0 * out_row) : d_out;
-    k_icwt<T><<<dim3((n0 + 255) / 256, (unsigned)nb), 256, 0, st>>>(src, S, n0, d_scales, factor, dst);
-    WTB_LAUNCH_CHECK();
-    if (!dev) {
-      WTB_TRY(copy_to_host((char *)out + b0 * out_row, d_out, out_row * nb, st));
-      WTB_CUDA(cudaStreamSynchronize(st));
-    }
-  }
-  return WTB_OK;
+  const int64_t rows = std::min<int64_t>(65535, host_rows(batch, in_row, flags));
+  return stage_rows(batch, rows, flags, st, {{coef, in_row}}, {{out, sizeof(T) * n0}}, 0,
+                    [&](const void *const *in, void *const *o, void *, int64_t, int64_t nb) {
+                      k_icwt<T><<<dim3((n0 + 255) / 256, (unsigned)nb), 256, 0, st>>>((const cplx<T> *)in[0], S, n0,
+                                                                                      d_scales, factor, (T *)o[0]);
+                      WTB_LAUNCH_CHECK();
+                      return WTB_OK;
+                    });
 }
 }  // namespace wtb
 

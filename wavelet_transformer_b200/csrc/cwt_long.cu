@@ -95,8 +95,7 @@ int cwt_long(const T *d_x, int64_t batch, int n0, int N, double dt, const Axes &
   const int64_t rows = batch * S;
   const int64_t wave_fwd = long_wave_rows(N, sizeof(cplx<T>), batch), wave = long_wave_rows(N, sizeof(cplx<T>), rows);
   // one reservation: a slot that grows is moved
-  auto al = [](size_t b) { return (b + 255) / 256 * 256; };
-  const size_t b_sc = al(sizeof(double) * S), b_xhat = al(sizeof(cplx<T>) * (size_t)batch * N);
+  const size_t b_sc = align256(sizeof(double) * S), b_xhat = align256(sizeof(cplx<T>) * (size_t)batch * N);
   void *scratch = nullptr;
   WTB_TRY(arena_reserve(b_sc + b_xhat + sizeof(cplx<T>) * (size_t)wave * N, &scratch));
   double *d_scales = (double *)scratch;

@@ -274,13 +274,14 @@ static int modwt_impl(const void *x, int64_t batch, int n, const Taps &taps, int
   WTB_TRY(fb_plan<T>(FbOp::kModwt, kern, n, taps.L, J, nullptr, flags, &p));
   if (p.path == FbPath::kLong) return modwt_long<T>(x, batch, n, taps, J, flags, out, st);
   if (p.path == FbPath::kGeneric) WTB_TRY(set_smem(kern, p.cta.smem));
-  return run_batched(x, out, batch, sizeof(T) * n, sizeof(T) * (size_t)(J + 1) * n, flags, st,
-                     [&](const void *di, void *dout, int64_t nb) -> int {
-                       if (p.path == FbPath::kBlocked) return modwt_fast<T>(p.cta, di, nb, n, taps, J, dout, st);
-                       kern<<<(unsigned)nb, p.cta.threads, p.cta.smem, st>>>((const T *)di, n, J, taps, (T *)dout);
-                       WTB_LAUNCH_CHECK();
-                       return WTB_OK;
-                     });
+  const size_t in_row = sizeof(T) * n, out_row = sizeof(T) * (size_t)(J + 1) * n;
+  return stage_rows(batch, host_rows(batch, in_row + out_row, flags), flags, st, {{x, in_row}}, {{out, out_row}}, 0,
+                    [&](const void *const *di, void *const *dout, void *, int64_t, int64_t nb) -> int {
+                      if (p.path == FbPath::kBlocked) return modwt_fast<T>(p.cta, di[0], nb, n, taps, J, dout[0], st);
+                      kern<<<(unsigned)nb, p.cta.threads, p.cta.smem, st>>>((const T *)di[0], n, J, taps, (T *)dout[0]);
+                      WTB_LAUNCH_CHECK();
+                      return WTB_OK;
+                    });
 }
 
 template <typename T>
@@ -291,13 +292,14 @@ static int imodwt_impl(const void *w, int64_t batch, int n, const Taps &taps, in
   WTB_TRY(fb_plan<T>(FbOp::kImodwt, kern, n, taps.L, J, nullptr, flags, &p));
   if (p.path == FbPath::kLong) return imodwt_long<T>(w, batch, n, taps, J, flags, out, st);
   if (p.path == FbPath::kGeneric) WTB_TRY(set_smem(kern, p.cta.smem));
-  return run_batched(w, out, batch, sizeof(T) * (size_t)(J + 1) * n, sizeof(T) * n, flags, st,
-                     [&](const void *di, void *dout, int64_t nb) -> int {
-                       if (p.path == FbPath::kBlocked) return imodwt_fast<T>(p.cta, di, nb, n, taps, J, dout, st);
-                       kern<<<(unsigned)nb, p.cta.threads, p.cta.smem, st>>>((const T *)di, n, J, taps, (T *)dout);
-                       WTB_LAUNCH_CHECK();
-                       return WTB_OK;
-                     });
+  const size_t in_row = sizeof(T) * (size_t)(J + 1) * n, out_row = sizeof(T) * n;
+  return stage_rows(batch, host_rows(batch, in_row + out_row, flags), flags, st, {{w, in_row}}, {{out, out_row}}, 0,
+                    [&](const void *const *di, void *const *dout, void *, int64_t, int64_t nb) -> int {
+                      if (p.path == FbPath::kBlocked) return imodwt_fast<T>(p.cta, di[0], nb, n, taps, J, dout[0], st);
+                      kern<<<(unsigned)nb, p.cta.threads, p.cta.smem, st>>>((const T *)di[0], n, J, taps, (T *)dout[0]);
+                      WTB_LAUNCH_CHECK();
+                      return WTB_OK;
+                    });
 }
 
 // k_modwtmra over the batch with the periodised filters filt [J+1, n] (host), on a kGeneric plan
@@ -313,7 +315,7 @@ static int mra_generic(const FbPlan &p, const void *w, int64_t batch, int n, con
     flen[j] = len;
   }
   void *scratch = nullptr;
-  const size_t b_f = (sizeof(double) * (size_t)(J + 1) * n + 255) / 256 * 256;
+  const size_t b_f = align256(sizeof(double) * (size_t)(J + 1) * n);
   WTB_TRY(arena_reserve(b_f + sizeof(int) * (J + 1), &scratch));
   double *d_filt = (double *)scratch;
   int *d_flen = (int *)((char *)scratch + b_f);
@@ -321,9 +323,11 @@ static int mra_generic(const FbPlan &p, const void *w, int64_t batch, int n, con
   WTB_CUDA(cudaMemcpyAsync(d_flen, flen.data(), sizeof(int) * (J + 1), cudaMemcpyHostToDevice, st));
   WTB_CUDA(cudaStreamSynchronize(st));  // flen is a local
   const size_t row = sizeof(T) * (size_t)(J + 1) * n;
-  return run_batched(w, out, batch, row, row, flags, st, [&](const void *di, void *dout, int64_t nb) -> int {
+  return stage_rows(batch, host_rows(batch, 2 * row, flags), flags, st, {{w, row}}, {{out, row}}, 0,
+                    [&](const void *const *di, void *const *dout, void *, int64_t, int64_t nb) -> int {
     WTB_REQUIRE(nb * (J + 1) < (1LL << 31), WTB_EUNSUPPORTED, "batch too large");
-    k_modwtmra<T><<<(unsigned)(nb * (J + 1)), p.cta.threads, p.cta.smem, st>>>((const T *)di, n, J, d_filt, d_flen, (T *)dout);
+    k_modwtmra<T><<<(unsigned)(nb * (J + 1)), p.cta.threads, p.cta.smem, st>>>((const T *)di[0], n, J, d_filt, d_flen,
+                                                                               (T *)dout[0]);
     WTB_LAUNCH_CHECK();
     return WTB_OK;
   });
@@ -381,9 +385,10 @@ static int mra_taps_impl(const void *w, int64_t batch, int n, const Taps &taps, 
     return mra_generic<T>(p, w, batch, n, filt.data(), J, flags, out, st);
   }
   const size_t row = sizeof(T) * (size_t)(J + 1) * n;
-  return run_batched(w, out, batch, row, row, flags, st, [&](const void *di, void *dout, int64_t nb) -> int {
+  return stage_rows(batch, host_rows(batch, 2 * row, flags), flags, st, {{w, row}}, {{out, row}}, 0,
+                    [&](const void *const *di, void *const *dout, void *, int64_t, int64_t nb) -> int {
     WTB_REQUIRE(nb * (J + 1) < (1LL << 31), WTB_EUNSUPPORTED, "batch too large");
-    return mra_fast<T>(p.cta, di, nb, n, taps, J, dout, st);
+    return mra_fast<T>(p.cta, di[0], nb, n, taps, J, dout[0], st);
   });
 }
 
@@ -415,13 +420,15 @@ static int wavedec_impl(const void *x, int64_t batch, int n, const Taps &taps, i
   WTB_TRY(fb_plan<T>(FbOp::kWavedec, k_wavedec<T>, n, taps.L, level, &plan, flags, &p));
   if (p.path == FbPath::kLong) return wavedec_long<T>(x, batch, plan, taps, flags, coeffs, st);
   if (p.path == FbPath::kGeneric) WTB_TRY(set_smem(k_wavedec<T>, p.cta.smem));
-  return run_batched(x, coeffs, batch, sizeof(T) * n, sizeof(T) * (size_t)plan.total, flags, st,
-                     [&](const void *di, void *dout, int64_t nb) -> int {
-                       if (p.path == FbPath::kBlocked) return wavedec_fast<T>(p.cta, di, nb, plan, taps, dout, st);
-                       k_wavedec<T><<<(unsigned)nb, p.cta.threads, p.cta.smem, st>>>((const T *)di, plan, taps, (T *)dout);
-                       WTB_LAUNCH_CHECK();
-                       return WTB_OK;
-                     });
+  const size_t in_row = sizeof(T) * n, out_row = sizeof(T) * (size_t)plan.total;
+  return stage_rows(batch, host_rows(batch, in_row + out_row, flags), flags, st, {{x, in_row}}, {{coeffs, out_row}}, 0,
+                    [&](const void *const *di, void *const *dout, void *, int64_t, int64_t nb) -> int {
+                      if (p.path == FbPath::kBlocked) return wavedec_fast<T>(p.cta, di[0], nb, plan, taps, dout[0], st);
+                      k_wavedec<T><<<(unsigned)nb, p.cta.threads, p.cta.smem, st>>>((const T *)di[0], plan, taps,
+                                                                                   (T *)dout[0]);
+                      WTB_LAUNCH_CHECK();
+                      return WTB_OK;
+                    });
 }
 
 template <typename T>
@@ -435,13 +442,15 @@ static int waverec_impl(const void *coeffs, int64_t batch, const int *lens, int 
   WTB_TRY(fb_plan<T>(FbOp::kWaverec, k_waverec<T>, nout, taps.L, level, &plan, flags, &p));
   if (p.path == FbPath::kLong) return waverec_long<T>(coeffs, batch, plan, taps, flags, x, st);
   if (p.path == FbPath::kGeneric) WTB_TRY(set_smem(k_waverec<T>, p.cta.smem));
-  return run_batched(coeffs, x, batch, sizeof(T) * (size_t)plan.total, sizeof(T) * (size_t)nout, flags, st,
-                     [&](const void *di, void *dout, int64_t nb) -> int {
-                       if (p.path == FbPath::kBlocked) return waverec_fast<T>(p.cta, di, nb, plan, taps, dout, st);
-                       k_waverec<T><<<(unsigned)nb, p.cta.threads, p.cta.smem, st>>>((const T *)di, plan, taps, (T *)dout);
-                       WTB_LAUNCH_CHECK();
-                       return WTB_OK;
-                     });
+  const size_t in_row = sizeof(T) * (size_t)plan.total, out_row = sizeof(T) * (size_t)nout;
+  return stage_rows(batch, host_rows(batch, in_row + out_row, flags), flags, st, {{coeffs, in_row}}, {{x, out_row}}, 0,
+                    [&](const void *const *di, void *const *dout, void *, int64_t, int64_t nb) -> int {
+                      if (p.path == FbPath::kBlocked) return waverec_fast<T>(p.cta, di[0], nb, plan, taps, dout[0], st);
+                      k_waverec<T><<<(unsigned)nb, p.cta.threads, p.cta.smem, st>>>((const T *)di[0], plan, taps,
+                                                                                   (T *)dout[0]);
+                      WTB_LAUNCH_CHECK();
+                      return WTB_OK;
+                    });
 }
 
 }  // namespace wtb
@@ -449,18 +458,6 @@ static int waverec_impl(const void *coeffs, int64_t batch, const int *lens, int 
 using namespace wtb;
 
 #define DISPATCH(fn, ...) ((flags & WTB_F64) ? fn<double>(__VA_ARGS__) : fn<float>(__VA_ARGS__))
-
-// Host-buffer batches with several GPUs (wtb_init_multi): contiguous blocks of rows, one per device.
-// `call(in, out, count, stream)` runs the transform on `count` rows starting at the given pointers.
-template <typename F>
-static int shard_rows(const void *in, void *out, int64_t batch, size_t in_row, size_t out_row, int flags, void *stream,
-                      F call) {
-  if ((flags & WTB_DEVICE_PTRS) || pool_size() < 2 || batch < 2 * pool_size())
-    return call(in, out, batch, (cudaStream_t)stream);
-  return run_sharded_fn(batch, 2, (cudaStream_t)stream, [&](int, int64_t first, int64_t count, cudaStream_t s) {
-    return call((const char *)in + first * in_row, (char *)out + first * out_row, count, s);
-  });
-}
 
 extern "C" int wtb_modwt(const void *x, int64_t batch, int n, const double *g, const double *h, int L,
                          int J, int flags, void *w_out, void *stream) {
@@ -470,8 +467,10 @@ extern "C" int wtb_modwt(const void *x, int64_t batch, int n, const double *g, c
   WTB_ENTER(flags, x, stream);
   if (batch == 0) return WTB_OK;
   const size_t e = ((flags & WTB_F64) ? 8 : 4);
-  return shard_rows(x, w_out, batch, e * n, e * (size_t)(J + 1) * n, flags, stream,
-                    [&](const void *i, void *o, int64_t nb, cudaStream_t st) { return DISPATCH(modwt_impl, i, nb, n, taps, J, flags, o, st); });
+  return shard_host_rows(batch, flags, (cudaStream_t)stream, [&](int64_t first, int64_t nb, cudaStream_t st) {
+    return DISPATCH(modwt_impl, (const char *)x + first * e * n, nb, n, taps, J, flags,
+                    (char *)w_out + first * e * (J + 1) * n, st);
+  });
 }
 
 extern "C" int wtb_imodwt(const void *w, int64_t batch, int n, const double *g, const double *h, int L,
@@ -482,8 +481,10 @@ extern "C" int wtb_imodwt(const void *w, int64_t batch, int n, const double *g, 
   WTB_ENTER(flags, w, stream);
   if (batch == 0) return WTB_OK;
   const size_t e = ((flags & WTB_F64) ? 8 : 4);
-  return shard_rows(w, x_out, batch, e * (size_t)(J + 1) * n, e * n, flags, stream,
-                    [&](const void *i, void *o, int64_t nb, cudaStream_t st) { return DISPATCH(imodwt_impl, i, nb, n, taps, J, flags, o, st); });
+  return shard_host_rows(batch, flags, (cudaStream_t)stream, [&](int64_t first, int64_t nb, cudaStream_t st) {
+    return DISPATCH(imodwt_impl, (const char *)w + first * e * (J + 1) * n, nb, n, taps, J, flags,
+                    (char *)x_out + first * e * n, st);
+  });
 }
 
 extern "C" int wtb_modwtmra(const void *w, int64_t batch, int n, const double *filt, int J, int flags,
@@ -492,8 +493,10 @@ extern "C" int wtb_modwtmra(const void *w, int64_t batch, int n, const double *f
   WTB_ENTER(flags, w, stream);
   if (batch == 0) return WTB_OK;
   const size_t e = ((flags & WTB_F64) ? 8 : 4);
-  return shard_rows(w, out, batch, e * (size_t)(J + 1) * n, e * (size_t)(J + 1) * n, flags, stream,
-                    [&](const void *i, void *o, int64_t nb, cudaStream_t st) { return DISPATCH(mra_impl, i, nb, n, filt, J, flags, o, st); });
+  return shard_host_rows(batch, flags, (cudaStream_t)stream, [&](int64_t first, int64_t nb, cudaStream_t st) {
+    const size_t at = first * e * (J + 1) * n;
+    return DISPATCH(mra_impl, (const char *)w + at, nb, n, filt, J, flags, (char *)out + at, st);
+  });
 }
 
 extern "C" int wtb_modwtmra_taps(const void *w, int64_t batch, int n, const double *g, const double *h, int L,
@@ -504,8 +507,10 @@ extern "C" int wtb_modwtmra_taps(const void *w, int64_t batch, int n, const doub
   WTB_ENTER(flags, w, stream);
   if (batch == 0) return WTB_OK;
   const size_t e = ((flags & WTB_F64) ? 8 : 4);
-  return shard_rows(w, out, batch, e * (size_t)(J + 1) * n, e * (size_t)(J + 1) * n, flags, stream,
-                    [&](const void *i, void *o, int64_t nb, cudaStream_t st) { return DISPATCH(mra_taps_impl, i, nb, n, taps, g, h, J, flags, o, st); });
+  return shard_host_rows(batch, flags, (cudaStream_t)stream, [&](int64_t first, int64_t nb, cudaStream_t st) {
+    const size_t at = first * e * (J + 1) * n;
+    return DISPATCH(mra_taps_impl, (const char *)w + at, nb, n, taps, g, h, J, flags, (char *)out + at, st);
+  });
 }
 
 extern "C" int wtb_wavedec(const void *x, int64_t batch, int n, const double *dec_lo, const double *dec_hi,
@@ -520,8 +525,10 @@ extern "C" int wtb_wavedec(const void *x, int64_t batch, int n, const double *de
   WTB_TRY(wtb_dwt_coeff_lens(n, L, level, lens.data()));
   size_t total = 0;
   for (int v : lens) total += (size_t)v;
-  return shard_rows(x, coeffs, batch, e * n, e * total, flags, stream,
-                    [&](const void *i, void *o, int64_t nb, cudaStream_t st) { return DISPATCH(wavedec_impl, i, nb, n, taps, level, flags, o, st); });
+  return shard_host_rows(batch, flags, (cudaStream_t)stream, [&](int64_t first, int64_t nb, cudaStream_t st) {
+    return DISPATCH(wavedec_impl, (const char *)x + first * e * n, nb, n, taps, level, flags,
+                    (char *)coeffs + first * e * total, st);
+  });
 }
 
 extern "C" int wtb_waverec(const void *coeffs, int64_t batch, const int *lens, int level, const double *rec_lo,
@@ -536,6 +543,8 @@ extern "C" int wtb_waverec(const void *coeffs, int64_t batch, const int *lens, i
   for (int l = 0; l <= level; ++l) total += (size_t)lens[l];
   const int nout = wtb_waverec_len(lens, level, L);
   if (nout < 0) return nout;
-  return shard_rows(coeffs, x_out, batch, e * total, e * (size_t)nout, flags, stream,
-                    [&](const void *i, void *o, int64_t nb, cudaStream_t st) { return DISPATCH(waverec_impl, i, nb, lens, level, taps, flags, o, st); });
+  return shard_host_rows(batch, flags, (cudaStream_t)stream, [&](int64_t first, int64_t nb, cudaStream_t st) {
+    return DISPATCH(waverec_impl, (const char *)coeffs + first * e * total, nb, lens, level, taps, flags,
+                    (char *)x_out + first * e * nout, st);
+  });
 }

@@ -1,6 +1,6 @@
 // Pieces shared by the generic (filterbank.cu) and the register-blocked
-// (filterbank_fast.cu) MODWT / DWT kernels: tap tables, the DWT level plan, 1-D TMA
-// bulk copies (cp.async.bulk + mbarrier / bulk_group) and the batched host driver.
+// (filterbank_fast.cu) MODWT / DWT kernels: tap tables, the DWT level plan and 1-D TMA
+// bulk copies (cp.async.bulk + mbarrier / bulk_group).
 #pragma once
 
 #include <algorithm>
@@ -113,27 +113,6 @@ __device__ __forceinline__ int reflect_sym(int p, int n) {
 }
 
 // ---- host side -------------------------------------------------------------------------
-// Runs `launch(d_in, d_out, rows)` over the batch, staging host buffers through the arena.
-template <typename F>
-static int run_batched(const void *in, void *out, int64_t batch, size_t in_row, size_t out_row, int flags,
-                       cudaStream_t st, F launch) {
-  if (flags & WTB_DEVICE_PTRS) return launch(in, out, batch);
-  const size_t budget = size_t(1) << 30;
-  const int64_t rows = std::max<int64_t>(1, std::min<int64_t>(batch, (int64_t)(budget / (in_row + out_row))));
-  auto al = [](size_t b) { return (b + 255) / 256 * 256; };
-  void *stage = nullptr;
-  WTB_TRY(staging_reserve(al(in_row * rows) + al(out_row * rows), &stage));
-  char *d_in = (char *)stage, *d_out = d_in + al(in_row * rows);
-  for (int64_t b0 = 0; b0 < batch; b0 += rows) {
-    const int64_t nb = std::min(rows, batch - b0);
-    WTB_CUDA(cudaMemcpyAsync(d_in, (const char *)in + b0 * in_row, in_row * nb, cudaMemcpyHostToDevice, st));
-    WTB_TRY(launch(d_in, d_out, nb));
-    WTB_TRY(copy_to_host((char *)out + b0 * out_row, d_out, out_row * nb, st));
-    WTB_CUDA(cudaStreamSynchronize(st));
-  }
-  return WTB_OK;
-}
-
 constexpr size_t kSmemLimit = 227 * 1024;
 
 template <typename K> static int set_smem(K kernel, size_t bytes) {

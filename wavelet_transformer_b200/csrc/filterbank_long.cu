@@ -6,7 +6,7 @@
 // gathers its inputs through L1 / L2: a warp's reads for one tap are contiguous.  The level-to-level
 // intermediates live in two arena buffers, and series run in waves whose two buffers fit 64 MiB (half the
 // B200's 126 MB L2), so level j+1 finds level j's output in L2.  A series' arithmetic does not depend on its
-// wave, so results do not depend on the batch, the host chunk of run_batched, the pool or the pointers.
+// wave, so results do not depend on the batch, the host chunk of stage_rows, the pool or the pointers.
 //
 //   k_modwt_long     w_j, v_j from v_{j-1} (k_modwt)                      J launches per wave
 //   k_synth_long     h / g synthesis at one dilation: the inverse MODWT     J launches per wave (wtb_imodwt)
@@ -35,8 +35,6 @@ static int64_t long_wave(size_t per_series, int64_t batch) {
 static dim3 long_grid(int64_t n, int64_t series, int rows = 1) {
   return dim3((unsigned)((n + kLongThreads - 1) / kLongThreads), (unsigned)series, (unsigned)rows);
 }
-
-static size_t al256(size_t b) { return (b + 255) / 256 * 256; }
 
 // Taps in the kernel's precision and the level's circular offsets (2^(j-1) l) mod n, from 64-bit host arithmetic
 // so that a dilated filter that wraps the series several times is exact.
@@ -189,7 +187,7 @@ template <typename T>
 int modwt_long(const void *x, int64_t batch, int n, const Taps &taps, int J, int flags, void *out, cudaStream_t st) {
   const int64_t ser = (int64_t)(J + 1) * n;
   const int64_t cap = long_wave(2 * sizeof(T) * (size_t)n, batch);
-  const size_t b_buf = al256(sizeof(T) * (size_t)cap * n);
+  const size_t b_buf = align256(sizeof(T) * (size_t)cap * n);
   T *buf[2] = {nullptr, nullptr};
   if (J > 1) {
     void *scratch = nullptr;
@@ -197,31 +195,32 @@ int modwt_long(const void *x, int64_t batch, int n, const Taps &taps, int J, int
     buf[0] = (T *)scratch;
     buf[1] = (T *)((char *)scratch + b_buf);
   }
-  return run_batched(x, out, batch, sizeof(T) * n, sizeof(T) * (size_t)ser, flags, st,
-                     [&](const void *di, void *dout, int64_t nb) -> int {
-                       for (int64_t b0 = 0; b0 < nb; b0 += cap) {
-                         const int64_t nw = std::min(cap, nb - b0);
-                         const T *xin = (const T *)di + b0 * n;
-                         T *o = (T *)dout + b0 * ser;
-                         // level j reads v_{j-1} (x, then buf[(j-1)&1]) and writes v_j to buf[j&1], v_J to row J
-                         for (int j = 1; j <= J; ++j) {
-                           const T *src = j == 1 ? xin : buf[(j - 1) & 1];
-                           T *dst = j == J ? o + (int64_t)J * n : buf[j & 1];
-                           k_modwt_long<T><<<long_grid(n, nw), kLongThreads, 0, st>>>(
-                               src, n, n, long_taps<T>(taps, j, n), o + (int64_t)(j - 1) * n, ser, dst,
-                               j == J ? ser : n);
-                           WTB_LAUNCH_CHECK();
-                         }
-                       }
-                       return WTB_OK;
-                     });
+  const size_t in_row = sizeof(T) * n, out_row = sizeof(T) * (size_t)ser;
+  return stage_rows(batch, host_rows(batch, in_row + out_row, flags), flags, st, {{x, in_row}}, {{out, out_row}}, 0,
+                    [&](const void *const *di, void *const *dout, void *, int64_t, int64_t nb) -> int {
+                      for (int64_t b0 = 0; b0 < nb; b0 += cap) {
+                        const int64_t nw = std::min(cap, nb - b0);
+                        const T *xin = (const T *)di[0] + b0 * n;
+                        T *o = (T *)dout[0] + b0 * ser;
+                        // level j reads v_{j-1} (x, then buf[(j-1)&1]) and writes v_j to buf[j&1], v_J to row J
+                        for (int j = 1; j <= J; ++j) {
+                          const T *src = j == 1 ? xin : buf[(j - 1) & 1];
+                          T *dst = j == J ? o + (int64_t)J * n : buf[j & 1];
+                          k_modwt_long<T><<<long_grid(n, nw), kLongThreads, 0, st>>>(
+                              src, n, n, long_taps<T>(taps, j, n), o + (int64_t)(j - 1) * n, ser, dst,
+                              j == J ? ser : n);
+                          WTB_LAUNCH_CHECK();
+                        }
+                      }
+                      return WTB_OK;
+                    });
 }
 
 template <typename T>
 int imodwt_long(const void *w, int64_t batch, int n, const Taps &taps, int J, int flags, void *out, cudaStream_t st) {
   const int64_t ser = (int64_t)(J + 1) * n;
   const int64_t cap = long_wave(2 * sizeof(T) * (size_t)n, batch);
-  const size_t b_buf = al256(sizeof(T) * (size_t)cap * n);
+  const size_t b_buf = align256(sizeof(T) * (size_t)cap * n);
   T *buf[2] = {nullptr, nullptr};
   if (J > 1) {
     void *scratch = nullptr;
@@ -229,27 +228,28 @@ int imodwt_long(const void *w, int64_t batch, int n, const Taps &taps, int J, in
     buf[0] = (T *)scratch;
     buf[1] = (T *)((char *)scratch + b_buf);
   }
-  return run_batched(w, out, batch, sizeof(T) * (size_t)ser, sizeof(T) * n, flags, st,
-                     [&](const void *di, void *dout, int64_t nb) -> int {
-                       for (int64_t b0 = 0; b0 < nb; b0 += cap) {
-                         const int64_t nw = std::min(cap, nb - b0);
-                         const T *wi = (const T *)di + b0 * ser;
-                         // level j reads v_j (row J, then buf[(j+1)&1]) and writes v_{j-1} to buf[j&1], x at j = 1
-                         for (int j = J; j >= 1; --j) {
-                           SynthRows<T> r;
-                           r.a = wi + (int64_t)(j - 1) * n;
-                           r.a_ser = ser;
-                           r.b = j == J ? wi + (int64_t)J * n : buf[(j + 1) & 1];
-                           r.b_ser = j == J ? ser : n;
-                           r.zb = 0;
-                           r.out = j == 1 ? (T *)dout + b0 * n : buf[j & 1];
-                           r.out_ser = n;
-                           k_synth_long<T><<<long_grid(n, nw), kLongThreads, 0, st>>>(r, n, long_taps<T>(taps, j, n));
-                           WTB_LAUNCH_CHECK();
-                         }
-                       }
-                       return WTB_OK;
-                     });
+  const size_t in_row = sizeof(T) * (size_t)ser, out_row = sizeof(T) * n;
+  return stage_rows(batch, host_rows(batch, in_row + out_row, flags), flags, st, {{w, in_row}}, {{out, out_row}}, 0,
+                    [&](const void *const *di, void *const *dout, void *, int64_t, int64_t nb) -> int {
+                      for (int64_t b0 = 0; b0 < nb; b0 += cap) {
+                        const int64_t nw = std::min(cap, nb - b0);
+                        const T *wi = (const T *)di[0] + b0 * ser;
+                        // level j reads v_j (row J, then buf[(j+1)&1]) and writes v_{j-1} to buf[j&1], x at j = 1
+                        for (int j = J; j >= 1; --j) {
+                          SynthRows<T> r;
+                          r.a = wi + (int64_t)(j - 1) * n;
+                          r.a_ser = ser;
+                          r.b = j == J ? wi + (int64_t)J * n : buf[(j + 1) & 1];
+                          r.b_ser = j == J ? ser : n;
+                          r.zb = 0;
+                          r.out = j == 1 ? (T *)dout[0] + b0 * n : buf[j & 1];
+                          r.out_ser = n;
+                          k_synth_long<T><<<long_grid(n, nw), kLongThreads, 0, st>>>(r, n, long_taps<T>(taps, j, n));
+                          WTB_LAUNCH_CHECK();
+                        }
+                      }
+                      return WTB_OK;
+                    });
 }
 
 // D_j = G_1' .. G_{j-1}' H_j' w_j and S_J = G_1' .. G_J' v_J, level k = J .. 1 in one launch each: row k-1 enters
@@ -259,7 +259,7 @@ int mra_taps_long(const void *w, int64_t batch, int n, const Taps &taps, int J, 
                   cudaStream_t st) {
   const int64_t ser = (int64_t)(J + 1) * n;
   const int64_t cap = long_wave(2 * sizeof(T) * (size_t)ser, batch);
-  const size_t b_buf = al256(sizeof(T) * (size_t)(cap * ser));
+  const size_t b_buf = align256(sizeof(T) * (size_t)(cap * ser));
   T *buf[2] = {nullptr, nullptr};
   if (J > 1) {
     void *scratch = nullptr;
@@ -267,28 +267,29 @@ int mra_taps_long(const void *w, int64_t batch, int n, const Taps &taps, int J, 
     buf[0] = (T *)scratch;
     buf[1] = (T *)((char *)scratch + b_buf);
   }
-  return run_batched(w, out, batch, sizeof(T) * (size_t)ser, sizeof(T) * (size_t)ser, flags, st,
-                     [&](const void *di, void *dout, int64_t nb) -> int {
-                       for (int64_t b0 = 0; b0 < nb; b0 += cap) {
-                         const int64_t nw = std::min(cap, nb - b0);
-                         const T *wi = (const T *)di + b0 * ser;
-                         // level k writes rows k-1 .. J to buf[k&1] (the output at k = 1) in the [J+1, n] layout
-                         for (int k = J; k >= 1; --k) {
-                           SynthRows<T> r;
-                           r.a = wi + (int64_t)(k - 1) * n;
-                           r.a_ser = ser;
-                           r.b = k == J ? wi + (int64_t)J * n : buf[(k + 1) & 1] + (int64_t)k * n;
-                           r.b_ser = ser;
-                           r.zb = 1;
-                           r.out = (k == 1 ? (T *)dout + b0 * ser : buf[k & 1]) + (int64_t)(k - 1) * n;
-                           r.out_ser = ser;
-                           k_synth_long<T><<<long_grid(n, nw, J - k + 2), kLongThreads, 0, st>>>(
-                               r, n, long_taps<T>(taps, k, n));
-                           WTB_LAUNCH_CHECK();
-                         }
-                       }
-                       return WTB_OK;
-                     });
+  const size_t in_row = sizeof(T) * (size_t)ser, out_row = sizeof(T) * (size_t)ser;
+  return stage_rows(batch, host_rows(batch, in_row + out_row, flags), flags, st, {{w, in_row}}, {{out, out_row}}, 0,
+                    [&](const void *const *di, void *const *dout, void *, int64_t, int64_t nb) -> int {
+                      for (int64_t b0 = 0; b0 < nb; b0 += cap) {
+                        const int64_t nw = std::min(cap, nb - b0);
+                        const T *wi = (const T *)di[0] + b0 * ser;
+                        // level k writes rows k-1 .. J to buf[k&1] (the output at k = 1) in the [J+1, n] layout
+                        for (int k = J; k >= 1; --k) {
+                          SynthRows<T> r;
+                          r.a = wi + (int64_t)(k - 1) * n;
+                          r.a_ser = ser;
+                          r.b = k == J ? wi + (int64_t)J * n : buf[(k + 1) & 1] + (int64_t)k * n;
+                          r.b_ser = ser;
+                          r.zb = 1;
+                          r.out = (k == 1 ? (T *)dout[0] + b0 * ser : buf[k & 1]) + (int64_t)(k - 1) * n;
+                          r.out_ser = ser;
+                          k_synth_long<T><<<long_grid(n, nw, J - k + 2), kLongThreads, 0, st>>>(
+                              r, n, long_taps<T>(taps, k, n));
+                          WTB_LAUNCH_CHECK();
+                        }
+                      }
+                      return WTB_OK;
+                    });
 }
 
 template <typename T>
@@ -308,7 +309,7 @@ int mra_filt_long(const void *w, int64_t batch, int n, const double *filt, int J
     first[j + 1] = (int)off.size();
   }
   const size_t nnz = std::max<size_t>(1, off.size());
-  const size_t b_first = al256(sizeof(int) * (J + 2)), b_off = al256(sizeof(int) * nnz);
+  const size_t b_first = align256(sizeof(int) * (J + 2)), b_off = align256(sizeof(int) * nnz);
   void *scratch = nullptr;
   WTB_TRY(arena_reserve(b_first + b_off + sizeof(T) * nnz, &scratch));
   int *d_first = (int *)scratch, *d_off = (int *)((char *)scratch + b_first);
@@ -321,16 +322,17 @@ int mra_filt_long(const void *w, int64_t batch, int n, const double *filt, int J
   WTB_CUDA(cudaStreamSynchronize(st));  // the tables are locals
   const int64_t ser = (int64_t)(J + 1) * n;
   const int64_t cap = long_wave(2 * sizeof(T) * (size_t)ser, batch);
-  return run_batched(w, out, batch, sizeof(T) * (size_t)ser, sizeof(T) * (size_t)ser, flags, st,
-                     [&](const void *di, void *dout, int64_t nb) -> int {
-                       for (int64_t b0 = 0; b0 < nb; b0 += cap) {
-                         const int64_t nw = std::min(cap, nb - b0);
-                         k_mra_filt_long<T><<<long_grid(n, nw, J + 1), kLongThreads, 0, st>>>(
-                             (const T *)di + b0 * ser, n, J + 1, d_first, d_off, d_val, (T *)dout + b0 * ser);
-                         WTB_LAUNCH_CHECK();
-                       }
-                       return WTB_OK;
-                     });
+  const size_t in_row = sizeof(T) * (size_t)ser, out_row = sizeof(T) * (size_t)ser;
+  return stage_rows(batch, host_rows(batch, in_row + out_row, flags), flags, st, {{w, in_row}}, {{out, out_row}}, 0,
+                    [&](const void *const *di, void *const *dout, void *, int64_t, int64_t nb) -> int {
+                      for (int64_t b0 = 0; b0 < nb; b0 += cap) {
+                        const int64_t nw = std::min(cap, nb - b0);
+                        k_mra_filt_long<T><<<long_grid(n, nw, J + 1), kLongThreads, 0, st>>>(
+                            (const T *)di[0] + b0 * ser, n, J + 1, d_first, d_off, d_val, (T *)dout[0] + b0 * ser);
+                        WTB_LAUNCH_CHECK();
+                      }
+                      return WTB_OK;
+                    });
 }
 
 template <typename T>
@@ -340,7 +342,7 @@ int wavedec_long(const void *x, int64_t batch, const LevelPlan &plan, const Taps
   const int64_t total = plan.total;
   const int64_t cap = long_wave(2 * sizeof(T) * (size_t)n, batch);
   const int64_t mid = plan.level > 0 ? plan.len[plan.level] : 0;  // cA_1, the longest intermediate
-  const size_t b_buf = al256(sizeof(T) * (size_t)(cap * mid));
+  const size_t b_buf = align256(sizeof(T) * (size_t)(cap * mid));
   T *buf[2] = {nullptr, nullptr};
   if (plan.level > 1) {
     void *scratch = nullptr;
@@ -348,32 +350,33 @@ int wavedec_long(const void *x, int64_t batch, const LevelPlan &plan, const Taps
     buf[0] = (T *)scratch;
     buf[1] = (T *)((char *)scratch + b_buf);
   }
-  return run_batched(x, coeffs, batch, sizeof(T) * n, sizeof(T) * (size_t)total, flags, st,
-                     [&](const void *di, void *dout, int64_t nb) -> int {
-                       if (plan.level == 0) {  // cA_0 is the signal
-                         WTB_CUDA(cudaMemcpyAsync(dout, di, sizeof(T) * (size_t)(nb * n), cudaMemcpyDeviceToDevice, st));
-                         return WTB_OK;
-                       }
-                       for (int64_t b0 = 0; b0 < nb; b0 += cap) {
-                         const int64_t nw = std::min(cap, nb - b0);
-                         T *o = (T *)dout + b0 * total;
-                         int cur = n;
-                         // level lev reads cA_{lev-1} (x, then buf[(lev-1)&1]) and writes cA_lev to buf[lev&1],
-                         // cA_L to slot 0
-                         for (int lev = 1; lev <= plan.level; ++lev) {
-                           const int slot = plan.level - lev + 1;  // cD_lev
-                           const int nout = plan.len[slot];
-                           const bool last = lev == plan.level;
-                           const T *src = lev == 1 ? (const T *)di + b0 * n : buf[(lev - 1) & 1];
-                           k_dwt_long<T><<<long_grid(nout, nw), kLongThreads, 0, st>>>(
-                               src, lev == 1 ? n : mid, cur, nout, long_taps<T>(taps, 0, 1), o + plan.off[slot], total,
-                               last ? o : buf[lev & 1], last ? total : mid);
-                           WTB_LAUNCH_CHECK();
-                           cur = nout;
-                         }
-                       }
-                       return WTB_OK;
-                     });
+  const size_t in_row = sizeof(T) * n, out_row = sizeof(T) * (size_t)total;
+  return stage_rows(batch, host_rows(batch, in_row + out_row, flags), flags, st, {{x, in_row}}, {{coeffs, out_row}}, 0,
+                    [&](const void *const *di, void *const *dout, void *, int64_t, int64_t nb) -> int {
+                      if (plan.level == 0) {  // cA_0 is the signal
+                        WTB_CUDA(cudaMemcpyAsync(dout[0], di[0], sizeof(T) * (size_t)(nb * n), cudaMemcpyDeviceToDevice, st));
+                        return WTB_OK;
+                      }
+                      for (int64_t b0 = 0; b0 < nb; b0 += cap) {
+                        const int64_t nw = std::min(cap, nb - b0);
+                        T *o = (T *)dout[0] + b0 * total;
+                        int cur = n;
+                        // level lev reads cA_{lev-1} (x, then buf[(lev-1)&1]) and writes cA_lev to buf[lev&1],
+                        // cA_L to slot 0
+                        for (int lev = 1; lev <= plan.level; ++lev) {
+                          const int slot = plan.level - lev + 1;  // cD_lev
+                          const int nout = plan.len[slot];
+                          const bool last = lev == plan.level;
+                          const T *src = lev == 1 ? (const T *)di[0] + b0 * n : buf[(lev - 1) & 1];
+                          k_dwt_long<T><<<long_grid(nout, nw), kLongThreads, 0, st>>>(
+                              src, lev == 1 ? n : mid, cur, nout, long_taps<T>(taps, 0, 1), o + plan.off[slot], total,
+                              last ? o : buf[lev & 1], last ? total : mid);
+                          WTB_LAUNCH_CHECK();
+                          cur = nout;
+                        }
+                      }
+                      return WTB_OK;
+                    });
 }
 
 template <typename T>
@@ -384,7 +387,7 @@ int waverec_long(const void *coeffs, int64_t batch, const LevelPlan &plan, const
   const int64_t cap = long_wave(2 * sizeof(T) * (size_t)nout, batch);
   int64_t mid = 0;  // longest intermediate approximation
   for (int slot = 1; slot < plan.level; ++slot) mid = std::max<int64_t>(mid, 2 * (int64_t)plan.len[slot] - taps.L + 2);
-  const size_t b_buf = al256(sizeof(T) * (size_t)(cap * mid));
+  const size_t b_buf = align256(sizeof(T) * (size_t)(cap * mid));
   T *buf[2] = {nullptr, nullptr};
   if (plan.level > 1) {
     void *scratch = nullptr;
@@ -392,29 +395,30 @@ int waverec_long(const void *coeffs, int64_t batch, const LevelPlan &plan, const
     buf[0] = (T *)scratch;
     buf[1] = (T *)((char *)scratch + b_buf);
   }
-  return run_batched(coeffs, x, batch, sizeof(T) * (size_t)total, sizeof(T) * (size_t)nout, flags, st,
-                     [&](const void *di, void *dout, int64_t nb) -> int {
-                       if (plan.level == 0) {  // the signal is cA_0
-                         WTB_CUDA(cudaMemcpyAsync(dout, di, sizeof(T) * (size_t)(nb * nout), cudaMemcpyDeviceToDevice, st));
-                         return WTB_OK;
-                       }
-                       for (int64_t b0 = 0; b0 < nb; b0 += cap) {
-                         const int64_t nw = std::min(cap, nb - b0);
-                         const T *c = (const T *)di + b0 * total;
-                         // slot s reads cA (slot 0, then buf[(s-1)&1]) and cD (slot s) and writes buf[s&1], x last
-                         for (int slot = 1; slot <= plan.level; ++slot) {
-                           const int m = plan.len[slot];
-                           const int len = 2 * m - taps.L + 2;
-                           const bool last = slot == plan.level;
-                           k_idwt_long<T><<<long_grid(len, nw), kLongThreads, 0, st>>>(
-                               slot == 1 ? c : buf[(slot - 1) & 1], slot == 1 ? total : mid, c + plan.off[slot], total,
-                               m, len, long_taps<T>(taps, 0, 1), last ? (T *)dout + b0 * nout : buf[slot & 1],
-                               last ? nout : mid);
-                           WTB_LAUNCH_CHECK();
-                         }
-                       }
-                       return WTB_OK;
-                     });
+  const size_t in_row = sizeof(T) * (size_t)total, out_row = sizeof(T) * (size_t)nout;
+  return stage_rows(batch, host_rows(batch, in_row + out_row, flags), flags, st, {{coeffs, in_row}}, {{x, out_row}}, 0,
+                    [&](const void *const *di, void *const *dout, void *, int64_t, int64_t nb) -> int {
+                      if (plan.level == 0) {  // the signal is cA_0
+                        WTB_CUDA(cudaMemcpyAsync(dout[0], di[0], sizeof(T) * (size_t)(nb * nout), cudaMemcpyDeviceToDevice, st));
+                        return WTB_OK;
+                      }
+                      for (int64_t b0 = 0; b0 < nb; b0 += cap) {
+                        const int64_t nw = std::min(cap, nb - b0);
+                        const T *c = (const T *)di[0] + b0 * total;
+                        // slot s reads cA (slot 0, then buf[(s-1)&1]) and cD (slot s) and writes buf[s&1], x last
+                        for (int slot = 1; slot <= plan.level; ++slot) {
+                          const int m = plan.len[slot];
+                          const int len = 2 * m - taps.L + 2;
+                          const bool last = slot == plan.level;
+                          k_idwt_long<T><<<long_grid(len, nw), kLongThreads, 0, st>>>(
+                              slot == 1 ? c : buf[(slot - 1) & 1], slot == 1 ? total : mid, c + plan.off[slot], total,
+                              m, len, long_taps<T>(taps, 0, 1), last ? (T *)dout[0] + b0 * nout : buf[slot & 1],
+                              last ? nout : mid);
+                          WTB_LAUNCH_CHECK();
+                        }
+                      }
+                      return WTB_OK;
+                    });
 }
 
 #define WTB_INSTANTIATE(T)                                                                                         \

@@ -51,79 +51,42 @@ template <typename T>
 static int ratio_impl(const void *plane, int64_t batch, int S, int n0, const double *signif, int64_t sig_rows, int flags,
                       void *power_out, void *ratio_out, cudaStream_t st) {
   const bool dev = flags & WTB_DEVICE_PTRS, cx = flags & WTB_PLANE_COMPLEX;
-  auto al = [](size_t b) { return (b + 255) / 256 * 256; };
   const size_t in_row = sizeof(T) * (size_t)S * n0 * (cx ? 2 : 1), out_row = sizeof(T) * (size_t)S * n0;
-  const size_t b_sig = al(sizeof(double) * (size_t)sig_rows * S);
   void *prm = nullptr;
   const double *d_sig = signif;
   // signif is small and always comes from the host side of the caller's pipeline unless DEVICE_PTRS
   if (!dev) {
-    WTB_TRY(arena_reserve(b_sig, &prm));
+    WTB_TRY(arena_reserve(align256(sizeof(double) * (size_t)sig_rows * S), &prm));
     WTB_CUDA(cudaMemcpyAsync(prm, signif, sizeof(double) * (size_t)sig_rows * S, cudaMemcpyHostToDevice, st));
     d_sig = (const double *)prm;
   }
-  const int64_t chunk = dev ? batch : std::max<int64_t>(1, std::min<int64_t>(batch, (int64_t)((size_t(1) << 30) / (in_row + 2 * out_row))));
-  const T *d_in = (const T *)plane;
-  T *d_pow = (T *)power_out, *d_rat = (T *)ratio_out;
-  if (!dev) {
-    void *stage = nullptr;
-    WTB_TRY(staging_reserve(al(in_row * chunk) + 2 * al(out_row * chunk), &stage));
-    d_in = (const T *)stage;
-    d_pow = power_out ? (T *)((char *)stage + al(in_row * chunk)) : nullptr;
-    d_rat = ratio_out ? (T *)((char *)stage + al(in_row * chunk) + al(out_row * chunk)) : nullptr;
-  }
-  for (int64_t b0 = 0; b0 < batch; b0 += chunk) {
-    const int64_t nb = std::min(chunk, batch - b0), rows = nb * S;
-    const T *in = dev ? (const T *)((const char *)plane + b0 * in_row) : d_in;
-    T *pw = dev ? (power_out ? (T *)((char *)power_out + b0 * out_row) : nullptr) : d_pow;
-    T *rt = dev ? (ratio_out ? (T *)((char *)ratio_out + b0 * out_row) : nullptr) : d_rat;
-    if (!dev) WTB_CUDA(cudaMemcpyAsync((void *)d_in, (const char *)plane + b0 * in_row, in_row * nb, cudaMemcpyHostToDevice, st));
-    const unsigned gy = (unsigned)std::min<int64_t>(rows, 65535), gz = (unsigned)((rows + gy - 1) / gy);
-    WTB_REQUIRE(gz <= 65535, WTB_EUNSUPPORTED, "batch too large for one launch");
-    const dim3 grid((unsigned)std::min(8, (n0 + 255) / 256), gy, gz);
-    const double *sg = d_sig + (sig_rows > 1 ? b0 * S : 0);
-    if (cx) k_ratio_planes<T, true><<<grid, 256, 0, st>>>(in, rows, S, n0, sg, sig_rows > 1, pw, rt);
-    else k_ratio_planes<T, false><<<grid, 256, 0, st>>>(in, rows, S, n0, sg, sig_rows > 1, pw, rt);
-    WTB_LAUNCH_CHECK();
-    if (!dev) {
-      if (power_out) WTB_TRY(copy_to_host((char *)power_out + b0 * out_row, d_pow, out_row * nb, st));
-      if (ratio_out) WTB_TRY(copy_to_host((char *)ratio_out + b0 * out_row, d_rat, out_row * nb, st));
-      WTB_CUDA(cudaStreamSynchronize(st));
-    }
-  }
-  return WTB_OK;
+  return stage_rows(batch, host_rows(batch, in_row + 2 * out_row, flags), flags, st, {{plane, in_row}},
+                    {{power_out, out_row}, {ratio_out, out_row}}, 0,
+                    [&](const void *const *in, void *const *out, void *, int64_t b0, int64_t nb) {
+                      const int64_t rows = nb * S;
+                      const unsigned gy = (unsigned)std::min<int64_t>(rows, 65535), gz = (unsigned)((rows + gy - 1) / gy);
+                      WTB_REQUIRE(gz <= 65535, WTB_EUNSUPPORTED, "batch too large for one launch");
+                      const dim3 grid((unsigned)std::min(8, (n0 + 255) / 256), gy, gz);
+                      const double *sg = d_sig + (sig_rows > 1 ? b0 * S : 0);
+                      const T *src = (const T *)in[0];
+                      T *pw = (T *)out[0], *rt = (T *)out[1];
+                      if (cx) k_ratio_planes<T, true><<<grid, 256, 0, st>>>(src, rows, S, n0, sg, sig_rows > 1, pw, rt);
+                      else k_ratio_planes<T, false><<<grid, 256, 0, st>>>(src, rows, S, n0, sg, sig_rows > 1, pw, rt);
+                      WTB_LAUNCH_CHECK();
+                      return WTB_OK;
+                    });
 }
 
 template <typename T>
 static int arrows_impl(const void *phase, int64_t count, int flags, void *u_out, void *v_out, cudaStream_t st) {
-  const bool dev = flags & WTB_DEVICE_PTRS;
-  auto al = [](size_t b) { return (b + 255) / 256 * 256; };
-  const int64_t chunk = dev ? count : std::min<int64_t>(count, (int64_t)((size_t(1) << 30) / (3 * sizeof(T))));
-  const T *d_in = (const T *)phase;
-  T *d_u = (T *)u_out, *d_v = (T *)v_out;
-  if (!dev) {
-    void *stage = nullptr;
-    WTB_TRY(staging_reserve(3 * al(sizeof(T) * chunk), &stage));
-    d_in = (const T *)stage;
-    d_u = u_out ? (T *)((char *)stage + al(sizeof(T) * chunk)) : nullptr;
-    d_v = v_out ? (T *)((char *)stage + 2 * al(sizeof(T) * chunk)) : nullptr;
-  }
-  for (int64_t i0 = 0; i0 < count; i0 += chunk) {
-    const int64_t n = std::min(chunk, count - i0);
-    const T *in = dev ? (const T *)phase + i0 : d_in;
-    T *pu = dev ? (u_out ? (T *)u_out + i0 : nullptr) : d_u;
-    T *pv = dev ? (v_out ? (T *)v_out + i0 : nullptr) : d_v;
-    if (!dev) WTB_CUDA(cudaMemcpyAsync((void *)d_in, (const T *)phase + i0, sizeof(T) * n, cudaMemcpyHostToDevice, st));
-    const unsigned blocks = (unsigned)std::min<int64_t>((n + 255) / 256, (int64_t)sm_count() * 16);
-    k_phase_arrows<T><<<blocks, 256, 0, st>>>(in, n, pu, pv);
-    WTB_LAUNCH_CHECK();
-    if (!dev) {
-      if (u_out) WTB_TRY(copy_to_host((T *)u_out + i0, d_u, sizeof(T) * n, st));
-      if (v_out) WTB_TRY(copy_to_host((T *)v_out + i0, d_v, sizeof(T) * n, st));
-      WTB_CUDA(cudaStreamSynchronize(st));
-    }
-  }
-  return WTB_OK;
+  return stage_rows(count, host_rows(count, 3 * sizeof(T), flags), flags, st, {{phase, sizeof(T)}},
+                    {{u_out, sizeof(T)}, {v_out, sizeof(T)}}, 0,
+                    [&](const void *const *in, void *const *out, void *, int64_t, int64_t n) {
+                      const unsigned blocks = (unsigned)std::min<int64_t>((n + 255) / 256, (int64_t)sm_count() * 16);
+                      k_phase_arrows<T><<<blocks, 256, 0, st>>>((const T *)in[0], n, (T *)out[0], (T *)out[1]);
+                      WTB_LAUNCH_CHECK();
+                      return WTB_OK;
+                    });
 }
 
 }  // namespace wtb

@@ -75,31 +75,17 @@ __global__ void k_series_prep(const T *__restrict__ x, int64_t batch, int n, int
 template <typename T>
 static int prep_impl(const void *x, int64_t batch, int n, int mode, int flags, void *y, double *ar1,
                      cudaStream_t st) {
-  const bool dev = flags & WTB_DEVICE_PTRS;
-  const T *d_x = (const T *)x;
-  T *d_y = (T *)y;
-  double *d_ar1 = ar1;
-  if (!dev) {
-    auto al = [](size_t b) { return (b + 255) / 256 * 256; };
-    void *stage = nullptr;
-    const size_t bx = al(sizeof(T) * (size_t)batch * n);
-    WTB_TRY(staging_reserve(2 * bx + al(sizeof(double) * batch), &stage));
-    d_x = (const T *)stage;
-    d_y = y ? (T *)((char *)stage + bx) : nullptr;
-    d_ar1 = ar1 ? (double *)((char *)stage + 2 * bx) : nullptr;
-    WTB_CUDA(cudaMemcpyAsync((void *)d_x, x, sizeof(T) * (size_t)batch * n, cudaMemcpyHostToDevice, st));
-  }
-  const int warps = 8;
-  const int64_t blocks = (batch + warps - 1) / warps;
-  WTB_REQUIRE(blocks < (1LL << 31), WTB_EUNSUPPORTED, "batch too large");
-  k_series_prep<T><<<(unsigned)blocks, warps * 32, 0, st>>>(d_x, batch, n, mode, d_y, d_ar1);
-  WTB_LAUNCH_CHECK();
-  if (!dev) {
-    if (y) WTB_TRY(copy_to_host(y, d_y, sizeof(T) * (size_t)batch * n, st));
-    if (ar1) WTB_TRY(copy_to_host(ar1, d_ar1, sizeof(double) * batch, st));
-    WTB_CUDA(cudaStreamSynchronize(st));
-  }
-  return WTB_OK;
+  // one chunk: the whole batch
+  return stage_rows(batch, batch, flags, st, {{x, sizeof(T) * n}}, {{y, sizeof(T) * n}, {ar1, sizeof(double)}}, 0,
+                    [&](const void *const *in, void *const *out, void *, int64_t, int64_t nb) {
+                      const int warps = 8;
+                      const int64_t blocks = (nb + warps - 1) / warps;
+                      WTB_REQUIRE(blocks < (1LL << 31), WTB_EUNSUPPORTED, "batch too large");
+                      k_series_prep<T><<<(unsigned)blocks, warps * 32, 0, st>>>((const T *)in[0], nb, n, mode,
+                                                                                (T *)out[0], (double *)out[1]);
+                      WTB_LAUNCH_CHECK();
+                      return WTB_OK;
+                    });
 }
 
 }  // namespace wtb

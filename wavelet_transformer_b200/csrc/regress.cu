@@ -64,10 +64,9 @@ static int ols_impl(const void *x, int64_t x_rows, const void *y, int64_t y_rows
   const T *d_x = (const T *)x, *d_y = (const T *)y;
   double *d_s = stats;
   if (!dev) {
-    auto al = [](size_t b) { return (b + 255) / 256 * 256; };
-    const size_t bx = al(sizeof(T) * (size_t)x_rows * n), by = al(sizeof(T) * (size_t)y_rows * n);
+    const size_t bx = align256(sizeof(T) * (size_t)x_rows * n), by = align256(sizeof(T) * (size_t)y_rows * n);
     void *stage = nullptr;
-    WTB_TRY(staging_reserve(bx + by + al(sizeof(double) * 8 * rows), &stage));
+    WTB_TRY(staging_reserve(bx + by + align256(sizeof(double) * 8 * rows), &stage));
     d_x = (const T *)stage;
     d_y = (const T *)((char *)stage + bx);
     d_s = (double *)((char *)stage + bx + by);

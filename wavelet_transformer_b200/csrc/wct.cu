@@ -196,13 +196,12 @@ static int wct_device(const T *d_y, int64_t pairs, int n0, int N, double dt, dou
   // daughters hold (f0 >= kMinF0), its shared-memory rows and its boxcar ring fit
   const bool fast_fwd = std::is_same<T, float>::value && !generic && N == 4096;
   const bool fast = fast_fwd && f0 >= kMinF0 && S <= kMaxRowsC && win.K <= 32;
-  auto al = [](size_t b) { return (b + 255) / 256 * 256; };
-  const size_t b_sc = al(sizeof(double) * S);
-  const size_t b_rng = al(sizeof(int) * S);
-  const size_t b_xh = al(sizeof(cplx<T>) * (size_t)pairs * 2 * N);
-  const size_t b_ts = smooth ? al(sizeof(vec4<T>) * (size_t)pairs * S * N) : 0;  // N >= n0: also fits the fast path's spectra
+  const size_t b_sc = align256(sizeof(double) * S);
+  const size_t b_rng = align256(sizeof(int) * S);
+  const size_t b_xh = align256(sizeof(cplx<T>) * (size_t)pairs * 2 * N);
+  const size_t b_ts = smooth ? align256(sizeof(vec4<T>) * (size_t)pairs * S * N) : 0;  // N >= n0: also fits the fast path's spectra
   void *scratch = nullptr;
-  const size_t b_rows = al(32 * (size_t)S);   // the fast path's row parameters (WRow)
+  const size_t b_rows = align256(32 * (size_t)S);   // the fast path's row parameters (WRow)
   WTB_TRY(arena_reserve(b_sc + 2 * b_rng + b_rows + b_xh + b_ts, &scratch));
   char *p = (char *)scratch;
   void *d_rows_scratch = p; p += b_rows;
@@ -243,67 +242,30 @@ template <typename T> static size_t pair_bytes(int n0, int N, int S) {
   return sizeof(cplx<T>) * 2 * (size_t)N + sizeof(vec4<T>) * (size_t)S * N;
 }
 
-static thread_local bool g_in_shard = false;   // set on a pool worker while it runs its block
-
 template <typename T>
 static int xwt_wct_entry(const void *y1, const void *y2, int64_t batch, int n0, int N, double dt,
                          double dj, const Axes &ax, double f0, int flags, void *wct_out,
                          void *phase_out, void *w12_out, cudaStream_t st) {
   const int S = ax.J + 1;
-  const size_t plane = (size_t)S * n0;
-  // host buffers, several GPUs (wtb_init_multi): contiguous blocks of pairs, one per device
-  if (!(flags & WTB_DEVICE_PTRS) && pool_size() > 1 && batch >= 2 * pool_size() && !g_in_shard) {
-    return run_sharded_fn(batch, 2, st, [&](int, int64_t first, int64_t count, cudaStream_t s) {
-      g_in_shard = true;
-      const int rc = xwt_wct_entry<T>((const T *)y1 + first * n0, (const T *)y2 + first * n0, count, n0, N, dt, dj, ax,
-                                      f0, flags, wct_out ? (T *)wct_out + first * plane : nullptr,
-                                      phase_out ? (T *)phase_out + first * plane : nullptr,
-                                      w12_out ? (cplx<T> *)w12_out + first * plane : nullptr, s);
-      g_in_shard = false;
-      return rc;
-    });
-  }
-  // stage inputs interleaved [pair, 2, n0] and outputs per chunk
+  const size_t plane = (size_t)S * n0, row = sizeof(T) * n0;
+  const InRows a{y1, row}, b{y2, row};
+  const OutRows wc{wct_out, sizeof(T) * plane}, ph{phase_out, sizeof(T) * plane}, xw{w12_out, sizeof(cplx<T>) * plane};
+  // pairs per chunk: their staged rows and their intermediates within 1 GiB, with host and device pointers alike
   const size_t per_pair = sizeof(T) * (2 * (size_t)n0 + (wct_out ? plane : 0) + (phase_out ? plane : 0) +
                                        (w12_out ? 2 * plane : 0));
-  const size_t budget = size_t(1) << 30;
-  const int64_t rows = std::max<int64_t>(
-      1, std::min<int64_t>(batch, (int64_t)(budget / (per_pair + pair_bytes<T>(n0, N, S)))));
-  auto al = [](size_t b) { return (b + 255) / 256 * 256; };
-  void *stage = nullptr;
-  WTB_TRY(staging_reserve(al(sizeof(T) * rows * 2 * n0) + al(sizeof(T) * rows * plane) * 4 + 1024, &stage));
-  char *p = (char *)stage;
-  T *d_y = (T *)p; p += al(sizeof(T) * rows * 2 * n0);
-  T *d_wct = nullptr, *d_phase = nullptr;
-  cplx<T> *d_w12 = nullptr;
-  const bool dev = flags & WTB_DEVICE_PTRS;
-  if (wct_out) { d_wct = (T *)p; p += al(sizeof(T) * rows * plane); }
-  if (phase_out) { d_phase = (T *)p; p += al(sizeof(T) * rows * plane); }
-  if (w12_out) { d_w12 = (cplx<T> *)p; }
-  const cudaMemcpyKind in_kind = dev ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice;
-  for (int64_t b0 = 0; b0 < batch; b0 += rows) {
-    const int64_t nb = std::min(rows, batch - b0);
-    // interleave y1/y2 rows: dst pitch 2*n0, src pitch n0
-    WTB_CUDA(cudaMemcpy2DAsync(d_y, sizeof(T) * 2 * n0, (const T *)y1 + b0 * n0, sizeof(T) * n0,
-                               sizeof(T) * n0, nb, in_kind, st));
-    WTB_CUDA(cudaMemcpy2DAsync(d_y + n0, sizeof(T) * 2 * n0, (const T *)y2 + b0 * n0, sizeof(T) * n0,
-                               sizeof(T) * n0, nb, in_kind, st));
-    T *o_wct = dev && wct_out ? (T *)wct_out + b0 * plane : d_wct;
-    T *o_phase = dev && phase_out ? (T *)phase_out + b0 * plane : d_phase;
-    cplx<T> *o_w12 = dev && w12_out ? (cplx<T> *)w12_out + b0 * plane : d_w12;
-    WTB_TRY(wct_device<T>(d_y, nb, n0, N, dt, dj, ax, f0, flags & WTB_GENERIC_ONLY, o_wct, o_phase, o_w12, nullptr,
-                          nullptr, nullptr, 0, st));
-    if (!dev) {
-      if (wct_out)
-        WTB_TRY(copy_to_host((T *)wct_out + b0 * plane, d_wct, sizeof(T) * nb * plane, st));
-      if (phase_out)
-        WTB_TRY(copy_to_host((T *)phase_out + b0 * plane, d_phase, sizeof(T) * nb * plane, st));
-      if (w12_out)
-        WTB_TRY(copy_to_host((cplx<T> *)w12_out + b0 * plane, d_w12, sizeof(cplx<T>) * nb * plane, st));
-      WTB_CUDA(cudaStreamSynchronize(st));
-    }  // device buffers: chunks reuse the arena without a host sync (all work is ordered on `st`)
-  }
-  return WTB_OK;
+  return shard_host_rows(batch, flags, st, [&](int64_t first, int64_t count, cudaStream_t s) {
+    const int64_t rows = std::max<int64_t>(
+        1, std::min<int64_t>(count, (int64_t)((size_t(1) << 30) / (per_pair + pair_bytes<T>(n0, N, S)))));
+    return stage_rows(count, rows, flags, s, {a.at(first), b.at(first)}, {wc.at(first), ph.at(first), xw.at(first)},
+                      2 * row * rows, [&](const void *const *in, void *const *out, void *extra, int64_t, int64_t nb) {
+                        // interleave the pairs' rows as [pair, 2, n0]: dst pitch 2 n0, src pitch n0
+                        T *d_y = (T *)extra;
+                        WTB_CUDA(cudaMemcpy2DAsync(d_y, 2 * row, in[0], row, row, nb, cudaMemcpyDeviceToDevice, s));
+                        WTB_CUDA(cudaMemcpy2DAsync(d_y + n0, 2 * row, in[1], row, row, nb, cudaMemcpyDeviceToDevice, s));
+                        return wct_device<T>(d_y, nb, n0, N, dt, dj, ax, f0, flags & WTB_GENERIC_ONLY, (T *)out[0],
+                                             (T *)out[1], (cplx<T> *)out[2], nullptr, nullptr, nullptr, 0, s);
+                      });
+  });
 }
 
 // implemented in noise.cu
@@ -405,7 +367,6 @@ static int mc_hist_entry(double a1, double a2, double dt, double dj, const Axes 
   coi_ranges(nsurr, dt, ax, f0, &tlo, &thi, &any);
   WTB_TRACE_POINT(st, "mc: coi ranges");
   const bool dev = flags & WTB_DEVICE_PTRS;
-  auto al = [](size_t b) { return (b + 255) / 256 * 256; };
   const size_t per_pair = sizeof(T) * 2 * (size_t)nsurr + pair_bytes<T>(nsurr, N, S);
   // Intermediates per chunk.  Launch tails are what chunking costs (1.5 GiB chunks: 253 k pairs/s,
   // one 18 GB chunk: 263 k at 2048 pairs), so the default spends a tenth of the 180 GB HBM3e;
@@ -425,8 +386,8 @@ static int mc_hist_entry(double a1, double a2, double dt, double dj, const Axes 
   const int64_t n_chunks = (mc_count + rows_max - 1) / rows_max;
   const int64_t rows = std::max<int64_t>(1, (mc_count + n_chunks - 1) / std::max<int64_t>(1, n_chunks));
   void *stage = nullptr;
-  const size_t b_hist = al(sizeof(uint64_t) * S * WTB_NBINS);
-  const size_t b_y = al(sizeof(T) * rows * 2 * nsurr);
+  const size_t b_hist = align256(sizeof(uint64_t) * S * WTB_NBINS);
+  const size_t b_y = align256(sizeof(T) * rows * 2 * nsurr);
   // Host-injected surrogates in several chunks: two staging buffers, the copy of chunk k + 1 runs
   // on a copy stream while the kernels of chunk k run (2.7 GB of H2D for 100 000 realisations is
   // 49 ms next to 290 ms of kernels when they are serial).

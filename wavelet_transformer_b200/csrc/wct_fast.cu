@@ -794,7 +794,7 @@ int wct_fast(const float2 *d_xhat, int64_t pairs, int n0, double dt, const Axes 
       dn[d + kDirDn] = make_float2((float)re, (float)im);
     }
     void *prm = nullptr;
-    const size_t b_dn = (sizeof(float2) * dn.size() + 255) / 256 * 256;
+    const size_t b_dn = align256(sizeof(float2) * dn.size());
     WTB_TRY(params_reserve(b_dn + sizeof(DRow) * kMaxRowsC, &prm));
     float2 *d_dn = (float2 *)prm;
     DRow *d_drows = (DRow *)((char *)prm + b_dn);

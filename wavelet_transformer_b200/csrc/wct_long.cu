@@ -220,10 +220,9 @@ int wct_long(const T *d_y, int64_t pairs, int n0, int N, double dt, const Axes &
   const int64_t wave_fwd = long_wave_rows(N, sizeof(cplx<T>), 2 * pairs);
   const int64_t wave = wct_long_wave_rows(N, sizeof(cplx<T>), smooth, rows);
   // one reservation: scales, COI ranges, X^, tsm (n0 per row, not N) and the wave buffers A, B
-  auto al = [](size_t b) { return (b + 255) / 256 * 256; };
-  const size_t b_sc = al(sizeof(double) * S), b_rng = al(sizeof(int) * S);
-  const size_t b_xh = al(sizeof(cplx<T>) * (size_t)pairs * 2 * N);
-  const size_t b_ts = smooth ? al(sizeof(vec4<T>) * (size_t)rows * n0) : 0;
+  const size_t b_sc = align256(sizeof(double) * S), b_rng = align256(sizeof(int) * S);
+  const size_t b_xh = align256(sizeof(cplx<T>) * (size_t)pairs * 2 * N);
+  const size_t b_ts = smooth ? align256(sizeof(vec4<T>) * (size_t)rows * n0) : 0;
   const size_t half = (size_t)wave * 2 * N;   // complex values of one wave buffer
   const size_t b_wave = sizeof(cplx<T>) * std::max((size_t)wave_fwd * N, (smooth ? 2 : 1) * half);
   void *scratch = nullptr;
