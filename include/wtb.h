@@ -168,6 +168,21 @@ int wtb_xwt_wct(const void *y1, const void *y2, int64_t batch, int n0, int nfft,
                 double dt, double dj, double s0, int J, double f0, int flags,
                 void *wct_out, void *phase_out, void *w12_out, void *stream);
 
+/* ---- partial and multiple wavelet coherence of three series (Aguiar-Conraria & Soares 2014;
+ * Ng & Chan 2012), built from pycwt's Morlet CWT and Morlet.smooth as pycwt.wct builds its spectra -- */
+/* y, x1, x2: [batch, n0] real (already normalised by the caller).  With the smoothed spectra
+ * S_ij = smooth(W_i conj(W_j) / s) of the three CWTs, outputs (any may be NULL, not all):
+ * pwc_out [batch,S,n0] real = |S_y1 S_22 - S_y2 conj(S_12)|^2 / ((S_yy S_22 - |S_y2|^2)(S_11 S_22 - |S_12|^2)),
+ * the partial coherence of y and x1 given x2; pphase_out [batch,S,n0] real = angle(S_y1 S_22 - S_y2 conj(S_12));
+ * mwc_out [batch,S,n0] real = (|S_y1|^2 S_22 + |S_y2|^2 S_11 - 2 Re(S_y1 conj(S_y2) S_12)) / (S_yy (S_11 S_22 -
+ * |S_12|^2)), the multiple coherence of y on x1 and x2.  The ratios are formed in double in both precisions and
+ * not clamped (0/0 gives NaN).  Morlet(f0) only; scales as wtb_cwt_axes.  nfft: one CTA per transform, a power
+ * of two up to 8192 in FP32 / 4096 in FP64, any other length up to 4096 / 2048; longer ones return
+ * WTB_EUNSUPPORTED before any work.  batch == 0 is a no-op. */
+int wtb_partial_wct(const void *y, const void *x1, const void *x2, int64_t batch, int n0, int nfft,
+                    double dt, double dj, double s0, int J, double f0, int flags,
+                    void *pwc_out, void *pphase_out, void *mwc_out, void *stream);
+
 /* ---- Monte Carlo coherence significance: replaces pycwt.wct_significance -- */
 /* Surrogate length N = ceil(6*s0*2^(J*dj)/dt) and the largest scale index
  * with any point inside the reliable region (pycwt's `maxscale`). */

@@ -99,6 +99,8 @@ _SIGNATURES = {
     "wtb_ratio_planes": ([_vp, _i64, _i32, _i32, _vp, _i64, _i32, _vp, _vp, _vp], _i32),
     "wtb_phase_arrows": ([_vp, _i64, _i32, _vp, _vp, _vp], _i32),
     "wtb_xwt_wct": ([_vp, _vp, _i64, _i32, _i32, _f64, _f64, _f64, _i32, _f64, _i32, _vp, _vp, _vp, _vp], _i32),
+    "wtb_partial_wct": ([_vp, _vp, _vp, _i64, _i32, _i32, _f64, _f64, _f64, _i32, _f64, _i32, _vp, _vp, _vp, _vp],
+                        _i32),
     "wtb_wct_mc_geometry": ([_f64, _f64, _f64, _i32, _f64, _pi, _pi], _i32),
     "wtb_wct_mc_hist": ([_f64, _f64, _f64, _f64, _f64, _i32, _f64, _i64, _i64, _u64, _vp, _i32, _vp, _vp], _i32),
     "wtb_wct_sig_from_hist": ([_vp, _i32, _i32, _f64, _vp, _pd], _i32),
@@ -478,6 +480,29 @@ def xwt_wct(y1, y2, dt, dj, s0, J, f0=6.0, *, nfft=None, f64=None, want_wct=True
     if np.ndim(y1) == 1:
         wct, phase, w12 = (None if v is None else v[0] for v in (wct, phase, w12))
     return wct, phase, w12
+
+
+def partial_wct(y, x1, x2, dt, dj, s0, J, f0=6.0, *, nfft=None, f64=None, want_pwc=True, want_phase=True,
+                want_mwc=True, generic_only=False):
+    """Batched partial and multiple wavelet coherence of already-normalised host series (wtb_partial_wct):
+    the partial coherence of y and x1 given x2, its phase, and the multiple coherence of y on x1 and x2.
+    Returns (pwc, phase, mwc), each [batch, S, n0] or None (batch axis dropped for 1-D input)."""
+    f64 = _resolve_f64(f64)
+    rt = _dtype(f64)
+    a, b, c = (np.ascontiguousarray(np.atleast_2d(np.asarray(v)), dtype=rt) for v in (y, x1, x2))
+    if not a.shape == b.shape == c.shape:
+        raise ValueError("y, x1 and x2 must have the same shape")
+    batch, n0 = a.shape
+    Jr, _, _, _ = cwt_axes(n0, dt, dj, s0, J, f0)
+    S = Jr + 1
+    nfft = int(nfft) if nfft else default_nfft(n0)
+    pwc, phase, mwc = (np.empty((batch, S, n0), dtype=rt) if w else None for w in (want_pwc, want_phase, want_mwc))
+    flags = (F64 if f64 else 0) | (GENERIC_ONLY if generic_only else 0)
+    _check(lib().wtb_partial_wct(_ptr(a), _ptr(b), _ptr(c), batch, n0, nfft, dt, dj, s0, int(J), f0, flags,
+                                 _ptr(pwc), _ptr(phase), _ptr(mwc), None), "wtb_partial_wct")
+    if np.ndim(y) == 1:
+        pwc, phase, mwc = (None if v is None else v[0] for v in (pwc, phase, mwc))
+    return pwc, phase, mwc
 
 
 # ---------------------------------------------------------------- Monte Carlo significance

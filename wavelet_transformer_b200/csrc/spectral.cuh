@@ -25,6 +25,16 @@ __device__ __forceinline__ T morlet_daughter(int k, int N, T s_over_dt, T norm, 
   return norm * dev_exp<T>(T(-0.5) * z * z);
 }
 
+// Time smoothing of Morlet.smooth at bin k of an N-point grid, with the 1/N of the inverse transform folded in:
+// exp(-0.5 (s/dt)^2 w_k^2) / N, w_k = 2*pi*fftfreq(N)[k].  Real and even in k, so it filters the real and the
+// imaginary part of a packed row independently.
+template <typename T>
+__device__ __forceinline__ T smooth_gauss(int k, int N, T s_over_dt, T invN) {
+  const int kk = (k < (N + 1) / 2) ? k : k - N;
+  const T w = T(2.0 * kPi) * T(kk) / T(N) * s_over_dt;
+  return dev_exp<T>(T(-0.5) * w * w) * invN;
+}
+
 // X^[k] times the conjugated daughter of one scale at bin k of an N-point grid (k_cwt_rows, and the first pass
 // of the long transforms in cwt_long.cu).  Morlet: norm = (2 pi s / dt)^0.5 pi^-1/4 / N.  Paul: (sw)^m exp(-sw)
 // H(sw); DOG: (sw)^m exp(-(sw)^2/2); both times nrm = (2 pi s / dt)^0.5 / N and conj(prefactor) = pre.

@@ -75,9 +75,7 @@ __global__ void k_wct_rows(const cplx<T> *__restrict__ xhat, int n0, FftPlan<T> 
   // Gaussian in the Fourier domain: exp(-0.5 (s/dt)^2 k^2), k = 2*pi*fftfreq(N)
   const T invN = T(1.0 / N);
   for (int k = threadIdx.x; k < N; k += blockDim.x) {
-    const int kk = (k < (N + 1) / 2) ? k : k - N;
-    const T w = T(2.0 * kPi) * T(kk) / T(N) * s_over_dt;
-    const T g = dev_exp<T>(T(-0.5) * w * w) * invN;
+    const T g = smooth_gauss<T>(k, N, s_over_dt, invN);
     cplx<T> p = U[k], c = V[k];
     U[k] = mk<T>(p.x * g, p.y * g);
     V[k] = mk<T>(c.x * g, c.y * g);
@@ -129,21 +127,6 @@ __global__ void k_wct_scale(const vec4<T> *__restrict__ tsm, int64_t pairs, int 
       }
     }
   }
-}
-
-static int make_win(double dj, ScaleWin *win) {
-  // Morlet.smooth: rect(int(round(deltaj0/dj*2)), normalize=True), deltaj0 = 0.6
-  const int K = (int)std::nearbyint(0.6 / dj * 2);
-  WTB_REQUIRE(K >= 1 && K <= kMaxWin, WTB_EUNSUPPORTED, "scale window of %d taps (dj=%g) unsupported", K, dj);
-  win->K = K;
-  win->up = (K - 1) / 2;
-  double sum = 0;
-  for (int k = 0; k < K; ++k) {
-    win->w[k] = (k == 0 || k == K - 1) ? 0.5 : 1.0;
-    sum += win->w[k];
-  }
-  for (int k = 0; k < K; ++k) win->w[k] /= sum;
-  return WTB_OK;
 }
 
 // Scale boxcar and coherence of tsm [pairs, S, n0]: the plane, or the histogram when d_hist.

@@ -19,4 +19,19 @@ struct ScaleWin {
   double w[kMaxWin];
 };
 
+// Morlet.smooth: rect(int(round(deltaj0/dj*2)), normalize=True), deltaj0 = 0.6
+inline int make_win(double dj, ScaleWin *win) {
+  const int K = (int)std::nearbyint(0.6 / dj * 2);
+  WTB_REQUIRE(K >= 1 && K <= kMaxWin, WTB_EUNSUPPORTED, "scale window of %d taps (dj=%g) unsupported", K, dj);
+  win->K = K;
+  win->up = (K - 1) / 2;
+  double sum = 0;
+  for (int k = 0; k < K; ++k) {
+    win->w[k] = (k == 0 || k == K - 1) ? 0.5 : 1.0;
+    sum += win->w[k];
+  }
+  for (int k = 0; k < K; ++k) win->w[k] /= sum;
+  return WTB_OK;
+}
+
 }  // namespace wtb

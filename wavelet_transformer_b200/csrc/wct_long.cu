@@ -157,14 +157,12 @@ __global__ void k_wcl_g(LongPlan<T> p, int64_t row0, int S, const double *__rest
   }
   __syncthreads();
   long_columns<T, -1, C>(tile, stride, scratch, N1, p.log2N1, p.tw1);
-  // Gaussian in the Fourier domain: exp(-0.5 (s/dt)^2 k^2), k = 2*pi*fftfreq(N), with k_wct_rows' expression
+  // Gaussian in the Fourier domain: exp(-0.5 (s/dt)^2 k^2), k = 2*pi*fftfreq(N), as k_wct_rows applies it
   const T s_over_dt = T(scales[row % S] / dt);
   const T invN = T(1.0 / N);
   for (int i = tid; i < C * N1; i += nthr) {
     const int c = i % C, k1 = i / C, k = c0 + c + N2 * k1;
-    const int kk = (k < (N + 1) / 2) ? k : k - N;
-    const T w = T(2.0 * kPi) * T(kk) / T(N) * s_over_dt;
-    const T g = dev_exp<T>(T(-0.5) * w * w) * invN;
+    const T g = smooth_gauss<T>(k, N, s_over_dt, invN);
     const cplx<T> v = tile[c * stride + k1];
     tile[c * stride + k1] = mk<T>(v.x * g, v.y * g);
   }
