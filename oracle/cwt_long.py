@@ -40,7 +40,8 @@ def _elem(f64):
 
 
 def long_takes(nfft, f64):
-    """cwt_long_takes: a power of two whose two shared-memory buffers (2 nfft complex) exceed 227 KB."""
+    """Route::kLong of route_of (cwt_paths.cuh): a power of two whose two shared-memory buffers (2 nfft complex)
+    exceed 227 KB, i.e. past 8192 in FP32 and 4096 in FP64."""
     return nfft > 0 and nfft & (nfft - 1) == 0 and 2 * 2 * _elem(f64) * nfft > SMEM_LIMIT
 
 

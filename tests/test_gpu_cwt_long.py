@@ -164,6 +164,12 @@ def test_refusals(shim, f64):
         assert lib.wtb_cwt(p(x), 1, 5000, 5000, DT, 1.0, 2.0, 8, 0, 6.0, flags, p(out), None, None) == EUNSUPPORTED
         assert lib.wtb_last_error() == (b"nfft=5000 needs 262144 B of shared memory per CTA (limit 227 KB): a power of "
                                         b"two up to 8192, any other length up to 4096 for float")
+    # an empty batch returns before the length is looked at, for wtb_cwt and wtb_cwt_averages alike
+    glob = np.zeros((1, 9), rt)
+    for nfft in (5000, 1 << 23, 1_500_000_001):
+        assert lib.wtb_cwt(p(x), 0, 5000, nfft, DT, 1.0, 2.0, 8, 0, 6.0, flags, p(out), None, None) == 0, nfft
+        assert lib.wtb_cwt_averages(p(x), 0, 5000, nfft, DT, 1.0, 2.0, 8, 0, 6.0, 0, 0, 1.0, flags, p(glob), None,
+                                    None) == 0, nfft
     assert shim.kernel_launches() == before
 
 

@@ -319,17 +319,20 @@ def _refusal(nfft, f64, buffers):
 @pytest.mark.parametrize("f64", [False, True], ids=["fp32", "fp64"])
 def test_unpadded_limit_is_refused(shim, f64):
     """The longest un-padded length is served (test_cwt_length_classes, test_xwt_wct_rows); the next one is
-    refused by wtb_cwt, wtb_cwt_averages and wtb_xwt_wct with WTB_EUNSUPPORTED, before any launch."""
+    refused by wtb_cwt, wtb_cwt_averages and wtb_xwt_wct with WTB_EUNSUPPORTED, before any launch.  So are lengths
+    whose Bluestein work length (2^31, 2^32) does not fit an int, for a series of 100 samples."""
     n0 = 2049 if f64 else 4097
-    x = _inputs("white", 2, n0, seed=1)
     before = shim.kernel_launches()
-    for call, buffers in ((lambda: shim.cwt(x, DT, DJ, -1, -1, 2, 2.0, nfft=n0, f64=f64), 2),
-                          (lambda: shim.cwt_averages(x, DT, DJ, -1, -1, 0, 6.0, nfft=n0, f64=f64), 2),
-                          (lambda: shim.xwt_wct(x, x[::-1], DT, DJ, -1, -1, nfft=n0, f64=f64), 3)):
-        with pytest.raises(shim.WaveletEngineError) as err:
-            call()
-        assert f"(status {EUNSUPPORTED}): {_refusal(n0, f64, buffers)}" in str(err.value)
+    for n, nfft in ((n0, n0), (100, 600_000_001), (100, 1_500_000_001)):
+        x = _inputs("white", 2, n, seed=1)
+        for call, buffers in ((lambda: shim.cwt(x, DT, DJ, -1, -1, 2, 2.0, nfft=nfft, f64=f64), 2),
+                              (lambda: shim.cwt_averages(x, DT, DJ, -1, -1, 0, 6.0, nfft=nfft, f64=f64), 2),
+                              (lambda: shim.xwt_wct(x, x[::-1], DT, DJ, -1, -1, nfft=nfft, f64=f64), 3)):
+            with pytest.raises(shim.WaveletEngineError) as err:
+                call()
+            assert f"(status {EUNSUPPORTED}): {_refusal(nfft, f64, buffers)}" in str(err.value)
     assert shim.kernel_launches() == before
+    x = _inputs("white", 2, n0, seed=1)
     shim.cwt(x[:, :-2], DT, DJ, -1, -1, 2, 2.0, nfft=n0 - 2, f64=f64)        # and the longest accepted length
 
 

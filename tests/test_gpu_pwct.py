@@ -146,6 +146,12 @@ def test_refusals(shim, f64):
         assert f"nfft={nfft}" in msg and limit in msg, msg
     assert call(565, 1024, 0.01, p(out)) == EUNSUPPORTED          # 120 boxcar taps
     assert b"scale window" in lib.wtb_last_error()
+    # the length is checked before the scale window and before an empty batch returns
+    assert call(other + 1, other + 1, 0.01, p(out)) == EUNSUPPORTED
+    assert limit in lib.wtb_last_error().decode()
+    assert lib.wtb_partial_wct(p(x), p(x), p(x), 0, 565, 1_500_000_001, DT, 0.5, 2.0, 8, 6.0, flags, p(out), None,
+                               None, None) == EUNSUPPORTED
+    assert limit in lib.wtb_last_error().decode()
     assert lib.wtb_partial_wct(p(x), p(x), p(x), 0, 565, 1024, DT, 0.5, 2.0, 8, 6.0, flags, p(out), None, None,
                                None) == 0
     assert shim.kernel_launches() == before and not out.any()

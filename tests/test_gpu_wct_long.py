@@ -169,9 +169,21 @@ def test_refusals(shim, f64):
     assert lib.wtb_xwt_wct(p(x), p(x), 1, 5000, 5000, DT, 1.0, 2.0, 8, 6.0, flags, p(out), None, None,
                            None) == EUNSUPPORTED
     B = 3 * (16 if f64 else 8) * 16384
-    assert lib.wtb_last_error() == (f"nfft=5000 needs {B} B of shared memory per CTA (limit 227 KB): a power of two "
-                                    f"up to {4096 if f64 else 8192}, any other length up to {2048 if f64 else 4096} "
-                                    f"for {'double' if f64 else 'float'}").encode()
+    refusal = (f"nfft=5000 needs {B} B of shared memory per CTA (limit 227 KB): a power of two up to "
+               f"{4096 if f64 else 8192}, any other length up to {2048 if f64 else 4096} for "
+               f"{'double' if f64 else 'float'}").encode()
+    assert lib.wtb_last_error() == refusal
+    # with a scale window of 1200 taps as well: the one-CTA refusal comes first, the 2^22 one after the window
+    assert lib.wtb_xwt_wct(p(x), p(x), 1, 5000, 5000, DT, 0.001, 2.0, 8, 6.0, flags, p(out), None, None,
+                           None) == EUNSUPPORTED
+    assert lib.wtb_last_error() == refusal
+    assert lib.wtb_xwt_wct(p(x), p(x), 1, 5000, 1 << 23, DT, 0.001, 2.0, 8, 6.0, flags, p(out), None, None,
+                           None) == EUNSUPPORTED
+    assert b"scale window of 1200 taps" in lib.wtb_last_error()
+    # an empty batch returns before the length is looked at
+    for nfft in (5000, 1 << 23, 1_500_000_001):
+        assert lib.wtb_xwt_wct(p(x), p(x), 0, 5000, nfft, DT, 1.0, 2.0, 8, 6.0, flags, p(out), None, None,
+                               None) == 0, nfft
     assert shim.kernel_launches() == before
 
 

@@ -59,7 +59,7 @@ static unsigned averages_parts(int64_t nb, int S, int n0) {
 // budget alone counts, and a series whose plane exceeds it is a chunk of its own.
 static int64_t averages_chunk_rows(int64_t batch, int S, int n0, int N, size_t elem) {
   const int64_t by_bytes = (int64_t)((size_t(1) << 30) / (elem * (size_t)S * n0));
-  if (cwt_long_takes(N, elem)) return std::min(batch, std::max<int64_t>(1, by_bytes));
+  if (route_of(N, elem) == Route::kLong) return std::min(batch, std::max<int64_t>(1, by_bytes));
   const int64_t fill = 16LL * sm_count();
   return std::min(batch, std::max(fill, by_bytes) & ~int64_t(1));
 }

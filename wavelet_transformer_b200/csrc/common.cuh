@@ -86,6 +86,7 @@ template <typename C> __device__ __forceinline__ C cmulc(C a, C b) {
 }
 
 constexpr double kPi = 3.14159265358979323846264338327950288;
+constexpr size_t kSmemLimit = 227 << 10;   // shared memory of one CTA on sm_100 (B200), static and dynamic
 
 // ---- per-call context, device scratch, tables (host side) -----------------------
 // Every C-ABI entry point opens a CallScope first.  It decides which device the call runs on
@@ -250,8 +251,10 @@ int stage_rows(int64_t batch, int64_t rows, int flags, cudaStream_t st, std::ini
   return WTB_OK;
 }
 
-inline int ilog2(int n) { int l = 0; while ((1 << l) < n) ++l; return l; }
+inline int ilog2(int n) { int l = 0; while ((int64_t(1) << l) < n) ++l; return l; }   // ceil(log2 n), any int n
 inline bool is_pow2(int n) { return n > 0 && (n & (n - 1)) == 0; }
+// make_plan's work length, any int nfft: a power of two itself, else Bluestein's 2^m >= 2 nfft - 1 (2 << ilog2)
+inline int64_t work_length(int nfft) { return is_pow2(nfft) ? nfft : int64_t(2) << ilog2(nfft); }
 
 // Morlet constants (pycwt.mothers.Morlet)
 inline double morlet_flambda(double f0) { return 4.0 * kPi / (f0 + std::sqrt(2.0 + f0 * f0)); }

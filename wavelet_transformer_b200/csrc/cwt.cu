@@ -68,7 +68,7 @@ CwtPlan cwt_plan(int64_t batch, int n0, int N, int S, double f0, int mother, siz
   if (fast && power_only && (N == 1024 || N == 512) && f0 >= kZCut && S <= kMaxRows &&
       batch >= min_fast_batch(N == 512 ? 20 : 1))
     return {Fwd::kInKernel, N == 512 ? Rows::kFast512Pairs : Rows::kFast1024};
-  if (cwt_long_takes(N, elem)) return {Fwd::kInKernel, Rows::kLong};
+  if (route_of(N, elem) == Route::kLong) return {Fwd::kInKernel, Rows::kLong};
   if (!fast) return {Fwd::kGeneric, Rows::kGeneric};
   // k_cwt_dif stores the first half of a row unconditionally (n0 > nfft / 2).  The rows of a series are split over
   // CTAs when the batch is small, but this path also pays for the separate forward-FFT launch: 0.040 ms for 12
@@ -92,6 +92,7 @@ CwtPlan cwt_plan(int64_t batch, int n0, int N, int S, double f0, int mother, siz
 template <typename T>
 int cwt_device(const T *d_x, int64_t batch, int n0, int N, double dt, const Axes &ax,
                const Mother &mo, int flags, T *d_power, cplx<T> *d_coef, cudaStream_t st) {
+  if (route_of(N, sizeof(T)) == Route::kRefused) return refuse_length(N, sizeof(T), 2);
   const int S = ax.J + 1;
   const double f0 = mo.kind == WTB_MORLET ? mo.param : 0.0;
   const CwtPlan pl = cwt_plan(batch, n0, N, S, f0, mo.kind, sizeof(T), flags, d_power != nullptr, d_coef != nullptr);
@@ -108,17 +109,13 @@ int cwt_device(const T *d_x, int64_t batch, int n0, int N, double dt, const Axes
   FftPlan<T> plan;
   WTB_TRY(make_plan<T>(N, &plan));
   const size_t smem = 2 * sizeof(cplx<T>) * (size_t)plan.M;
-  WTB_REQUIRE(smem <= 227 * 1024, WTB_EUNSUPPORTED,
-              "nfft=%d needs %zu B of shared memory per CTA (limit 227 KB): a power of two up to %d, any other "
-              "length up to %d for %s", N, smem, sizeof(T) == 4 ? 8192 : 4096, sizeof(T) == 4 ? 4096 : 2048,
-              sizeof(T) == 4 ? "float" : "double");
   void *scratch = nullptr;
   const size_t sc_bytes = align256(sizeof(double) * S);
   WTB_TRY(arena_reserve(sc_bytes + sizeof(cplx<T>) * (size_t)batch * N, &scratch));
   double *d_scales = (double *)scratch;
   cplx<T> *d_xhat = (cplx<T> *)((char *)scratch + sc_bytes);
   WTB_CUDA(cudaMemcpyAsync(d_scales, ax.scales.data(), sizeof(double) * S, cudaMemcpyHostToDevice, st));
-  const int threads = plan.M >= 1024 ? 256 : (plan.M >= 256 ? 128 : 64);
+  const int threads = plan_threads(plan.M);
   WTB_CUDA(cudaFuncSetAttribute(k_fwd_fft<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   WTB_CUDA(cudaFuncSetAttribute(k_cwt_rows<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   if (pl.rows == Rows::kDif2048 || pl.rows == Rows::kDif4096)   // with its own forward transforms (group layout)
@@ -192,15 +189,15 @@ extern "C" int wtb_cwt(const void *x, int64_t batch, int n0, int nfft, double dt
   return cwt_entry<float>(x, batch, n0, nfft, dt, ax, mo, flags, power_out, coef_out, st);
 }
 
-// The Morlet entry point keeps the transform lengths it has always served: one CTA per transform (powers of two
-// up to 8192 in FP32, 4096 in FP64).  Longer series go through wtb_cwt, which takes them up to 2^22.
+// The Morlet entry point keeps the lengths it has always served, one CTA per transform; wtb_cwt takes longer ones.
 extern "C" int wtb_cwt_morlet(const void *x, int64_t batch, int n0, int nfft, double dt, double dj,
                               double s0, int J, double f0, int flags, void *power_out,
                               void *coef_out, void *stream) {
-  const bool f64 = flags & WTB_F64;
-  WTB_REQUIRE(!cwt_long_takes(nfft, f64 ? sizeof(double) : sizeof(float)), WTB_EUNSUPPORTED,
+  const size_t elem = (flags & WTB_F64) ? sizeof(double) : sizeof(float);
+  WTB_REQUIRE(route_of(nfft, elem) != Route::kLong, WTB_EUNSUPPORTED,
               "wtb_cwt_morlet: nfft=%d is past the one-CTA transform (a power of two up to %d for %s); wtb_cwt with "
-              "WTB_MORLET takes powers of two up to 2^22", nfft, f64 ? 4096 : 8192, f64 ? "double" : "float");
+              "WTB_MORLET takes powers of two up to 2^22", nfft, cta_max_work(elem),
+              elem == sizeof(float) ? "float" : "double");
   return wtb_cwt(x, batch, n0, nfft, dt, dj, s0, J, WTB_MORLET, f0, flags, power_out, coef_out, stream);
 }
 

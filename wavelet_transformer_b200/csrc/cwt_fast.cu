@@ -390,7 +390,7 @@ template <int D> struct CtaSmemP {
                                     // reading the last draw of one series when the leader draws for the next)
   WarpSmemP w[kDifWarps];
 };
-static_assert(sizeof(CtaSmemP<2>) <= 227 * 1024 && sizeof(CtaSmemP<4>) <= 227 * 1024,
+static_assert(sizeof(CtaSmemP<2>) <= kSmemLimit && sizeof(CtaSmemP<4>) <= kSmemLimit,
               "the tables, ring and per-warp buffers of the decimation-in-frequency kernels must fit one CTA");
 
 template <int D> __device__ __forceinline__ void group_sync(int group) {

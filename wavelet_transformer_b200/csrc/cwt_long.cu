@@ -1,5 +1,4 @@
-// CWT of long series: power-of-two transforms whose two shared-memory buffers do not fit one CTA
-// (nfft >= 16384 in FP32, >= 8192 in FP64), up to nfft = 2^22.  cwt_device (cwt.cu) branches here.
+// CWT of long series: the powers of two past one CTA (Route::kLong), up to 2^22; cwt_device (cwt.cu) branches here.
 //
 // The four-step transforms and their launch shapes are in long_fft.cuh.
 //
@@ -11,10 +10,6 @@
 #include "long_fft.cuh"
 
 namespace wtb {
-
-// The long path takes exactly the power-of-two lengths whose two shared-memory buffers exceed 227 KB
-// (nfft > 2^22 included: cwt_long refuses them).
-bool cwt_long_takes(int N, size_t elem) { return is_pow2(N) && 2 * 2 * elem * (size_t)N > 227 * 1024; }
 
 // exp(-2 pi i j / N) for j < 2048, then exp(-2 pi i 2048 j / N) for j < N / 2048; cached per (device, N), kept
 // until wtb_shutdown (at most 48 KB in FP64 at N = 2^22).

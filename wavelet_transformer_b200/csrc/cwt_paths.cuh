@@ -1,10 +1,34 @@
-// Which kernels serve a CWT (cwt_plan, cwt.cu), and the host functions the CWT and coherence translation units
-// call across files.
+// The length rule of the CWT and coherence transforms (route_of), which kernels serve a CWT (cwt_plan, cwt.cu), and
+// the host functions the CWT and coherence translation units call across files.
 #pragma once
 
 #include "wct_common.cuh"
 
 namespace wtb {
+
+// The length rule.  One-CTA kernels hold M-point complex buffers in shared memory, M = work_length(nfft): two in
+// k_fwd_fft, k_cwt_rows and k_pwct_smooth, three in k_wct_rows.  cta_max_work: the largest M at which two fit.
+constexpr int cta_max_work(size_t elem, int m = 1) {
+  return 2 * 2 * elem * (size_t)(2 * m) > kSmemLimit ? m : cta_max_work(elem, 2 * m);
+}
+static_assert(3 * 2 * sizeof(float) * cta_max_work(sizeof(float)) <= kSmemLimit &&
+                  3 * 2 * sizeof(double) * cta_max_work(sizeof(double)) <= kSmemLimit,
+              "k_wct_rows' three buffers fit one CTA at the largest one-CTA work length");
+// kOneCta: M <= cta_max_work (8192 in FP32, 4096 in FP64).  kLong: the powers of two above it (cwt_long.cu,
+// wct_long.cu; long_plan refuses those past 2^22).  kRefused: the rest.  nfft is compared, so nothing overflows.
+enum class Route { kOneCta, kLong, kRefused };
+inline Route route_of(int nfft, size_t elem) {
+  const int m = cta_max_work(elem);
+  if (is_pow2(nfft)) return nfft <= m ? Route::kOneCta : Route::kLong;
+  return nfft <= m / 2 ? Route::kOneCta : Route::kRefused;   // Bluestein: M = 2^k >= 2 nfft - 1
+}
+// Sets the message of a refused length for a kernel of `buffers` M-point buffers (2: k_cwt_rows, 3: k_wct_rows)
+inline int refuse_length(int nfft, size_t elem, int buffers) {
+  set_error("nfft=%d needs %zu B of shared memory per CTA (limit %zu KB): a power of two up to %d, any other length "
+            "up to %d for %s", nfft, buffers * 2 * elem * (size_t)work_length(nfft), kSmemLimit / 1024,
+            cta_max_work(elem), cta_max_work(elem) / 2, elem == sizeof(float) ? "float" : "double");
+  return WTB_EUNSUPPORTED;
+}
 
 // Limits of the FP32 Morlet kernels that the plan reads (each kernel's own transform size kN stays in its file).
 constexpr int kMaxRows = 256;    // scale rows k_cwt_fast_1024 stages in shared memory (cwt_fast.cu)
@@ -58,8 +82,7 @@ int wct_fast(const float2 *d_xhat, int64_t pairs, int n0, double dt, const Axes 
              float4 *d_spec, const ScaleWin &win, float *d_wct, float *d_phase, float2 *d_w12,
              unsigned long long *d_hist, const int *d_tlo, const int *d_thi, int maxscale, cudaStream_t st);
 
-// cwt_long.cu: four-step transforms for the powers of two past one CTA's shared memory (long_fft.cuh)
-bool cwt_long_takes(int N, size_t elem);
+// cwt_long.cu: four-step transforms for the lengths route_of sends to Route::kLong (long_fft.cuh)
 template <typename T> struct LongPlan;
 template <typename T> int long_plan(int N, cudaStream_t st, LongPlan<T> *p);
 template <typename T>
@@ -67,7 +90,7 @@ int cwt_long(const T *d_x, int64_t batch, int n0, int N, double dt, const Axes &
              T *d_power, cplx<T> *d_coef, cudaStream_t st);
 
 // wct_long.cu: the smoothed spectra tsm [pairs, S, n0] (when smooth), W12 and its phase of the interleaved
-// series d_y [pairs, 2, n0] at a length cwt_long_takes; scales, COI ranges (when h_tlo) and tsm live in its scratch.
+// series d_y [pairs, 2, n0] at a Route::kLong length; scales, COI ranges (when h_tlo) and tsm live in its scratch.
 template <typename T> struct WctLongOut {
   vec4<T> *tsm;
   int *tlo, *thi;

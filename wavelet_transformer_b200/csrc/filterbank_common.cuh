@@ -113,8 +113,6 @@ __device__ __forceinline__ int reflect_sym(int p, int n) {
 }
 
 // ---- host side -------------------------------------------------------------------------
-constexpr size_t kSmemLimit = 227 * 1024;
-
 template <typename K> static int set_smem(K kernel, size_t bytes) {
   WTB_REQUIRE(bytes <= kSmemLimit, WTB_EUNSUPPORTED,
               "series too long for the in-shared-memory filterbank (%zu B > 227 KB per CTA)", bytes);

@@ -164,7 +164,7 @@ template <typename T> inline LongLaunch long_launch(int pass, int L) {
   const int tx = std::min(L / 4, 128);
   int G = C;
   auto bytes = [&](int g) { return sizeof(cplx<T>) * ((size_t)C * (L + long_pad<T>(pass)) + (size_t)g * L); };
-  while (G > 1 && (bytes(G) > 227 * 1024 || tx * G > 512)) G /= 2;
+  while (G > 1 && (bytes(G) > kSmemLimit || tx * G > 512)) G /= 2;
   return {dim3(tx, G), bytes(G)};
 }
 

@@ -124,9 +124,6 @@ __global__ void k_pwct_scale(const T *__restrict__ sm, int64_t triples, int n0, 
   }
 }
 
-// Work length of a plan (make_plan): n itself for a power of two, else the Bluestein length 2^m >= 2 n - 1
-static int plan_work_len(int n) { return is_pow2(n) ? n : 1 << ilog2(2 * n - 1); }
-
 // bytes of staging one triple costs: interleaved series, coefficients, smoothed fields
 template <typename T> static size_t triple_bytes(int n0, int S) {
   return sizeof(T) * 3 * (size_t)n0 + sizeof(cplx<T>) * 3 * (size_t)S * n0 + sizeof(T) * kPwctFields * (size_t)S * n0;
@@ -149,7 +146,7 @@ static int pwct_device(const T *d_y, int64_t nb, int n0, int N, double dt, const
   WTB_TRY(arena_reserve(align256(sizeof(double) * S), &scratch));
   double *d_scales = (double *)scratch;
   WTB_CUDA(cudaMemcpyAsync(d_scales, ax.scales.data(), sizeof(double) * S, cudaMemcpyHostToDevice, st));
-  const int threads = plan.M >= 1024 ? 256 : (plan.M >= 256 ? 128 : 64);
+  const int threads = plan_threads(plan.M);
   WTB_CUDA(cudaFuncSetAttribute(k_pwct_smooth<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   k_pwct_smooth<T><<<(unsigned)(nb * S), threads, smem, st>>>(d_W, n0, plan, S, d_scales, dt, d_sm);
   WTB_LAUNCH_CHECK();
@@ -202,11 +199,10 @@ extern "C" int wtb_partial_wct(const void *y, const void *x1, const void *x2, in
   WTB_REQUIRE(pwc_out || pphase_out || mwc_out, WTB_EINVAL, "wtb_partial_wct: no output requested");
   WTB_REQUIRE(nfft >= n0 && nfft >= 2, WTB_EINVAL, "nfft=%d must be >= n0=%d", nfft, n0);
   const bool f64 = flags & WTB_F64;
-  // one CTA per transform, two work-length buffers of shared memory (as the generic CWT kernel)
-  const size_t smem = nfft <= 8192 ? 2 * (f64 ? sizeof(double2) : sizeof(float2)) * (size_t)plan_work_len(nfft) : 0;
-  WTB_REQUIRE(smem && smem <= 227 * 1024, WTB_EUNSUPPORTED,
+  const size_t elem = f64 ? sizeof(double) : sizeof(float);
+  WTB_REQUIRE(route_of(nfft, elem) == Route::kOneCta, WTB_EUNSUPPORTED,   // partial coherence has no long kernels
               "wtb_partial_wct: nfft=%d is past one CTA per transform: a power of two up to %d, any other length up "
-              "to %d for %s", nfft, f64 ? 4096 : 8192, f64 ? 2048 : 4096, f64 ? "double" : "float");
+              "to %d for %s", nfft, cta_max_work(elem), cta_max_work(elem) / 2, f64 ? "double" : "float");
   WTB_ENTER(flags, y, stream);
   Axes ax;
   WTB_TRY(resolve_axes(n0, dt, dj, s0, J, f0, &ax));

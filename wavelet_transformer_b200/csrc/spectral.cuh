@@ -74,11 +74,11 @@ __global__ void k_fwd_fft(const T *__restrict__ x, int n0, FftPlan<T> plan, cplx
   for (int k = threadIdx.x; k < N; k += blockDim.x) o[k] = r[k];
 }
 
-// Host side: the plan for transforms of length nfft on the current device (tables are cached).
+// Host side: the plan for a one-CTA length nfft (route_of) on the current device (tables are cached).
 template <typename T> static int make_plan(int nfft, FftPlan<T> *plan) {
   plan->n = nfft;
   const bool pow2 = is_pow2(nfft);
-  plan->M = pow2 ? nfft : (1 << ilog2(2 * nfft - 1));
+  plan->M = (int)work_length(nfft);
   plan->log2M = ilog2(plan->M);
   WTB_TRY(twiddles<T>(plan->M, &plan->tw));
   plan->chirp = nullptr;
@@ -86,5 +86,7 @@ template <typename T> static int make_plan(int nfft, FftPlan<T> *plan) {
   if (!pow2) WTB_TRY(bluestein_tables<T>(nfft, plan->M, &plan->chirp, &plan->chat));
   return WTB_OK;
 }
+// CTA size of the one-CTA kernels that run a plan (k_fwd_fft, k_cwt_rows, k_wct_rows, k_pwct_smooth)
+inline int plan_threads(int M) { return M >= 1024 ? 256 : (M >= 256 ? 128 : 64); }
 
 }  // namespace wtb

@@ -153,12 +153,13 @@ static int wct_device(const T *d_y, int64_t pairs, int n0, int N, double dt, dou
                       cudaStream_t st) {
   const int S = ax.J + 1;
   const bool smooth = d_wct || d_hist;
-  if (cwt_long_takes(N, sizeof(T))) {
-    // powers of two past one CTA's shared memory, up to 2^22: the four-step rows of wct_long.cu, then the same
-    // scale boxcar and coherence kernels (WTB_GENERIC_ONLY has no other kernels for these lengths)
-    ScaleWin win;
-    WTB_TRY(make_win(dj, &win));
-    WTB_REQUIRE(pairs * S < (1LL << 31) && pairs * 2 < (1LL << 31), WTB_EUNSUPPORTED, "batch too large");
+  const Route route = route_of(N, sizeof(T));
+  if (route == Route::kRefused) return refuse_length(N, sizeof(T), 3);
+  ScaleWin win;
+  WTB_TRY(make_win(dj, &win));
+  WTB_REQUIRE(pairs * S < (1LL << 31) && pairs * 2 < (1LL << 31), WTB_EUNSUPPORTED, "batch too large");
+  if (route == Route::kLong) {
+    // the four-step rows of wct_long.cu, then the same scale pass (WTB_GENERIC_ONLY has no other kernels here)
     WctLongOut<T> o;
     WTB_TRY(wct_long<T>(d_y, pairs, n0, N, dt, ax, f0, smooth, d_phase, d_w12, d_hist ? h_tlo : nullptr,
                         d_hist ? h_thi : nullptr, &o, st));
@@ -169,12 +170,6 @@ static int wct_device(const T *d_y, int64_t pairs, int n0, int N, double dt, dou
   WTB_TRY(make_plan<T>(N, &plan));
   const size_t smem_fwd = 2 * sizeof(cplx<T>) * (size_t)plan.M;
   const size_t smem_rows = 3 * sizeof(cplx<T>) * (size_t)plan.M;
-  WTB_REQUIRE(smem_rows <= 227 * 1024, WTB_EUNSUPPORTED,
-              "nfft=%d needs %zu B of shared memory per CTA (limit 227 KB): a power of two up to %d, any other "
-              "length up to %d for %s", N, smem_rows, sizeof(T) == 4 ? 8192 : 4096, sizeof(T) == 4 ? 4096 : 2048,
-              sizeof(T) == 4 ? "float" : "double");
-  ScaleWin win;
-  WTB_TRY(make_win(dj, &win));
   // FP32, nfft = 4096: the radix-16 forward kernel, and the register-FFT pipeline of wct_fast.cu where its one-sided
   // daughters hold (f0 >= kMinF0), its shared-memory rows and its boxcar ring fit
   const bool fast_fwd = std::is_same<T, float>::value && !generic && N == 4096;
@@ -198,10 +193,9 @@ static int wct_device(const T *d_y, int64_t pairs, int n0, int N, double dt, dou
     WTB_CUDA(cudaMemcpyAsync(d_tlo, h_tlo, sizeof(int) * S, cudaMemcpyHostToDevice, st));
     WTB_CUDA(cudaMemcpyAsync(d_thi, h_thi, sizeof(int) * S, cudaMemcpyHostToDevice, st));
   }
-  const int threads = plan.M >= 1024 ? 256 : (plan.M >= 256 ? 128 : 64);
+  const int threads = plan_threads(plan.M);
   WTB_CUDA(cudaFuncSetAttribute(k_fwd_fft<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_fwd));
   WTB_CUDA(cudaFuncSetAttribute(k_wct_rows<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_rows));
-  WTB_REQUIRE(pairs * S < (1LL << 31) && pairs * 2 < (1LL << 31), WTB_EUNSUPPORTED, "batch too large");
   WTB_TRACE_POINT(st, "wct: scratch + small copies");
   if (fast_fwd) {
     WTB_TRY(fwd_fft_4096((const float *)d_y, pairs * 2, n0, (float2 *)d_xhat, st));

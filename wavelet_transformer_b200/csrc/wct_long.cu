@@ -1,7 +1,7 @@
-// Cross spectra and coherence of long series: the rows of k_wct_rows (wct.cu) at the power-of-two lengths whose
-// shared-memory buffers do not fit one CTA (nfft >= 16384 in FP32, >= 8192 in FP64), up to nfft = 2^22, built
-// from the four-step transforms of long_fft.cuh.  wct_device (wct.cu) branches here; its scale boxcar and
-// coherence kernels (k_wct_scale) do not depend on the length and read tsm as they do after k_wct_rows.
+// Cross spectra and coherence of long series: the rows of k_wct_rows (wct.cu) at the power-of-two lengths past one
+// CTA (Route::kLong, cwt_paths.cuh), up to nfft = 2^22, built from the four-step transforms of long_fft.cuh.
+// wct_device (wct.cu) branches here; its scale boxcar and coherence kernels (k_wct_scale) do not depend on the
+// length and read tsm as they do after k_wct_rows.
 //
 // One call:
 //   k_long_pass1<T,false>, k_long_pass2<T,false>   X^ [pairs, 2, N] of the interleaved series (as cwt_long)
@@ -19,15 +19,6 @@
 #include "long_fft.cuh"
 
 namespace wtb {
-
-// Every length that the generic row kernel served before fits its 3 N complex values in 227 KB: the long path
-// starts where cwt_long_takes does, right above them.
-static_assert(3 * sizeof(float2) * 8192 <= 227 * 1024 && 2 * 2 * sizeof(float) * 8192 <= 227 * 1024 &&
-                  2 * 2 * sizeof(float) * 16384 > 227 * 1024,
-              "FP32: nfft 8192 is the last generic length, 16384 the first long one");
-static_assert(3 * sizeof(double2) * 4096 <= 227 * 1024 && 2 * 2 * sizeof(double) * 4096 <= 227 * 1024 &&
-                  2 * 2 * sizeof(double) * 8192 > 227 * 1024,
-              "FP64: nfft 4096 is the last generic length, 8192 the first long one");
 
 // The wave rule: rows per wave = those whose intermediates fit 64 MiB (long_wave_rows), four N-point fields per
 // row (two buffers of P and C) when the row is smoothed, two (W1, W2) when it is not.
