@@ -226,6 +226,33 @@ int wtb_wct_significance(double a1, double a2, double dt, double dj, double s0, 
 int wtb_rednoise(double a1, double a2, int nsurr, int64_t first, int64_t count,
                  uint64_t seed, int flags, void *out, void *stream);
 
+/* The surrogate triples of wtb_partial_wct_mc_hist: out [count, 3, nsurr], series 0, 1, 2 with coefficients ay, a1,
+ * a2 (each its own burn-in).  Series `which` of realisation m draws Philox counter (t >> 2, which, m lo, m hi), so
+ * series 0 and 1 of a triple are wtb_rednoise(ay, a1)'s pair. */
+int wtb_rednoise_triples(double ay, double a1, double a2, int nsurr, int64_t first, int64_t count,
+                         uint64_t seed, int flags, void *out, void *stream);
+
+/* ---- Monte Carlo significance of partial and multiple coherence (Ng & Chan 2012): the recipe of
+ * wtb_wct_mc_hist applied to three independent AR(1) series -- */
+/* hist: [2, J+1, WTB_NBINS] uint64 (PWC rows, then MWC rows), ADDED to.  surrogates: NULL -> device
+ * Philox AR(1) triples (wtb_rednoise_triples), else [mc_count, 3, nsurr] real.  Geometry (nsurr, maxscale) as
+ * wtb_wct_mc_geometry; rows s < maxscale, columns inside the reliable region, bins as wtb_wct_mc_hist (NaN and
+ * negative values skipped).  Flags: WTB_F64, WTB_DEVICE_PTRS (hist and surrogates in device memory),
+ * WTB_NOISE_WHITE, WTB_FFT_NO_PAD (surrogates transformed at their own length, else padded to a power of two),
+ * WTB_GENERIC_ONLY.  One CTA per transform only: nfft up to 8192 in FP32 / 4096 in FP64 padded (series of about
+ * 1365 / 680 samples with s0 = 2 dt), any other length up to 4096 / 2048; longer ones, |a| >= 1, NaN coefficients
+ * and J < 0 are refused before any copy or launch.  mc_count == 0 is a no-op. */
+int wtb_partial_wct_mc_hist(double ay, double a1, double a2, double dt, double dj, double s0, int J, double f0,
+                            int64_t mc_first, int64_t mc_count, uint64_t seed, const void *surrogates,
+                            int flags, uint64_t *hist, void *stream);
+/* One call over the pool (realisations 0 .. mc_count-1 split by global index; the result does not depend on the
+ * number of GPUs): sig_pwc, sig_mwc [J+1] (NaN / 0 rows as wtb_wct_sig_from_hist); hist_out may be NULL.  Host
+ * buffers only; limits and refusals as wtb_partial_wct_mc_hist. */
+int wtb_partial_wct_significance(double ay, double a1, double a2, double dt, double dj, double s0, int J,
+                                 double f0, double level, int64_t mc_count, uint64_t seed,
+                                 const void *surrogates, int flags, double *sig_pwc, double *sig_mwc,
+                                 uint64_t *hist_out);
+
 /* ---- MODWT: replaces src/modwt.py:126 modwt, :147 imodwt, :163 modwtmra --- */
 /* Every filterbank entry point below (wtb_modwt .. wtb_waverec) takes any n.
  * One CTA holds a series in shared memory while its buffers fit 227 KB: up to

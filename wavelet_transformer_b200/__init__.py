@@ -14,11 +14,12 @@ Layout
     pywt_compat.py    PyWavelets-shaped facade (``import ... as pywt``)
     api/              re-authored reference entry points (same names/signatures)
     engine.py         batched / multi-GPU entry points (series and Monte Carlo shards)
-    partial_coherence.py  partial and multiple wavelet coherence of three series (``partial_wct``)
+    partial_coherence.py  partial and multiple wavelet coherence of three series (``partial_wct``) and their
+                      Monte-Carlo significance (``partial_wct_significance``)
 """
 
 from ._shim import (WaveletEngineError, device_count, get_fft_padding, get_precision, gpu_count, init,  # noqa: F401
                     init_multi, lib_path, set_fft_padding, set_precision, shutdown)
-from .partial_coherence import partial_wct  # noqa: F401
+from .partial_coherence import partial_wct, partial_wct_significance  # noqa: F401
 
 __version__ = "0.1.0"

@@ -107,6 +107,11 @@ _SIGNATURES = {
     "wtb_wct_sig_from_hist_device": ([_vp, _i32, _i32, _f64, _vp, _vp, _vp], _i32),
     "wtb_wct_significance": ([_f64, _f64, _f64, _f64, _f64, _i32, _f64, _f64, _i64, _u64, _vp, _i32, _pd, _vp], _i32),
     "wtb_rednoise": ([_f64, _f64, _i32, _i64, _i64, _u64, _i32, _vp, _vp], _i32),
+    "wtb_rednoise_triples": ([_f64, _f64, _f64, _i32, _i64, _i64, _u64, _i32, _vp, _vp], _i32),
+    "wtb_partial_wct_mc_hist": ([_f64, _f64, _f64, _f64, _f64, _f64, _i32, _f64, _i64, _i64, _u64, _vp, _i32, _vp,
+                                 _vp], _i32),
+    "wtb_partial_wct_significance": ([_f64, _f64, _f64, _f64, _f64, _f64, _i32, _f64, _f64, _i64, _u64, _vp, _i32,
+                                      _pd, _pd, _vp], _i32),
     "wtb_modwt": ([_vp, _i64, _i32, _pd, _pd, _i32, _i32, _i32, _vp, _vp], _i32),
     "wtb_imodwt": ([_vp, _i64, _i32, _pd, _pd, _i32, _i32, _i32, _vp, _vp], _i32),
     "wtb_modwtmra": ([_vp, _i64, _i32, _pd, _i32, _i32, _vp, _vp], _i32),
@@ -597,6 +602,63 @@ def rednoise(a1, a2, nsurr, first, count, seed, *, f64=False, white=False):
     flags = (F64 if f64 else 0) | (NOISE_WHITE if white else 0)
     _check(lib().wtb_rednoise(a1, a2, nsurr, int(first), int(count), C.c_uint64(int(seed)), flags,
                               _ptr(out), None), "wtb_rednoise")
+    return out
+
+
+def _mc_flags(f64, white, generic_only):
+    return ((F64 if f64 else 0) | (NOISE_WHITE if white else 0) | (GENERIC_ONLY if generic_only else 0)
+            | (FFT_NO_PAD if _fft_pad == "none" else 0))
+
+
+def _triples(surrogates, mc_count, dt, dj, s0, J, f0, f64):
+    if surrogates is None:
+        return None
+    nsurr, _ = wct_mc_geometry(dt, dj, s0, J, f0)
+    sur = np.ascontiguousarray(surrogates, dtype=_dtype(f64))
+    if sur.shape != (mc_count, 3, nsurr):
+        raise ValueError(f"surrogates must have shape ({mc_count}, 3, {nsurr}), got {sur.shape}")
+    return sur
+
+
+def partial_wct_mc_hist(ay, a1, a2, dt, dj, s0, J, f0=6.0, *, mc_first=0, mc_count=300, seed=0, surrogates=None,
+                        f64=None, white=False, hist=None, generic_only=False):
+    """Per-scale histograms [2, S, 1000] (uint64; PWC rows, then MWC rows) of the partial and multiple coherence
+    of `mc_count` AR(1) surrogate triples (y, x1, x2) with coefficients (ay, a1, a2).  `surrogates`
+    ([mc_count, 3, nsurr] host array) switches to injected-noise mode."""
+    f64 = _resolve_f64(f64)
+    S = int(J) + 1
+    if hist is None:
+        hist = np.zeros((2, S, NBINS), dtype=np.uint64)
+    sur = _triples(surrogates, mc_count, dt, dj, s0, J, f0, f64)
+    _check(lib().wtb_partial_wct_mc_hist(ay, a1, a2, dt, dj, s0, int(J), f0, int(mc_first), int(mc_count),
+                                         C.c_uint64(int(seed)), _ptr(sur), _mc_flags(f64, white, generic_only),
+                                         _ptr(hist), None), "wtb_partial_wct_mc_hist")
+    return hist
+
+
+def partial_wct_significance(ay, a1, a2, dt, dj, s0, J, f0=6.0, *, level=0.95, mc_count=300, seed=0,
+                             surrogates=None, f64=None, white=False, generic_only=False, return_hist=False):
+    """Monte-Carlo significance of partial and multiple coherence in one call (wtb_partial_wct_significance):
+    every device of init_multi() takes a block of realisations.  Returns (sig_pwc, sig_mwc), each [J+1] (and the
+    summed histogram [2, J+1, 1000] with return_hist)."""
+    f64 = _resolve_f64(f64)
+    S = int(J) + 1
+    sur = _triples(surrogates, mc_count, dt, dj, s0, J, f0, f64)
+    sig_pwc, sig_mwc = np.empty(S), np.empty(S)
+    hist = np.zeros((2, S, NBINS), dtype=np.uint64) if return_hist else None
+    _check(lib().wtb_partial_wct_significance(ay, a1, a2, dt, dj, s0, int(J), f0, float(level), int(mc_count),
+                                              C.c_uint64(int(seed)), _ptr(sur), _mc_flags(f64, white, generic_only),
+                                              _dp(sig_pwc), _dp(sig_mwc), _ptr(hist)),
+           "wtb_partial_wct_significance")
+    return (sig_pwc, sig_mwc, hist) if return_hist else (sig_pwc, sig_mwc)
+
+
+def rednoise_triples(ay, a1, a2, nsurr, first, count, seed, *, f64=False, white=False):
+    """The device surrogate triples of partial_wct_mc_hist: [count, 3, nsurr]."""
+    out = np.empty((count, 3, nsurr), dtype=_dtype(f64))
+    flags = (F64 if f64 else 0) | (NOISE_WHITE if white else 0)
+    _check(lib().wtb_rednoise_triples(ay, a1, a2, nsurr, int(first), int(count), C.c_uint64(int(seed)), flags,
+                                      _ptr(out), None), "wtb_rednoise_triples")
     return out
 
 

@@ -101,5 +101,9 @@ int wct_long(const T *d_y, int64_t pairs, int n0, int N, double dt, const Axes &
 
 // wct.cu: rows with at least one sample inside the reliable region (multi.cu's percentile step)
 void mc_row_has_points(int nsurr, double dt, const Axes &ax, double f0, std::vector<uint8_t> *any);
+// wct.cu: per scale, the columns [tlo, thi] inside the reliable region of nsurr-sample surrogates ([1, 0] for none),
+// and whether there are any (the Monte-Carlo histograms of wct.cu and pwct.cu)
+void coi_ranges(int nsurr, double dt, const Axes &ax, double f0, std::vector<int> *tlo, std::vector<int> *thi,
+                std::vector<uint8_t> *any);
 
 }  // namespace wtb

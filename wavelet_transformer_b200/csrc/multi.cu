@@ -357,3 +357,37 @@ extern "C" int wtb_wct_significance(double a1, double a2, double dt, double dj, 
   if (hist_out) std::memcpy(hist_out, hist.data(), sizeof(uint64_t) * cells);
   return wtb_wct_sig_from_hist(hist.data(), S, maxscale, level, any.data(), sig95);
 }
+
+// ---- Monte-Carlo significance of partial and multiple coherence in one call: every pool device bins its block of
+// realisations into its own histogram, the host sums them (1 MB each at most: no peer reduction needed) and runs the
+// percentile step on each half.
+extern "C" int wtb_partial_wct_significance(double ay, double a1, double a2, double dt, double dj, double s0, int J,
+                                            double f0, double level, int64_t mc_count, uint64_t seed,
+                                            const void *surrogates, int flags, double *sig_pwc, double *sig_mwc,
+                                            uint64_t *hist_out) {
+  WTB_REQUIRE(sig_pwc && sig_mwc && mc_count >= 0, WTB_EINVAL, "wtb_partial_wct_significance: bad arguments");
+  WTB_REQUIRE(!(flags & WTB_DEVICE_PTRS), WTB_EINVAL, "wtb_partial_wct_significance takes host buffers only");
+  WTB_REQUIRE(J >= 0, WTB_EINVAL, "wtb_partial_wct_significance needs a resolved J");
+  int nsurr = 0, maxscale = 0;
+  WTB_TRY(wtb_wct_mc_geometry(dt, dj, s0, J, f0, &nsurr, &maxscale));
+  Axes ax;
+  WTB_TRY(resolve_axes(nsurr, dt, dj, s0, J, f0, &ax));
+  const int S = J + 1;
+  const size_t cells = 2 * (size_t)S * WTB_NBINS;
+  std::vector<uint8_t> any;
+  mc_row_has_points(nsurr, dt, ax, f0, &any);
+  const int G = (int)std::min<int64_t>(pool_size(), std::max<int64_t>(mc_count, 1));
+  std::vector<std::vector<uint64_t>> part(G, std::vector<uint64_t>(cells, 0));
+  const size_t triple_bytes = ((flags & WTB_F64) ? 8 : 4) * 3 * (size_t)nsurr;
+  WTB_TRY(run_sharded_fn(mc_count, 2, nullptr, [&](int r, int64_t first, int64_t count, cudaStream_t st) {
+    if (r >= G) { set_error("the GPU pool changed during the call"); return WTB_EINVAL; }
+    const void *sur = surrogates ? (const char *)surrogates + first * triple_bytes : nullptr;
+    return wtb_partial_wct_mc_hist(ay, a1, a2, dt, dj, s0, J, f0, first, count, seed, sur, flags, part[r].data(), st);
+  }));
+  std::vector<uint64_t> hist(cells, 0);
+  for (int r = 0; r < G; ++r)
+    for (size_t i = 0; i < cells; ++i) hist[i] += part[r][i];
+  if (hist_out) std::memcpy(hist_out, hist.data(), sizeof(uint64_t) * cells);
+  WTB_TRY(wtb_wct_sig_from_hist(hist.data(), S, maxscale, level, any.data(), sig_pwc));
+  return wtb_wct_sig_from_hist(hist.data() + (size_t)S * WTB_NBINS, S, maxscale, level, any.data(), sig_mwc);
+}

@@ -2,9 +2,10 @@
 // by pycwt.wct_significance): y[t] = g*y[t-1] + eps[t], eps ~ N(0,1), with the
 // first tau = ceil(-2/ln|g|) samples dropped.
 //
-// Philox4x32-10 keyed by `seed`; the counter is (sample block, series 0/1,
+// Philox4x32-10 keyed by `seed`; the counter is (sample block, series 0 .. K-1,
 // GLOBAL realisation index lo/hi), so a realisation's noise does not depend on
-// how realisations are partitioned over GPUs or chunks.
+// how realisations are partitioned over GPUs or chunks.  K = 2 for coherence
+// pairs, K = 3 for the (y, x1, x2) triples of partial / multiple coherence.
 #include "common.cuh"
 
 namespace wtb {
@@ -37,25 +38,26 @@ __device__ __forceinline__ float2 box_muller(uint32_t a, uint32_t b) {
 
 constexpr int kNoiseThreads = 256;
 
-// One CTA = one series (realisation m, which in {0,1}).  Each thread owns a
+// One CTA = one series (realisation m, which in [0, K)).  Each thread owns a
 // contiguous chunk of the N+tau samples; chunk carries are chained in shared
 // memory (a 256-step serial pass, negligible next to the transforms).
-template <typename T>
-__global__ void k_rednoise(double g1, double g2, int tau1, int tau2, int nsurr, int64_t first,
-                           uint64_t seed, int white, T *__restrict__ out) {
+// out: [count, K, nsurr]; series `which` has coefficient g[which], burn-in tau[which].
+template <typename T, int K>
+__global__ void k_rednoise(double g0, double g1, double g2, int tau0, int tau1, int tau2, int nsurr,
+                           int64_t first, uint64_t seed, int white, T *__restrict__ out) {
   __shared__ double s_end[kNoiseThreads];
   __shared__ double s_carry[kNoiseThreads];
-  const int64_t local = blockIdx.x >> 1;
-  const int which = blockIdx.x & 1;
+  const int64_t local = blockIdx.x / K;
+  const int which = blockIdx.x % K;
   const uint64_t real = (uint64_t)(first + local);
-  const double g = which ? g2 : g1;
-  const int tau = which ? tau2 : tau1;
+  const double g = which == 0 ? g0 : (which == 1 ? g1 : g2);
+  const int tau = which == 0 ? tau0 : (which == 1 ? tau1 : tau2);
   const int M = nsurr + tau;
   int chunk = (M + kNoiseThreads - 1) / kNoiseThreads;
   chunk = (chunk + 3) & ~3;  // whole Philox blocks of 4 normals
   const int t0 = threadIdx.x * chunk;
   const uint2 key = make_uint2((uint32_t)seed, (uint32_t)(seed >> 32));
-  T *dst = out + ((int64_t)local * 2 + which) * nsurr;
+  T *dst = out + ((int64_t)local * K + which) * nsurr;
 
   // pass 1: local recurrence with zero carry-in, remember the chunk-end value
   double y = 0.0;
@@ -102,38 +104,69 @@ static int burn_in(double g) {
   return (int)std::ceil(-2.0 / std::log(std::fabs(g)));
 }
 
-template <typename T>
-int rednoise_device(double a1, double a2, int nsurr, int64_t first, int64_t count, uint64_t seed,
-                    bool white, T *d_out, cudaStream_t st) {
-  WTB_REQUIRE(count * 2 < (1LL << 31), WTB_EUNSUPPORTED, "too many surrogates in one launch");
-  k_rednoise<T><<<(unsigned)(count * 2), kNoiseThreads, 0, st>>>(
-      a1, a2, burn_in(a1), burn_in(a2), nsurr, first, seed, white ? 1 : 0, d_out);
+template <typename T, int K>
+static int rednoise_launch(const double (&g)[3], int nsurr, int64_t first, int64_t count, uint64_t seed, bool white,
+                           T *d_out, cudaStream_t st) {
+  WTB_REQUIRE(count * K < (1LL << 31), WTB_EUNSUPPORTED, "too many surrogates in one launch");
+  k_rednoise<T, K><<<(unsigned)(count * K), kNoiseThreads, 0, st>>>(
+      g[0], g[1], g[2], burn_in(g[0]), burn_in(g[1]), burn_in(g[2]), nsurr, first, seed, white ? 1 : 0, d_out);
   WTB_LAUNCH_CHECK();
   return WTB_OK;
 }
+
+template <typename T>
+int rednoise_device(double a1, double a2, int nsurr, int64_t first, int64_t count, uint64_t seed,
+                    bool white, T *d_out, cudaStream_t st) {
+  return rednoise_launch<T, 2>({a1, a2, 0.0}, nsurr, first, count, seed, white, d_out, st);
+}
 template int rednoise_device<float>(double, double, int, int64_t, int64_t, uint64_t, bool, float *, cudaStream_t);
 template int rednoise_device<double>(double, double, int, int64_t, int64_t, uint64_t, bool, double *, cudaStream_t);
+
+template <typename T>
+int rednoise_triples_device(double ay, double a1, double a2, int nsurr, int64_t first, int64_t count,
+                            uint64_t seed, bool white, T *d_out, cudaStream_t st) {
+  return rednoise_launch<T, 3>({ay, a1, a2}, nsurr, first, count, seed, white, d_out, st);
+}
+template int rednoise_triples_device<float>(double, double, double, int, int64_t, int64_t, uint64_t, bool, float *,
+                                            cudaStream_t);
+template int rednoise_triples_device<double>(double, double, double, int, int64_t, int64_t, uint64_t, bool, double *,
+                                             cudaStream_t);
 
 }  // namespace wtb
 
 using namespace wtb;
 
-extern "C" int wtb_rednoise(double a1, double a2, int nsurr, int64_t first, int64_t count, uint64_t seed,
-                            int flags, void *out, void *stream) {
-  WTB_REQUIRE(out && nsurr > 0 && count >= 0 && first >= 0, WTB_EINVAL, "wtb_rednoise: bad arguments");
-  WTB_REQUIRE(fabs(a1) < 1 && fabs(a2) < 1, WTB_EINVAL, "AR(1) coefficients must lie in (-1, 1)");
+// wtb_rednoise (K = 2) and wtb_rednoise_triples (K = 3)
+template <int K>
+static int rednoise_entry(const char *name, const double (&g)[3], int nsurr, int64_t first, int64_t count,
+                          uint64_t seed, int flags, void *out, void *stream) {
+  WTB_REQUIRE(out && nsurr > 0 && count >= 0 && first >= 0, WTB_EINVAL, "%s: bad arguments", name);
+  for (int i = 0; i < K; ++i)
+    WTB_REQUIRE(fabs(g[i]) < 1, WTB_EINVAL, "AR(1) coefficients must lie in (-1, 1)");
   WTB_ENTER(flags, out, stream);
   if (count == 0) return WTB_OK;
   cudaStream_t st = (cudaStream_t)stream;
   const bool f64 = flags & WTB_F64;
-  const size_t bytes = (f64 ? 8 : 4) * (size_t)count * 2 * nsurr;
+  const size_t bytes = (f64 ? 8 : 4) * (size_t)count * K * nsurr;
   void *d = out;
   if (!(flags & WTB_DEVICE_PTRS)) WTB_TRY(staging_reserve(bytes, &d));
-  if (f64) WTB_TRY(rednoise_device<double>(a1, a2, nsurr, first, count, seed, flags & WTB_NOISE_WHITE, (double *)d, st));
-  else WTB_TRY(rednoise_device<float>(a1, a2, nsurr, first, count, seed, flags & WTB_NOISE_WHITE, (float *)d, st));
+  const bool white = flags & WTB_NOISE_WHITE;
+  const int rc = f64 ? rednoise_launch<double, K>(g, nsurr, first, count, seed, white, (double *)d, st)
+                     : rednoise_launch<float, K>(g, nsurr, first, count, seed, white, (float *)d, st);
+  WTB_TRY(rc);
   if (!(flags & WTB_DEVICE_PTRS)) {
     WTB_TRY(copy_to_host(out, d, bytes, st));
     WTB_CUDA(cudaStreamSynchronize(st));
   }
   return WTB_OK;
+}
+
+extern "C" int wtb_rednoise(double a1, double a2, int nsurr, int64_t first, int64_t count, uint64_t seed,
+                            int flags, void *out, void *stream) {
+  return rednoise_entry<2>("wtb_rednoise", {a1, a2, 0.0}, nsurr, first, count, seed, flags, out, stream);
+}
+
+extern "C" int wtb_rednoise_triples(double ay, double a1, double a2, int nsurr, int64_t first, int64_t count,
+                                    uint64_t seed, int flags, void *out, void *stream) {
+  return rednoise_entry<3>("wtb_rednoise_triples", {ay, a1, a2}, nsurr, first, count, seed, flags, out, stream);
 }

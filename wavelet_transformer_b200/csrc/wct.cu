@@ -251,7 +251,7 @@ int rednoise_device(double a1, double a2, int nsurr, int64_t first, int64_t coun
                     bool white, T *d_out, cudaStream_t st);
 
 // Reliable-region column range per scale, evaluated in double exactly as pycwt does.
-static void coi_ranges(int nsurr, double dt, const Axes &ax, double f0, std::vector<int> *tlo,
+void coi_ranges(int nsurr, double dt, const Axes &ax, double f0, std::vector<int> *tlo,
                        std::vector<int> *thi, std::vector<uint8_t> *any) {
   const int S = ax.J + 1;
   const double c = morlet_flambda(f0) / std::sqrt(2.0) * dt;
