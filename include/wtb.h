@@ -284,6 +284,27 @@ int wtb_modwtmra_taps(const void *w, int64_t batch, int n, const double *g,
                       const double *h, int L, int J, int flags, void *out,
                       void *stream);
 
+/* ---- MODWT wavelet variance, covariance and cross-correlation by level (Percival & Walden 2000, ch. 8;
+ * Whitcher, Guttorp & Percival 2000): the time_scale_regression companion, reduced on the device --------- */
+/* The MODWT is wtb_modwt's (same kernels, same bits): W_j[t] = sum_l h~_l V_{j-1}[(t - 2^(j-1) l) mod n] with
+ * h~ = h / sqrt 2, g~ = g / sqrt 2.  For a filter of length L, L_j = (2^j - 1)(L - 1) + 1; W_j[t] is free of
+ * the circular wrap exactly for t >= L_j - 1, and M_j = n - L_j + 1 coefficients are.  For j = 1..J (the
+ * scaling row V_J is not included):
+ *   var_x_out [batch, J]          nu2_X(j) = (1/M_j) sum_{t=L_j-1}^{n-1} W_{X,j}[t]^2 (var_y_out likewise for y)
+ *   xcov_out  [batch, J, 2K+1]    gamma_XY(j, tau) = (1/M_j) sum_t W_{X,j}[t] W_{Y,j}[t+tau], lags tau = -K..K,
+ *                                 over the t with t and t+tau in [L_j-1, n-1]; divisor M_j at every lag
+ *                                 (biased); lag 0 is the wavelet covariance.
+ * NaN where M_j <= 0 and for |tau| >= M_j, never an error.  Outputs are double in both precisions (host or
+ * device memory per WTB_DEVICE_PTRS); sums run in double in a fixed order that depends on n, L and j only, so
+ * results are bit-identical across batch, chunking, pool size and host vs device pointers.  y == NULL is the
+ * variance of x alone (var_y_out and xcov_out must then be NULL; var_x_out has the pair call's bits).
+ * K = max_lag.  WTB_EINVAL: no output requested, J outside [1, 30], max_lag outside [0, 8192] or >= n; L outside
+ * [2, 32]: WTB_EUNSUPPORTED.  Refusals come before any copy or launch; batch == 0 is a no-op.  Flags: WTB_F64,
+ * WTB_DEVICE_PTRS, WTB_GENERIC_ONLY (the MODWT's generic kernels). */
+int wtb_modwt_wavelet_stats(const void *x, const void *y, int64_t batch, int n, const double *g,
+                            const double *h, int L, int J, int max_lag, int flags,
+                            double *var_x_out, double *var_y_out, double *xcov_out, void *stream);
+
 /* ---- DWT: replaces pywt.wavedec / pywt.waverec (src/dwt.py:104,71,120) ---- */
 /* lens: [level+1] lengths of cA_L, cD_L, ..., cD_1 for symmetric mode. */
 int wtb_dwt_coeff_lens(int n, int L, int level, int *lens);

@@ -16,10 +16,13 @@ Layout
     engine.py         batched / multi-GPU entry points (series and Monte Carlo shards)
     partial_coherence.py  partial and multiple wavelet coherence of three series (``partial_wct``) and their
                       Monte-Carlo significance (``partial_wct_significance``)
+    wavelet_stats.py  MODWT wavelet variance, covariance and cross-correlation by level with confidence
+                      intervals (``wavelet_variance``, ``wavelet_correlation``)
 """
 
 from ._shim import (WaveletEngineError, device_count, get_fft_padding, get_precision, gpu_count, init,  # noqa: F401
                     init_multi, lib_path, set_fft_padding, set_precision, shutdown)
 from .partial_coherence import partial_wct, partial_wct_significance  # noqa: F401
+from .wavelet_stats import wavelet_correlation, wavelet_variance  # noqa: F401
 
 __version__ = "0.1.0"

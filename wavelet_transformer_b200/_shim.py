@@ -116,6 +116,7 @@ _SIGNATURES = {
     "wtb_imodwt": ([_vp, _i64, _i32, _pd, _pd, _i32, _i32, _i32, _vp, _vp], _i32),
     "wtb_modwtmra": ([_vp, _i64, _i32, _pd, _i32, _i32, _vp, _vp], _i32),
     "wtb_modwtmra_taps": ([_vp, _i64, _i32, _pd, _pd, _i32, _i32, _i32, _vp, _vp], _i32),
+    "wtb_modwt_wavelet_stats": ([_vp, _vp, _i64, _i32, _pd, _pd, _i32, _i32, _i32, _i32, _vp, _vp, _vp, _vp], _i32),
     "wtb_dwt_coeff_lens": ([_i32, _i32, _i32, _pi], _i32),
     "wtb_dwt_max_level": ([_i32, _i32], _i32),
     "wtb_rowwise_ols": ([_vp, _i64, _vp, _i64, _i32, _i32, _i32, _pd, _vp], _i32),
@@ -749,6 +750,43 @@ def modwtmra_taps(w, g, h, *, f64=None, generic_only=False):
                                    (F64 if f64 else 0) | (GENERIC_ONLY if generic_only else 0), _ptr(out), None),
            "wtb_modwtmra_taps")
     return out[0] if w.ndim == 2 else out
+
+
+def modwt_wavelet_stats(x, y, g, h, J, max_lag=0, f64=None, generic_only=False):
+    """MODWT wavelet variance and cross-covariance by level over the coefficients free of the circular wrap
+    (wtb_modwt_wavelet_stats).  x, y: [n] or [batch, n] (y None: the variance of x alone).  Returns
+    (var_x [batch, J], var_y [batch, J] or None, xcov [batch, J, 2 max_lag + 1] or None), float64, lags
+    -max_lag..max_lag; NaN where a level has no such coefficients or a lag reaches past them.  The batch axis is
+    dropped for 1-D input."""
+    f64 = _resolve_f64(f64)
+    g, h = _taps(g, h)
+    x2 = np.ascontiguousarray(np.atleast_2d(np.asarray(x)), dtype=_dtype(f64))
+    y2 = None if y is None else np.ascontiguousarray(np.atleast_2d(np.asarray(y)), dtype=_dtype(f64))
+    if y2 is not None and y2.shape != x2.shape:
+        raise ValueError("x and y must have the same shape")
+    batch, n = x2.shape
+    J, K = int(J), int(max_lag)
+    var_x = np.empty((batch, max(J, 0)))
+    var_y = None if y2 is None else np.empty((batch, max(J, 0)))
+    xcov = None if y2 is None else np.empty((batch, max(J, 0), 2 * max(K, 0) + 1))
+    flags = (F64 if f64 else 0) | (GENERIC_ONLY if generic_only else 0)
+    _check(lib().wtb_modwt_wavelet_stats(_ptr(x2), _ptr(y2), batch, n, _dp(g), _dp(h), g.size, J, K, flags,
+                                         _ptr(var_x), _ptr(var_y), _ptr(xcov), None), "wtb_modwt_wavelet_stats")
+    if np.ndim(x) == 1:
+        var_x, var_y, xcov = (None if v is None else v[0] for v in (var_x, var_y, xcov))
+    return var_x, var_y, xcov
+
+
+def modwt_wavelet_stats_device(x_ptr, y_ptr, batch, n, g, h, J, max_lag, var_x_ptr, var_y_ptr, xcov_ptr, *,
+                               f64=False, generic_only=False, stream=0):
+    """Device-resident wtb_modwt_wavelet_stats: raw device addresses (y_ptr and any output may be 0 for "none"),
+    float64 outputs, asynchronous on `stream`."""
+    g, h = _taps(g, h)
+    dp = lambda v: _ptr(int(v)) if v else None
+    flags = DEVICE_PTRS | (F64 if f64 else 0) | (GENERIC_ONLY if generic_only else 0)
+    _check(lib().wtb_modwt_wavelet_stats(dp(x_ptr), dp(y_ptr), int(batch), int(n), _dp(g), _dp(h), g.size, int(J),
+                                         int(max_lag), flags, dp(var_x_ptr), dp(var_y_ptr), dp(xcov_ptr),
+                                         C.c_void_p(int(stream))), "wtb_modwt_wavelet_stats")
 
 
 def waverec_len(lens, L):

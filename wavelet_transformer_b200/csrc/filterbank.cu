@@ -224,7 +224,7 @@ __global__ void k_waverec(const T *__restrict__ coeffs, LevelPlan plan, Taps tap
 }
 
 // ---- host side -----------------------------------------------------------------------------
-static int make_taps(const double *lo, const double *hi, int L, double scale, Taps *t) {
+int make_taps(const double *lo, const double *hi, int L, double scale, Taps *t) {
   WTB_REQUIRE(lo && hi && L >= 2 && L <= kMaxTaps, WTB_EUNSUPPORTED, "filter length %d outside [2,%d]", L, kMaxTaps);
   t->L = L;
   for (int i = 0; i < L; ++i) {
@@ -283,6 +283,13 @@ static int modwt_impl(const void *x, int64_t batch, int n, const Taps &taps, int
                       return WTB_OK;
                     });
 }
+
+template <typename T>
+int modwt_device(const T *x, int64_t batch, int n, const Taps &taps, int J, int flags, T *out, cudaStream_t st) {
+  return modwt_impl<T>(x, batch, n, taps, J, flags | WTB_DEVICE_PTRS, out, st);
+}
+template int modwt_device<float>(const float *, int64_t, int, const Taps &, int, int, float *, cudaStream_t);
+template int modwt_device<double>(const double *, int64_t, int, const Taps &, int, int, double *, cudaStream_t);
 
 template <typename T>
 static int imodwt_impl(const void *w, int64_t batch, int n, const Taps &taps, int J, int flags, void *out,

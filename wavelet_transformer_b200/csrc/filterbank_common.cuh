@@ -129,6 +129,10 @@ template <typename K> static int fits_one_cta(K kernel, size_t dyn, bool *fits) 
   return WTB_OK;
 }
 
+// Taps of the kernels from the caller's lo / hi, each multiplied by `scale` (1/sqrt 2 for the MODWT);
+// WTB_EUNSUPPORTED for L outside [2, kMaxTaps] (filterbank.cu)
+int make_taps(const double *lo, const double *hi, int L, double scale, Taps *t);
+
 // wtb_modwt, wtb_imodwt, wtb_modwtmra, wtb_modwtmra_taps, wtb_wavedec, wtb_waverec
 enum class FbOp { kModwt, kImodwt, kMra, kMraTaps, kWavedec, kWaverec };
 // One-CTA launch of a shape: CTA size (0: not covered), dynamic shared memory, k_mra_blk's chain length R and the
@@ -149,6 +153,12 @@ template <typename T> int wavedec_fast(const BlkShape &s, const void *x, int64_t
                                        const Taps &taps, void *coeffs, cudaStream_t st);
 template <typename T> int waverec_fast(const BlkShape &s, const void *coeffs, int64_t batch, const LevelPlan &plan,
                                        const Taps &taps, void *x, cudaStream_t st);
+
+// ---- wtb_modwt on device rows x [batch, n] -> out [batch, J+1, n], enqueued on st (filterbank.cu): the plan and
+// every kernel of wtb_modwt, bit for bit.  It reserves no staging (stage_rows takes none for device pointers), so a
+// caller may hold staging across it; the long path takes the arena.
+template <typename T>
+int modwt_device(const T *x, int64_t batch, int n, const Taps &taps, int J, int flags, T *out, cudaStream_t st);
 
 // ---- long series (filterbank_long.cu): one launch per level per wave of series, for the shapes whose generic
 // kernel above needs more than kSmemLimit of shared memory.  Each runs the whole call, host chunks included ----
